@@ -1,6 +1,6 @@
 """Benchmark of the Gram + attention classifier on B200 (contract: one JSON line on stdout from rank 0).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 Workload (BASELINE.json configs[1]): truncated ResNet50 (truncate_layer 7) + Gram + attention, random-init weights,
@@ -26,6 +26,9 @@ the sm_100a head (3 pooled-Gram launches + attention/classifier). Multi-GPU: the
   train      BASELINE.json configs[2]: full training step (forward + Gram backward + AdamW), global batch 512 sharded
              over the N ranks with DDP/NCCL (strong scaling); reported as an extra object, not as `value`; its headline
              scalars are repeated as the LAST keys of the line (train_strong_img_s, head_fwd_bwd_frac_of_bf16_peak, ...)
+
+--dump-outputs DIR writes what the last timed step returned (embeddings, logits) as DIR/<name>.npy; the weights and the
+batch come from fixed seeds, so two builds run with the same arguments can be compared output for output.
 
 --impl reference times the reference's own CPU implementation of the same forward (the unmodified reference class,
 kind "reference"; the oracle port, kind "port", only when baseline/_ref was not staged) with every host thread.
@@ -123,6 +126,28 @@ def guarded(name, fn, *a, **kw):
         import traceback
         traceback.print_exc()
         return {"error": f"{name}: {type(exc).__name__}: {exc}"[:400]}
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(directory, arrays):
+    """Writes `arrays` (name -> tensor, one row per image) as <directory>/<name>.npy in float32, so that two builds can be
+    compared output for output on the same inputs. Above DUMP_LIMIT_BYTES in all, the same fixed, seeded sample of rows
+    is kept from every array."""
+    import numpy as np
+    rows = next(iter(arrays.values())).shape[0]
+    row_bytes = sum(t[0].numel() * 4 for t in arrays.values())
+    keep = min(rows, DUMP_LIMIT_BYTES // row_bytes)
+    if keep == 0:
+        raise ValueError(f"dump_outputs: one row takes {row_bytes} bytes, more than the {DUMP_LIMIT_BYTES}-byte limit")
+    index = None
+    if keep < rows:
+        index = torch.from_numpy(np.sort(np.random.default_rng(0).choice(rows, keep, replace=False)))
+    os.makedirs(directory, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach().float().cpu()
+        np.save(os.path.join(directory, name + ".npy"), (t if index is None else t[index]).numpy())
 
 
 def timed_region(fn, steps, device, dist_mod):
@@ -454,12 +479,15 @@ def run_ours(args):
     x = x_host.to(device)
     total = B * world
 
+    last = {}
+
     def infer_step():
         with torch.no_grad():
             emb, logits = model(x)
             if world > 1:
                 logits = D.gather_rows(logits, total, world)
                 emb = D.gather_rows(emb, total, world)
+        last["embeddings"], last["logits"] = emb, logits
         return emb, logits
 
     for _ in range(args.warmup):
@@ -468,6 +496,8 @@ def run_ours(args):
     ops.LAUNCHES = 0
     with ClockSampler(device) as clocks:
         ms = timed_region(infer_step, args.steps, device, D)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)          # the last timed step's results, before any other leg runs
     records, ops.PROFILE = ops.PROFILE, None
     launches = ops.LAUNCHES
     kernels, roof = summarise_profile(records, peaks)
@@ -863,7 +893,13 @@ def main():
     ap.add_argument("--skip-reference-gpu", action="store_true")
     ap.add_argument("--skip-uint8", action="store_true", help="no e2e_uint8 leg (opt-in uint8 upload)")
     ap.add_argument("--no-graph-train", action="store_true", help="training leg: eager step only")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the embeddings and logits of the last timed step as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours (the reference arm's sample size depends on the host's speed)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

@@ -97,3 +97,33 @@ def test_peaks_and_clock_sampler_degrade_without_a_gpu(bench):
     with bench.ClockSampler(torch.device("cpu")) as c:
         pass
     assert c.summary() == {"sm_mhz": None, "sm_max_mhz": None, "reasons": [], "samples": 0}
+
+
+def test_dump_outputs_writes_float32_and_samples_the_same_rows_above_the_limit(bench, tmp_path, monkeypatch):
+    import numpy as np
+    import torch
+    emb, logits = torch.randn(10, 6, dtype=torch.float64), torch.randn(10, 2)
+    bench.dump_outputs(str(tmp_path / "all"), {"embeddings": emb, "logits": logits})
+    got = {n: np.load(tmp_path / "all" / f"{n}.npy") for n in ("embeddings", "logits")}
+    assert got["embeddings"].dtype == np.float32 and np.array_equal(got["embeddings"], emb.float().numpy())
+    assert np.array_equal(got["logits"], logits.numpy())
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 4 * 8 * 4)                    # room for 4 rows of 6 + 2 floats
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), {"embeddings": emb, "logits": logits})
+    a = {n: np.load(tmp_path / "a" / f"{n}.npy") for n in ("embeddings", "logits")}
+    assert a["embeddings"].shape == (4, 6) and a["logits"].shape == (4, 2)
+    rows = [int(np.flatnonzero((got["embeddings"] == r).all(1))[0]) for r in a["embeddings"]]
+    assert rows == sorted(rows) and np.array_equal(a["logits"], got["logits"][rows])      # the same rows of every array
+    assert all(np.array_equal(a[n], np.load(tmp_path / "b" / f"{n}.npy")) for n in a)      # and the same from run to run
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 8 * 4 - 1)                    # not even one row fits
+    with pytest.raises(ValueError, match="limit"):
+        bench.dump_outputs(str(tmp_path / "c"), {"embeddings": emb, "logits": logits})
+
+
+@pytest.mark.parametrize("argv", [["--steps", "0"], ["--impl", "reference", "--dump-outputs", "out"]])
+def test_bench_rejects_arguments_it_cannot_honour(argv, tmp_path):
+    import subprocess
+    import sys
+    res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *argv], cwd=str(tmp_path), capture_output=True,
+                         text=True, timeout=300)
+    assert res.returncode == 2 and "error:" in res.stderr and not (tmp_path / "out").exists()

@@ -67,7 +67,9 @@ def _worker(rank, world, port, out):
     dist.destroy_process_group()
 
 
-def test_two_rank_gloo_sharded_inference_and_ddp():
+def test_two_rank_gloo_sharded_inference_and_ddp(monkeypatch):
+    # the workers are CPU ranks whatever the machine has: with a GPU visible, init_from_env would give rank r cuda:r
+    monkeypatch.setenv("CUDA_VISIBLE_DEVICES", "")
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
     port = _free_port()

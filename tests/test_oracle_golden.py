@@ -106,9 +106,19 @@ def test_bf16_round_matches_torch():
     assert np.array_equal(O.bf16_round(x.numpy()), x.bfloat16().float().numpy())
 
 
-@pytest.mark.skipif(not reference_available(), reason="/root/reference only exists in the build container")
-def test_port_is_bitwise_the_reference_live():
+def test_port_is_bitwise_the_reference_live(golden_resnet):
+    """The whole port model against the reference: always against the embeddings and logits the reference computed for
+    tests/golden/resnet_g32.npz (seeded construction and batch, train-mode batch norm), and bit for bit against the
+    live reference classes when a checkout of the reference is available."""
     from torchvision import models
+    d = golden_resnet
+    m = _seeded_resnet_params().train()
+    torch.manual_seed(1)
+    with torch.no_grad():
+        emb, logits = m(torch.randn(2, 3, 64, 64))
+    assert O.rel_err(emb.numpy(), d["embeddings"]) <= 1e-6 and O.rel_err(logits.numpy(), d["logits"]) <= 1e-6
+    if not reference_available():
+        return
     ref = load_reference_models()
     for cls, ret in ((ref.TruncatedResNet50, False), (ref.TruncatedResNet50_for_test, True)):
         torch.manual_seed(0)

@@ -15,7 +15,8 @@ from oracle.ref_loader import load_reference_patchgan, reference_available
 from oracle.torch_port import patchgan_forward, patchgan_multiscale_forward
 
 GOLDEN = os.path.join(ROOT, "tests", "golden", "patchgan_head.npz")
-needs_reference = pytest.mark.skipif(not reference_available(), reason="/root/reference only exists in the build container")
+needs_reference = pytest.mark.skipif(not reference_available(),
+                                     reason="needs a checkout of the reference project (GH_REFERENCE_ROOT)")
 
 
 def rel(a, b):
@@ -71,6 +72,38 @@ def test_oracle_and_port_against_the_live_reference(norm, patch, size):
     assert rel(r["gram_norms"], torch.stack(m.get_gram_norms()).numpy()) < 2e-6
 
 
+def test_drop_in_init_and_port_reproduce_the_recorded_reference():
+    """The drop-in class rebuilt the way tests/golden/make_golden_patchgan.py built the reference's: same seed, same
+    edits of the batch-norm statistics and attention biases, then the input. Identical random init shows as the same
+    input (the constructor consumed the generator identically) and the same head tensors; the same convolution weights
+    as the same projections; the port on its submodules as the reference's embeddings, output and Gram norms."""
+    z, maps, params = load_golden()
+    torch.manual_seed(1234)
+    m = P.VariablePatchesNLayerDiscriminator_test(ndf=16, norm='batch', patch_size=30, num_classes=5,
+                                                  gram_matrix_dim=16).eval()
+    with torch.no_grad():
+        for mod in m.modules():
+            if isinstance(mod, torch.nn.BatchNorm2d):
+                mod.running_mean.normal_(0, 0.2)
+                mod.running_var.uniform_(0.5, 1.5)
+        for name in ("attention_per_layer", "attention_per_patch"):
+            getattr(m, name).in_proj_bias.normal_(0, 0.1)
+            getattr(m, name).out_proj.bias.normal_(0, 0.1)
+    x = torch.randn(2, 3, 24, 40)
+    assert torch.equal(x, torch.from_numpy(z["input"]))
+    sd = m.state_dict()
+    assert all(np.array_equal(sd[k].numpy(), params[k]) for k in O.HEAD_KEYS)
+    raw = []
+    hooks = [p.register_forward_hook(lambda mod, i, o: raw.append(o.detach())) for p in m.projection_layers]
+    with torch.no_grad():
+        emb, out, norms = patchgan_forward(m, x)
+    for h in hooks:
+        h.remove()
+    assert len(raw) == len(maps) and all(rel(a, b) < 1e-6 for a, b in zip(raw, maps))
+    assert rel(emb, z["embeddings"]) < 1e-6 and rel(out, z["output"]) < 1e-6
+    assert rel(torch.stack(norms), z["gram_norms"]) < 1e-6
+
+
 @needs_reference
 @pytest.mark.parametrize("name,kw", [
     ("VariablePatchesNLayerDiscriminator_test", dict(ndf=16, norm='batch', patch_size=70, num_classes=5, gram_matrix_dim=16)),
@@ -92,11 +125,31 @@ def test_identical_signature_init_and_state_dict_as_reference(name, kw):
     assert [n for n, _ in a.named_modules()] == [n for n, _ in b.named_modules()]
 
 
-def test_reference_module_path_resolves_to_the_b200_classes():
+def _stand_in_reference_tree(root, files):
+    """A tree with the reference's layout whose files hold only the given sources: enough to show which file a name
+    resolves to, without a checkout of the reference."""
+    for rel_path, source in files.items():
+        path = root / rel_path
+        path.parent.mkdir(parents=True, exist_ok=True)
+        path.write_text(source)
+    return str(root)
+
+
+def test_reference_module_path_resolves_to_the_b200_classes(tmp_path, monkeypatch):
     import Models.Models_Multi_PatchGAN as M
+    from heuristique_style_transfer_code_b200 import _reference
     assert M.MultiScaleDiscriminator_test is P.MultiScaleDiscriminator_test
     assert M.VariablePatchesNLayerDiscriminator_test is P.VariablePatchesNLayerDiscriminator_test
-    assert M.MultiScaleDiscriminator is P.MultiScaleDiscriminator and M.PATCH_TYPES == P.PATCH_TYPES
+    assert M.PATCH_TYPES == P.PATCH_TYPES
+    # the head-less training classes are the reference's own, taken from the reference tree the loader finds
+    rel_path = os.path.join("Models", "Models_Multi_PatchGAN.py")
+    root = _stand_in_reference_tree(tmp_path, {rel_path: "class MultiScaleDiscriminator:\n    pass\n\n\n"
+                                                         "class VariablePatchesNLayerDiscriminator:\n    pass\n"})
+    monkeypatch.setenv("GRAMHEAD_REFERENCE_ROOT", root)
+    monkeypatch.setattr(_reference, "_LOADED", {})
+    ref = _reference.load_reference_file(rel_path)
+    assert M.MultiScaleDiscriminator is P.MultiScaleDiscriminator is ref.MultiScaleDiscriminator
+    assert M.VariablePatchesNLayerDiscriminator is P.VariablePatchesNLayerDiscriminator is ref.VariablePatchesNLayerDiscriminator
 
 
 def test_structure_and_loud_failures_without_cuda():
@@ -117,13 +170,14 @@ def test_structure_and_loud_failures_without_cuda():
     assert e.shape == (1, 16) and o.shape == (1, 10)
 
 
-@needs_reference
-def test_reference_scripts_resolve_the_drop_in_classes_and_keep_their_own_functions_file():
+def test_reference_scripts_resolve_the_drop_in_classes_and_keep_their_own_functions_file(tmp_path):
     """What tools/run_ref_script.py arranges for test_Multi_PatchGAN.py: the model classes come from this repository,
     functions.functions_Multi_PatchGAN (not provided here) from the reference tree through the namespace packages."""
     import subprocess
     import sys
-    from oracle.ref_loader import REFERENCE_ROOT
+    REFERENCE_ROOT = _stand_in_reference_tree(tmp_path / "reference", {
+        os.path.join("Models", "Models_Multi_PatchGAN.py"): "raise ImportError('shadowed by the drop-in')\n",
+        os.path.join("functions", "functions_Multi_PatchGAN.py"): ""})
     code = (
         "import sys, importlib.util\n"
         f"sys.path.insert(0, {ROOT!r})\n"
@@ -134,5 +188,5 @@ def test_reference_scripts_resolve_the_drop_in_classes_and_keep_their_own_functi
         "spec = importlib.util.find_spec('functions.functions_Multi_PatchGAN')\n"
         f"assert spec is not None and spec.origin.startswith({REFERENCE_ROOT!r}), spec\n"
         "print('ok')\n")
-    out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd="/tmp")
+    out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd=str(tmp_path))
     assert out.returncode == 0 and out.stdout.strip() == "ok", out.stderr
