@@ -1,7 +1,8 @@
-// Device-side building blocks shared by the sm_100a kernels of the Gram+attention head:
+// Device-side building blocks shared by the sm_100a kernels of the library:
 // mbarrier, proxy fences, TMEM allocation, tcgen05.mma / commit / ld wrappers and the
-// UMMA shared-memory / instruction descriptors for the one operand layout every kernel
-// in this library uses: bf16, K-major, 128-byte swizzle (8-row x 128 B atoms, 1024 B apart).
+// UMMA shared-memory / instruction descriptors for the two operand layouts in use: bf16, K-major, 128-byte swizzle
+// (8-row x 128 B atoms, 1024 B apart; the Gram and attention kernels), and tf32, K-major, no swizzle (8-row x 16 B
+// core matrices; the fused stem, stem.cuh).
 //
 // Nothing here includes torch/ATen headers; the library is a plain C-ABI .so (include/gramhead.h).
 #pragma once
@@ -226,6 +227,31 @@ __host__ __device__ constexpr uint32_t make_idesc_bf16(uint32_t m, uint32_t n) {
 // Byte offset of the 8-byte group holding elements k..k+3 (k % 4 == 0) of row r inside a tile.
 __device__ __forceinline__ uint32_t sw128_off(uint32_t r, uint32_t k) {
   return (r >> 3) * kAtomBytes + (r & 7u) * kRowBytes + ((((k >> 3) ^ r) & 7u) << 4) + ((k & 7u) << 1);
+}
+// kind::tf32, D = fp32, both operands K-major, dense.
+__host__ __device__ constexpr uint32_t make_idesc_tf32(uint32_t m, uint32_t n) {
+  return (1u << 4) | (2u << 7) | (2u << 10) | ((n >> 3) << 17) | ((m >> 4) << 24);
+}
+// K-major, SWIZZLE_NONE: 8-row x 16 B core matrices, SBO between 8-row groups, LBO between the two k-chunks.
+__host__ __device__ constexpr uint64_t make_smem_desc_noswz(uint32_t addr, uint32_t lbo, uint32_t sbo) {
+  return (uint64_t)((addr & 0x3FFFFu) >> 4) | ((uint64_t)((lbo >> 4) & 0x3FFFu) << 16) |
+         ((uint64_t)((sbo >> 4) & 0x3FFFu) << 32) | ((uint64_t)1 << 46);
+}
+__device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
+                                          uint32_t accumulate) {
+  asm volatile(
+      "{\n\t"
+      ".reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t"
+      "}\n" ::"r"(tmem_d),
+      "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+__device__ __forceinline__ uint32_t tf32_rna(float f) {
+  uint32_t r;
+  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(f));
+  return r;
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -15,6 +15,7 @@
 #include "transpose.cuh"
 #include "patchgan.cuh"
 #include "pool.cuh"
+#include "stem.cuh"
 #include "style_loss.cuh"
 #include <string>
 
@@ -808,6 +809,29 @@ int gh_stem_space_to_depth(const float* x, long long img_stride, long long c_str
   const int grid = (int)(want < cap ? want : cap);
   if (z_dtype == GH_DTYPE_F32) stem_space_to_depth_kernel<float><<<grid, 256, 0, (cudaStream_t)stream>>>(p);
   else stem_space_to_depth_kernel<__nv_bfloat16><<<grid, 256, 0, (cudaStream_t)stream>>>(p);
+  return (int)cudaGetLastError();
+}
+
+int gh_stem_conv_pool_nhwc(const float* x, long long img_stride, long long c_stride, long long y_stride,
+                           long long x_stride, int B, int H, int W, const float* w_packed, const float* bias, float* out,
+                           void* stream) {
+  if (!x || !w_packed || !bias || !out || B <= 0 || H <= 0 || W <= 0) return GH_ERR_BAD_ARG;
+  if ((H & 1) || (W & 1) || (uintptr_t)w_packed % 16 != 0 || (uintptr_t)out % 16 != 0) return GH_ERR_UNSUPPORTED;
+  StemConvPoolParams p{};
+  p.x = x; p.s_img = img_stride; p.s_c = c_stride; p.s_y = y_stride; p.s_x = x_stride;
+  p.w = w_packed; p.bias = bias; p.out = out;
+  p.B = B; p.OH = H / 2; p.OW = W / 2;
+  p.PH = (p.OH - 1) / 2 + 1;                                     // nn.MaxPool2d(3, 2, 1), floor mode
+  p.PW = (p.OW - 1) / 2 + 1;
+  p.tiles = (p.PW + kScTileCols - 1) / kScTileCols;
+  p.vec2 = x_stride == 1 && (uintptr_t)x % 8 == 0 && (img_stride % 2 == 0) && (c_stride % 2 == 0) && (y_stride % 2 == 0);
+  p.units = (long long)B * p.tiles * p.PH;
+  const int sms = sm_count_cached();
+  const int grid = (int)(p.units < sms ? p.units : sms);
+  cudaError_t e = cudaFuncSetAttribute(stem_conv_pool_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       (int)kScSmemBytes);
+  if (e != cudaSuccess) return (int)e;
+  stem_conv_pool_kernel<<<grid, kScThreads, kScSmemBytes, (cudaStream_t)stream>>>(p);
   return (int)cudaGetLastError();
 }
 

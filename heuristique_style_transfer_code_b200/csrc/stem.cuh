@@ -1,0 +1,321 @@
+// Fused stem of the inference plan (frozen_encoder.py): one kernel computes
+//   out = maxpool3x3/s2/p1( relu( conv7x7/s2/p3(x, W) + bias ) )
+// for the folded conv1 + bn1 + relu + maxpool children of the truncated encoder
+// (Models/Models_RESNET50_TRUNCATE_GRAM_with_Attention.py:17,37-40), with tf32 operands and fp32 accumulation on tcgen05.
+// The three-launch chain it replaces (space-to-depth staging, cuDNN convolution, max pool) moves 2.4 GB through HBM at
+// batch 256 x 224^2; this kernel reads the fp32 image once and writes only the pooled (B, 64, H/4, W/4) result.
+//
+// The convolution is the 4x4 stride-1 one over the 2x2 space-to-depth image (pool.cuh, gh_stem_space_to_depth):
+//   conv[y][x][o] = sum_{a,b < 4} sum_{k < 16} z[y + a][x + b][k] * W16[o][k][a][b]
+// with z's cell (Y + 2, X + 2) holding, per image channel c, the 2x2 pixel block {x[c][2Y][2X], x[c][2Y][2X+1],
+// x[c][2Y+1][2X], x[c][2Y+1][2X+1]} -- a 16-byte "k-chunk" -- and a zero 4th chunk (12 channels padded to 16).
+//
+// Implicit GEMM by descriptor shift. M = 128 consecutive conv columns of one conv row, N = 64 output channels, K = 16
+// taps x 16. The staged image rows live in shared memory K-major without swizzle as [k-chunk plane][row slot][cell][16 B]:
+// one core matrix is 8 consecutive cells (SBO = 128 B between 8-cell groups), the two k-chunks of one tf32 MMA (K = 8)
+// are two planes (LBO = plane stride). Tap (a, b) of the tile is then the same staged rows with the descriptor start moved
+// to row slot y + a and 16 B per cell of b: 16 taps x 2 MMAs of 128 x 64 x 8, no im2col copy.
+//
+// Tiles: 63 pooled columns per tile need the 127 conv columns 126 j - 1 .. 126 j + 125 (lane l = column 126 j - 1 + l),
+// i.e. staged cells 126 j - 1 .. 126 j + 129 of each padded row (131 cells). 224^2 is one tile per row (lanes with no
+// conv column are masked); wider images take ceil(PW / 63) tiles. The pooling windows of vertically adjacent pooled rows
+// share one conv row; a ring of 8 TMEM accumulators (one 64-column accumulator per conv row) keeps it.
+//
+// Epilogue: max over the (up to) three conv rows of the window straight from TMEM, then over columns x-1, x, x+1 with
+// shuffles (the one neighbour across a warp boundary goes through shared memory), then + bias and ReLU. Pooling the raw
+// sums first is exact: fl(a + b) is monotone in a, so max_i fl(a_i + b) = fl(max_i a_i + b), and ReLU is monotone.
+// NaN propagates as in nn.MaxPool2d / PoolVec::max_into, and ReLU keeps it, as torch's does.
+//
+// Work split: persistent CTAs, one per SM, each a contiguous range of (image, tile, pooled row) units; the conv row above
+// a range's first pooled row is recomputed (halo). No atomics: an image's result does not depend on its batch.
+// Warps: 0-7 producers (one staged row each, round robin), 8-11 epilogue (TMEM lane quadrants 0-3), 12 MMA issuer.
+#pragma once
+#include "common.cuh"
+
+namespace gh {
+
+constexpr int kScProducerWarps = 8;
+constexpr int kScEpiWarp0 = 8;
+constexpr int kScMmaWarp = 12;
+constexpr int kScThreads = 13 * 32;
+constexpr int kScTileCols = 63;                        // pooled columns per tile
+constexpr int kScCells = 131;                          // staged cells per row slot
+constexpr int kScItems = 3 * kScCells;                 // (image channel, cell) k-chunks a producer warp stores per row
+constexpr int kScItemIters = (kScItems + 31) / 32;
+constexpr int kScSlots = 12;                           // staged row ring: 4 rows in use by the MMAs + 8 being produced
+constexpr int kScAccSlots = 8;                         // TMEM accumulators (conv rows), 64 columns each
+constexpr uint32_t kScSlotBytes = kScCells * 16;       // 2096
+constexpr uint32_t kScPlaneBytes = kScSlots * kScSlotBytes;
+constexpr uint32_t kScWBytes = 16 * 2 * 2048;          // 16 taps x 2 MMAs x (64 rows x 2 k-chunks x 16 B)
+constexpr uint32_t kScAOff = kScWBytes;
+constexpr uint32_t kScBiasOff = kScAOff + 4 * kScPlaneBytes;
+constexpr uint32_t kScXbufOff = kScBiasOff + 64 * 4;
+constexpr uint32_t kScBarOff = kScXbufOff + 2 * 4 * 64 * 4;
+constexpr uint32_t kScBarBytes = 8 * (2 * kScSlots + 2 * kScAccSlots) + 16;
+constexpr uint32_t kScSmemBytes = kScBarOff + kScBarBytes + 1024;
+
+struct StemConvPoolParams {
+  const float* x;
+  long long s_img, s_c, s_y, s_x;      // element strides of x
+  const float* w;                      // packed tf32 weights, the shared-memory image of the B operands (kScWBytes)
+  const float* bias;                   // [64]
+  float* out;                          // (B, PH, PW, 64)
+  int B, OH, OW, PH, PW, tiles;        // conv size OH x OW = H/2 x W/2; pooled PH x PW; tiles per pooled row
+  int vec2;                            // x-contiguous pixel pairs 8 B aligned: float2 loads
+  long long units;                     // B * tiles * PH
+};
+
+__device__ __forceinline__ float max_nan(float a, float b) { return (b > a || b != b) ? b : a; }
+
+// A CTA's range of units, cut where (image, tile) changes: one segment = consecutive pooled rows py0..py1-1 of one
+// (image, tile), computed from conv rows y_lo..y_hi, staged from padded rows y_lo..y_hi + 3.
+struct ScSeg {
+  int b, j, py0, py1, y_lo, y_hi;
+};
+__device__ __forceinline__ bool sc_next(const StemConvPoolParams& p, long long& u, long long u1, ScSeg& s) {
+  if (u >= u1) return false;
+  const long long bj = u / p.PH;
+  const long long end = (bj + 1) * p.PH < u1 ? (bj + 1) * p.PH : u1;
+  s.b = (int)(bj / p.tiles);
+  s.j = (int)(bj - (long long)s.b * p.tiles);
+  s.py0 = (int)(u - bj * p.PH);
+  s.py1 = s.py0 + (int)(end - u);
+  s.y_lo = 2 * s.py0 - 1 > 0 ? 2 * s.py0 - 1 : 0;
+  s.y_hi = 2 * s.py1 - 1 < p.OH - 1 ? 2 * s.py1 - 1 : p.OH - 1;
+  u = end;
+  return true;
+}
+
+__global__ void __launch_bounds__(kScThreads, 1) stem_conv_pool_kernel(const StemConvPoolParams p) {
+  extern __shared__ uint8_t smem_raw[];
+  const uint32_t raw = smem_u32(smem_raw);
+  const uint32_t base = (raw + 1023u) & ~1023u;
+  uint8_t* gbase = smem_raw + (base - raw);
+  const uint32_t w_smem = base, a_smem = base + kScAOff;
+  const float* bias_s = reinterpret_cast<const float*>(gbase + kScBiasOff);
+  float* xbuf = reinterpret_cast<float*>(gbase + kScXbufOff);
+  const uint32_t bar_full = base + kScBarOff, bar_empty = bar_full + 8 * kScSlots;
+  const uint32_t bar_afull = bar_empty + 8 * kScSlots, bar_aempty = bar_afull + 8 * kScAccSlots;
+  const uint32_t tmem_slot = bar_aempty + 8 * kScAccSlots;
+  volatile uint32_t* tmem_slot_ptr = reinterpret_cast<volatile uint32_t*>(gbase + (tmem_slot - base));
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+
+  // Weights and bias for the CTA's life; plane 3 (the zero k-chunk of every cell) once.
+  {
+    const float4* wg = reinterpret_cast<const float4*>(p.w);
+    float4* ws = reinterpret_cast<float4*>(gbase);
+    for (int i = threadIdx.x; i < (int)(kScWBytes / 16); i += kScThreads) ws[i] = __ldg(wg + i);
+    if (threadIdx.x < 64) reinterpret_cast<float*>(gbase + kScBiasOff)[threadIdx.x] = __ldg(p.bias + threadIdx.x);
+    float4* z = reinterpret_cast<float4*>(gbase + kScAOff + 3 * kScPlaneBytes);
+    for (int i = threadIdx.x; i < (int)(kScPlaneBytes / 16); i += kScThreads) z[i] = make_float4(0.f, 0.f, 0.f, 0.f);
+    fence_proxy_async_smem();
+  }
+  if (threadIdx.x == 0) {
+    for (int s = 0; s < kScSlots; ++s) {
+      mbar_init(bar_full + 8 * s, 1);
+      mbar_init(bar_empty + 8 * s, 1);
+    }
+    for (int s = 0; s < kScAccSlots; ++s) {
+      mbar_init(bar_afull + 8 * s, 1);
+      mbar_init(bar_aempty + 8 * s, 4);
+    }
+    mbar_fence_init();
+  }
+  if (warp == kScMmaWarp) tmem_alloc(tmem_slot, 512);
+  tc_fence_before_sync();
+  __syncthreads();
+  tc_fence_after_sync();
+  const uint32_t tmem_base = *tmem_slot_ptr;
+
+  const long long u0 = p.units * blockIdx.x / gridDim.x, u1 = p.units * (blockIdx.x + 1) / gridDim.x;
+
+  if (warp < kScProducerWarps) {
+    // =========================== producers: one padded s2d row per warp, round robin ===========================
+    uint32_t gs = 0;                                   // staged rows so far (all segments)
+    long long u = u0;
+    ScSeg sg;
+    while (sc_next(p, u, u1, sg)) {
+      const int n_stage = sg.y_hi - sg.y_lo + 4;
+      const float* img = p.x + (long long)sg.b * p.s_img;
+      for (int k = 0; k < n_stage; ++k) {
+        const uint32_t g = gs + (uint32_t)k;
+        if ((int)(g % kScProducerWarps) != warp) continue;
+        const uint32_t slot = g % kScSlots;
+        const int Y = sg.y_lo + k - 2;                 // image cell row of padded row y_lo + k
+        const bool row_ok = Y >= 0 && Y < p.OH;
+        float4 v[kScItemIters];
+#pragma unroll
+        for (int it = 0; it < kScItemIters; ++it) {
+          const int i = it * 32 + lane;
+          const int c = i / kScCells, s = i - c * kScCells;
+          const int X = kScTileCols * 2 * sg.j + s - 3;
+          v[it] = make_float4(0.f, 0.f, 0.f, 0.f);
+          if (i < kScItems && row_ok && X >= 0 && X < p.OW) {
+            const float* q = img + (long long)c * p.s_c + (long long)(2 * Y) * p.s_y + (long long)(2 * X) * p.s_x;
+            if (p.vec2) {
+              const float2 t0 = __ldg(reinterpret_cast<const float2*>(q));
+              const float2 t1 = __ldg(reinterpret_cast<const float2*>(q + p.s_y));
+              v[it] = make_float4(t0.x, t0.y, t1.x, t1.y);
+            } else {
+              v[it] = make_float4(__ldg(q), __ldg(q + p.s_x), __ldg(q + p.s_y), __ldg(q + p.s_y + p.s_x));
+            }
+          }
+        }
+        mbar_wait(bar_empty + 8 * slot, ((g / kScSlots) & 1u) ^ 1u, 300u + slot);
+#pragma unroll
+        for (int it = 0; it < kScItemIters; ++it) {
+          const int i = it * 32 + lane;
+          if (i < kScItems) {
+            const int c = i / kScCells, s = i - c * kScCells;
+            sts_u4(a_smem + (uint32_t)c * kScPlaneBytes + slot * kScSlotBytes + (uint32_t)s * 16u, tf32_rna(v[it].x),
+                   tf32_rna(v[it].y), tf32_rna(v[it].z), tf32_rna(v[it].w));
+          }
+        }
+        fence_proxy_async_smem();
+        __syncwarp();
+        if (lane == 0) mbar_arrive(bar_full + 8 * slot);
+      }
+      gs += (uint32_t)n_stage;
+    }
+  } else if (warp == kScMmaWarp) {
+    // =========================== MMA issuer ===========================
+    constexpr uint32_t idesc = make_idesc_tf32(128, 64);
+    // k-chunks (0, 1) of the cells are planes 0 and 1 (LBO = one plane); the second MMA of a tap starts 2 planes on
+    const uint64_t adesc0 = make_smem_desc_noswz(a_smem, kScPlaneBytes, 128);
+    const uint64_t bdesc0 = make_smem_desc_noswz(w_smem, 1024, 128);
+    uint32_t gs = 0, gc = 0;
+    long long u = u0;
+    ScSeg sg;
+    while (sc_next(p, u, u1, sg)) {
+      const int n_conv = sg.y_hi - sg.y_lo + 1;
+      for (int k = 0; k < n_conv; ++k, ++gc) {
+        const uint32_t acc = gc % kScAccSlots;
+        mbar_wait(bar_aempty + 8 * acc, ((gc / kScAccSlots) & 1u) ^ 1u, 400u + acc);
+        uint32_t slot[4];
+#pragma unroll
+        for (int a = 0; a < 4; ++a) {
+          const uint32_t g = gs + (uint32_t)(k + a);
+          slot[a] = g % kScSlots;
+          mbar_wait(bar_full + 8 * slot[a], (g / kScSlots) & 1u, 500u + slot[a]);
+        }
+        tc_fence_after_sync();
+        if (elect_one()) {
+          const uint32_t d = tmem_base + acc * 64u;
+#pragma unroll
+          for (int a = 0; a < 4; ++a) {
+            const uint64_t arow = adesc0 + ((slot[a] * kScSlotBytes) >> 4);
+#pragma unroll
+            for (int b = 0; b < 4; ++b)
+#pragma unroll
+              for (int h = 0; h < 2; ++h) {
+                const uint64_t da = arow + ((b * 16 + h * 2 * kScPlaneBytes) >> 4);
+                const uint64_t db = bdesc0 + ((((a * 4 + b) * 2 + h) * 2048) >> 4);
+                umma_tf32(d, da, db, idesc, (a | b | h) != 0);
+              }
+          }
+          umma_commit(bar_afull + 8 * acc);
+          umma_commit(bar_empty + 8 * slot[0]);        // padded row y is not read by conv rows below y
+          if (k == n_conv - 1)
+            for (int a = 1; a < 4; ++a) umma_commit(bar_empty + 8 * slot[a]);
+        }
+        __syncwarp();
+      }
+      gs += (uint32_t)(n_conv + 3);
+    }
+  } else {
+    // =========================== epilogue: TMEM -> 3x3/s2 max -> + bias, ReLU -> NHWC ===========================
+    const int quad = warp - kScEpiWarp0;
+    const uint32_t tlane = tmem_base + ((uint32_t)(32 * quad) << 16);
+    const float neg_inf = -__int_as_float(0x7f800000);
+    uint32_t gc = 0, xb = 0;
+    long long u = u0;
+    ScSeg sg;
+    while (sc_next(p, u, u1, sg)) {
+      const int x = kScTileCols * 2 * sg.j - 1 + 32 * quad + lane;     // this lane's conv column
+      const bool col_ok = x >= 0 && x < p.OW;
+      auto acc_of = [&](int y) { return (gc + (uint32_t)(y - sg.y_lo)) % kScAccSlots; };
+      auto wait_row = [&](int y) {
+        const uint32_t g = gc + (uint32_t)(y - sg.y_lo);
+        mbar_wait(bar_afull + 8 * (g % kScAccSlots), (g / kScAccSlots) & 1u, 600u + g % kScAccSlots);
+      };
+      for (int py = sg.py0; py < sg.py1; ++py) {
+        const int ya = 2 * py - 1, yb = 2 * py, yc = 2 * py + 1;
+        const bool ha = ya >= sg.y_lo, hc = yc <= sg.y_hi;
+        if (py == sg.py0 && ha) wait_row(ya);
+        wait_row(yb);
+        if (hc) wait_row(yc);
+        tc_fence_after_sync();
+        float m[64];
+#pragma unroll
+        for (int h = 0; h < 2; ++h) {
+          uint32_t r[32];
+          tmem_ld32_nowait(tlane + acc_of(yb) * 64u + 32u * h, r);
+          tmem_ld_wait();
+#pragma unroll
+          for (int i = 0; i < 32; ++i) m[32 * h + i] = __uint_as_float(r[i]);
+          if (ha) {
+            tmem_ld32_nowait(tlane + acc_of(ya) * 64u + 32u * h, r);
+            tmem_ld_wait();
+#pragma unroll
+            for (int i = 0; i < 32; ++i) m[32 * h + i] = max_nan(m[32 * h + i], __uint_as_float(r[i]));
+          }
+          if (hc) {
+            tmem_ld32_nowait(tlane + acc_of(yc) * 64u + 32u * h, r);
+            tmem_ld_wait();
+#pragma unroll
+            for (int i = 0; i < 32; ++i) m[32 * h + i] = max_nan(m[32 * h + i], __uint_as_float(r[i]));
+          }
+        }
+        // rows ya and yb are done; yc is the next window's first row unless the segment ends here
+        tc_fence_before_sync();
+        __syncwarp();
+        if (lane == 0) {
+          if (ha) mbar_arrive(bar_aempty + 8 * acc_of(ya));
+          mbar_arrive(bar_aempty + 8 * acc_of(yb));
+          if (hc && py == sg.py1 - 1) mbar_arrive(bar_aempty + 8 * acc_of(yc));
+        }
+        if (!col_ok) {
+#pragma unroll
+          for (int i = 0; i < 64; ++i) m[i] = neg_inf;
+        }
+        // column x + 2 of lane 30 is lane 0 of the next quadrant
+        float* xs = xbuf + xb * 256;
+        if (lane == 0 && quad > 0) {
+#pragma unroll
+          for (int i = 0; i < 64; i += 4)
+            *reinterpret_cast<float4*>(xs + quad * 64 + i) = make_float4(m[i], m[i + 1], m[i + 2], m[i + 3]);
+        }
+        asm volatile("bar.sync 1, 128;" ::: "memory");
+        const bool from_next = lane == 30 && quad < 3;
+        const int qx = 16 * quad + (lane >> 1);                         // pooled column within the tile
+        const int px = kScTileCols * sg.j + qx;
+        const bool store = !(lane & 1) && qx < kScTileCols && px < p.PW;
+        float4* o = reinterpret_cast<float4*>(p.out + (((long long)sg.b * p.PH + py) * p.PW + px) * 64);
+#pragma unroll
+        for (int i = 0; i < 64; i += 4) {
+          float r4[4];
+#pragma unroll
+          for (int e = 0; e < 4; ++e) {
+            const float v1 = __shfl_down_sync(0xffffffffu, m[i + e], 1);
+            float v2 = __shfl_down_sync(0xffffffffu, m[i + e], 2);
+            if (from_next) v2 = xs[(quad + 1) * 64 + i + e];
+            float t = max_nan(max_nan(m[i + e], v1), v2) + bias_s[i + e];
+            r4[e] = t != t ? t : fmaxf(t, 0.f);
+          }
+          if (store) o[i / 4] = make_float4(r4[0], r4[1], r4[2], r4[3]);
+        }
+        xb ^= 1u;
+      }
+      gc += (uint32_t)(sg.y_hi - sg.y_lo + 1);
+    }
+  }
+
+  tc_fence_before_sync();
+  __syncthreads();
+  if (warp == kScMmaWarp) {
+    tc_fence_after_sync();
+    tmem_dealloc(tmem_base, 512);
+  }
+}
+
+}  // namespace gh

@@ -7,7 +7,9 @@ kernels (torchvision's Bottleneck.forward; Models_RESNET50_TRUNCATE_GRAM_with_At
 on a B200 69 % of the fp32 channels_last encoder's time at batch 256 is those element-wise passes
 (`bn_fw_inf` 37 %, ReLU 15 %, residual add 12 %, max-pool 5 %; profiles/r01w_launch_shares.txt), all HBM-bound.
 
-The plan keeps every convolution on cuDNN and the module's parameters untouched: folded weight copies are built lazily
+The plan keeps every convolution but the stem's on cuDNN, and the module's parameters untouched. The stem (conv1 + bn1 +
+relu + maxpool) of an fp32 plan with TF32 convolutions allowed is one kernel of the library (gh_stem_conv_pool_nhwc);
+elsewhere it is the space-to-depth chain below. Folded weight copies are built lazily
 from the live parameters / running statistics, and rebuilt whenever any of them changes (in-place update, load_state_dict,
 .to(): detected through tensor versions and storage addresses). It is used only when the result is the same function --
 module in eval mode, gradients disabled, every BatchNorm tracking running statistics -- and only for the structure it
@@ -41,6 +43,20 @@ def _stem_space_to_depth_weight(weight: torch.Tensor) -> torch.Tensor:
     w16 = weight.new_zeros((o, 16, 4, 4))
     w16[:, :12] = w12
     return w16.contiguous(memory_format=torch.channels_last)
+
+
+def _tf32_round(x: torch.Tensor) -> torch.Tensor:
+    """fp32 -> nearest tf32 (ties away from zero), as cvt.rna.tf32.f32 rounds the image side of the fused stem."""
+    bits = (x.contiguous().view(torch.int32).to(torch.int64) & 0xFFFFFFFF) + 0x1000
+    bits = bits & 0xFFFFE000
+    return torch.where(bits >= 2 ** 31, bits - 2 ** 32, bits).to(torch.int32).view(torch.float32)
+
+
+def pack_stem_weight(w16: torch.Tensor) -> torch.Tensor:
+    """(64, 16, 4, 4) space-to-depth stem weights -> the B operands of gh_stem_conv_pool_nhwc in its shared-memory
+    layout, rounded to tf32: [tap a*4+b][half h][k-chunk q][out channel n][e] = w16[n, (2h + q)*4 + e, a, b]."""
+    w = _tf32_round(w16.float().contiguous())
+    return w.view(64, 2, 2, 4, 4, 4).permute(4, 5, 1, 2, 0, 3).contiguous().view(-1)
 
 
 def _fold(conv: nn.Conv2d, bn: nn.BatchNorm2d, dtype: torch.dtype, channels_last: bool):
@@ -91,6 +107,8 @@ class FoldedEncoder:
     def __init__(self, stem, pool, stages, signature, dtype, channels_last):
         self.stem, self.pool, self.stages = stem, pool, stages
         self.stem_s2d = None
+        self.stem_packed = None        # tf32 B operands of the fused stem kernel (fp32 plans)
+        self._stem_fused = True        # A/B switch for tools/time_stem.py; the chain runs where the fused kernel does not apply
         self.signature, self.dtype, self.channels_last = signature, dtype, channels_last
 
     @staticmethod
@@ -134,6 +152,11 @@ class FoldedEncoder:
                 stages.append(blocks)
         plan = cls(stem, encoder[3], stages, encoder_signature(encoder), dtype, channels_last)
         plan.stem_s2d = stem_s2d
+        pool = encoder[3]
+        if (stem_s2d is not None and dtype == torch.float32 and conv1.out_channels == 64
+                and pool.kernel_size in (3, (3, 3)) and pool.stride in (2, (2, 2)) and pool.padding in (1, (1, 1))
+                and pool.dilation in (1, (1, 1)) and not pool.ceil_mode and not pool.return_indices):
+            plan.stem_packed = pack_stem_weight(stem_s2d[0])
         return plan
 
     @staticmethod
@@ -151,7 +174,13 @@ class FoldedEncoder:
             return ops.maxpool2d_nhwc(x, k, s, pad)
         return p(x)
 
-    def __call__(self, x: torch.Tensor):
+    def stem_forward(self, x: torch.Tensor) -> torch.Tensor:
+        """Children 0-3: conv1 + bn1 + relu + maxpool. One fused kernel (gh_stem_conv_pool_nhwc) when the chain below
+        would run in TF32 anyway (cudnn.allow_tf32, the torch default) on an fp32 plan; the chain otherwise."""
+        if (self.stem_packed is not None and self._stem_fused and torch.backends.cudnn.allow_tf32
+                and x.dtype == torch.float32 and x.dim() == 4 and x.shape[1] == 3 and x.shape[2] % 2 == 0
+                and x.shape[3] % 2 == 0):
+            return ops.stem_conv_pool(x, self.stem_packed, self.stem_s2d[1])
         if (self.stem_s2d is not None and x.dtype == torch.float32 and x.shape[1] == 3 and x.shape[2] % 2 == 0
                 and x.shape[3] % 2 == 0):
             x = self._conv_relu(ops.stem_space_to_depth(x, self.dtype), self.stem_s2d)
@@ -160,7 +189,10 @@ class FoldedEncoder:
             if self.channels_last:
                 x = x.contiguous(memory_format=torch.channels_last)
             x = self._conv_relu(x, self.stem)
-        x = self._pool(x)
+        return self._pool(x)
+
+    def __call__(self, x: torch.Tensor):
+        x = self.stem_forward(x)
         outs = []
         for blocks in self.stages:
             for c1, c2, c3, down in blocks:

@@ -296,6 +296,29 @@ def stem_space_to_depth(x: torch.Tensor, dtype: torch.dtype) -> torch.Tensor:
     return z
 
 
+def stem_conv_pool(x: torch.Tensor, packed_weight: torch.Tensor, bias: torch.Tensor) -> torch.Tensor:
+    """(B, 3, H, W) fp32 images (any strides, H and W even) -> channels_last (B, 64, PH, PW) fp32:
+    maxpool3x3/s2/p1(relu(conv7x7/s2/p3(x) + bias)) in one kernel with tf32 operands (gh_stem_conv_pool_nhwc).
+    packed_weight: frozen_encoder.pack_stem_weight() of the folded weights; bias: the folded (64,) bias."""
+    _require_cuda(x, "x")
+    if x.dim() != 4 or x.shape[1] != 3 or x.dtype != torch.float32 or x.shape[2] % 2 or x.shape[3] % 2:
+        raise GramHeadError("gramhead: stem_conv_pool takes fp32 (B, 3, H, W) images with even H and W")
+    if (packed_weight.dtype != torch.float32 or packed_weight.numel() != 16384 or not packed_weight.is_contiguous()
+            or bias.dtype != torch.float32 or bias.numel() != 64 or not bias.is_contiguous()
+            or packed_weight.device != x.device or bias.device != x.device):
+        raise GramHeadError("gramhead: stem_conv_pool takes the packed fp32 stem weights (16384) and bias (64) on x's device")
+    b, _, h, w = x.shape
+    oh, ow = h // 2, w // 2
+    ph, pw = (oh - 1) // 2 + 1, (ow - 1) // 2 + 1
+    out = torch.empty((b, 64, ph, pw), device=x.device, dtype=torch.float32, memory_format=torch.channels_last)
+    work = dict(bytes=(x.numel() + out.numel()) * 4, flops=2 * b * oh * ow * 64 * 147, kind="stem_conv_pool")
+    with torch.cuda.device(x.device), _Timed(f"stem_conv_pool[HW={h}x{w}]", 1, x.device, **work):
+        rc = _lib.lib().gh_stem_conv_pool_nhwc(x.data_ptr(), x.stride(0), x.stride(1), x.stride(2), x.stride(3), b, h, w,
+                                               packed_weight.data_ptr(), bias.data_ptr(), out.data_ptr(), _stream_ptr(x))
+    check(rc, "gh_stem_conv_pool_nhwc")
+    return out
+
+
 def normalize_u8(x: torch.Tensor, mean, std, out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """(B, C, H, W) uint8 pixels on the device -> the fp32 batch transforms.ToTensor() + transforms.Normalize(mean, std)
     produce on the host (reference test_RESNET50_Truncate_gram_attention.py:64-65), bit for bit (gh_normalize_u8).

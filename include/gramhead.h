@@ -180,6 +180,20 @@ int gh_maxpool2d_nhwc(const void* in, int dtype, void* out, int B, int H, int W,
 int gh_stem_space_to_depth(const float* x, long long img_stride, long long c_stride, long long y_stride,
                            long long x_stride, int B, int H, int W, void* z, int z_dtype, void* stream);
 
+/* The whole stem of the inference plan in one kernel (csrc/stem.cuh): conv1 (7x7, stride 2, padding 3) with bn1 folded
+ * in, relu and maxpool (3, stride 2, padding 1) -- children 0-3 of `self.truncated_encoder`,
+ * Models/Models_RESNET50_TRUNCATE_GRAM_with_Attention.py:17,37-40 -- in place of gh_stem_space_to_depth, the cuDNN
+ * convolution and gh_maxpool2d_nhwc. tf32 operands (rounded to nearest, ties away), fp32 accumulation (kind::tf32).
+ * x: fp32 (B, 3, H, W) with the given element strides (NCHW, channels_last or strided), H and W even
+ * (GH_ERR_UNSUPPORTED otherwise). w_packed: the 64 x 256 folded space-to-depth weights (frozen_encoder.py,
+ * _stem_space_to_depth_weight) rounded to tf32 and laid out as the kernel's shared-memory B operands:
+ * [tap a*4+b][half h][k-chunk q][out channel n][4] = W16[n][(2h + q)*4 + e][a][b], 16384 floats, 16 B aligned.
+ * bias: [64]. out: (B, PH, PW, 64) dense NHWC storage of a channels_last (B, 64, PH, PW) tensor, 16 B aligned,
+ * PH = (H/2 - 1)/2 + 1, PW = (W/2 - 1)/2 + 1 (nn.MaxPool2d's floor mode). NaN propagates as in the reference. */
+int gh_stem_conv_pool_nhwc(const float* x, long long img_stride, long long c_stride, long long y_stride,
+                           long long x_stride, int B, int H, int W, const float* w_packed, const float* bias, float* out,
+                           void* stream);
+
 /* ---- Gram head of the Multi-PatchGAN discriminator (the *_test classes of Models/Models_Multi_PatchGAN.py) ----------
  * gh_patch_gram_fwd replaces, for all L collected feature maps of one discriminator in one launch,
  *   F.layer_norm(x_proj, x_proj.shape[1:])                  :198   (only when ln_input != 0; otherwise pass the
