@@ -41,6 +41,7 @@ _SIGNATURES = {
     "gh_maxpool2d_nhwc": (c_int, [_P, c_int, _P] + [c_int] * 7 + [_P]),
     "gh_stem_space_to_depth": (c_int, [_P] + [c_longlong] * 4 + [c_int] * 3 + [_P, c_int, _P]),
     "gh_stem_conv_pool_nhwc": (c_int, [_P] + [c_longlong] * 4 + [c_int] * 3 + [_P] * 4),
+    "gh_stem_conv_pool_u8_nhwc": (c_int, [_P] + [c_longlong] * 4 + [c_int] * 3 + [_P] * 6),
     "gh_patch_gram_workspace": (c_longlong, [c_int, c_int, c_int]),
     "gh_patch_gram_fwd": (c_int, [_P, _P, _P, _P, c_int, c_int, c_int, c_int, _P, _P, _P, _P]),
     "gh_patch_attn_fwd": (c_int, [_P] * 11 + [c_int] * 5 + [_P, _P, _P]),

@@ -512,6 +512,27 @@ __global__ void adaptive_pool_bwd_kernel(const float* __restrict__ d_desc, long 
   dG[(long long)b * C * C + idx] = s;
 }
 
+// Shared by the fp32 and uint8 entry points: p.x, p.w, p.bias, p.out (and p.mean / p.std) are set and checked.
+template <typename T>
+static int stem_conv_pool_launch(StemConvPoolParams<T>& p, long long img_stride, long long c_stride, long long y_stride,
+                                 long long x_stride, int B, int H, int W, void* stream) {
+  p.s_img = img_stride; p.s_c = c_stride; p.s_y = y_stride; p.s_x = x_stride;
+  p.B = B; p.OH = H / 2; p.OW = W / 2;
+  p.PH = (p.OH - 1) / 2 + 1;                                     // nn.MaxPool2d(3, 2, 1), floor mode
+  p.PW = (p.OW - 1) / 2 + 1;
+  p.tiles = (p.PW + kScTileCols - 1) / kScTileCols;
+  p.vec2 = x_stride == 1 && (uintptr_t)p.x % (2 * sizeof(T)) == 0 && (img_stride % 2 == 0) && (c_stride % 2 == 0) &&
+           (y_stride % 2 == 0);
+  p.units = (long long)B * p.tiles * p.PH;
+  const int sms = sm_count_cached();
+  const int grid = (int)(p.units < sms ? p.units : sms);
+  const uint32_t smem = sizeof(T) == 1 ? kScSmemBytesU8 : kScSmemBytes;
+  cudaError_t e = cudaFuncSetAttribute(stem_conv_pool_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return (int)e;
+  stem_conv_pool_kernel<T><<<grid, kScThreads, smem, (cudaStream_t)stream>>>(p);
+  return (int)cudaGetLastError();
+}
+
 }  // namespace gh
 
 using namespace gh;
@@ -817,22 +838,23 @@ int gh_stem_conv_pool_nhwc(const float* x, long long img_stride, long long c_str
                            void* stream) {
   if (!x || !w_packed || !bias || !out || B <= 0 || H <= 0 || W <= 0) return GH_ERR_BAD_ARG;
   if ((H & 1) || (W & 1) || (uintptr_t)w_packed % 16 != 0 || (uintptr_t)out % 16 != 0) return GH_ERR_UNSUPPORTED;
-  StemConvPoolParams p{};
-  p.x = x; p.s_img = img_stride; p.s_c = c_stride; p.s_y = y_stride; p.s_x = x_stride;
-  p.w = w_packed; p.bias = bias; p.out = out;
-  p.B = B; p.OH = H / 2; p.OW = W / 2;
-  p.PH = (p.OH - 1) / 2 + 1;                                     // nn.MaxPool2d(3, 2, 1), floor mode
-  p.PW = (p.OW - 1) / 2 + 1;
-  p.tiles = (p.PW + kScTileCols - 1) / kScTileCols;
-  p.vec2 = x_stride == 1 && (uintptr_t)x % 8 == 0 && (img_stride % 2 == 0) && (c_stride % 2 == 0) && (y_stride % 2 == 0);
-  p.units = (long long)B * p.tiles * p.PH;
-  const int sms = sm_count_cached();
-  const int grid = (int)(p.units < sms ? p.units : sms);
-  cudaError_t e = cudaFuncSetAttribute(stem_conv_pool_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       (int)kScSmemBytes);
-  if (e != cudaSuccess) return (int)e;
-  stem_conv_pool_kernel<<<grid, kScThreads, kScSmemBytes, (cudaStream_t)stream>>>(p);
-  return (int)cudaGetLastError();
+  StemConvPoolParams<float> p{};
+  p.x = x; p.w = w_packed; p.bias = bias; p.out = out;
+  return stem_conv_pool_launch(p, img_stride, c_stride, y_stride, x_stride, B, H, W, stream);
+}
+
+int gh_stem_conv_pool_u8_nhwc(const unsigned char* x, long long img_stride, long long c_stride, long long y_stride,
+                              long long x_stride, int B, int H, int W, const float* mean3_host, const float* std3_host,
+                              const float* w_packed, const float* bias, float* out, void* stream) {
+  if (!x || !mean3_host || !std3_host || !w_packed || !bias || !out || B <= 0 || H <= 0 || W <= 0) return GH_ERR_BAD_ARG;
+  StemConvPoolParams<uint8_t> p{};
+  for (int c = 0; c < 3; ++c) {
+    if (!(std3_host[c] != 0.f && std3_host[c] == std3_host[c])) return GH_ERR_BAD_ARG;     // zero or NaN std
+    p.mean[c] = mean3_host[c]; p.std[c] = std3_host[c];
+  }
+  if ((H & 1) || (W & 1) || (uintptr_t)w_packed % 16 != 0 || (uintptr_t)out % 16 != 0) return GH_ERR_UNSUPPORTED;
+  p.x = x; p.w = w_packed; p.bias = bias; p.out = out;
+  return stem_conv_pool_launch(p, img_stride, c_stride, y_stride, x_stride, B, H, W, stream);
 }
 
 int gh_gram_mse_blocks(long long n) {

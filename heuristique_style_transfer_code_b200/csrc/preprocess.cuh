@@ -100,6 +100,12 @@ struct NormalizeU8Params {
 
 constexpr int kNormUnroll = 8;
 
+// ToTensor (/255) then Normalize ((v - mean) / std) of the byte value t, IEEE fp32 with correctly rounded divisions: the
+// host's result. normalize_u8_kernel and the uint8 fused stem (stem.cuh) build their tables with it.
+__device__ __forceinline__ float to_tensor_normalize(unsigned t, float mean, float std) {
+  return __fdiv_rn(__fdiv_rn((float)t, 255.0f) - mean, std);
+}
+
 template <int VEC>
 __global__ void __launch_bounds__(256) normalize_u8_kernel(const NormalizeU8Params p) {
   __shared__ float table[256];
@@ -107,7 +113,7 @@ __global__ void __launch_bounds__(256) normalize_u8_kernel(const NormalizeU8Para
   const int c = (int)(blockIdx.x % (unsigned)p.C);
   const float m = c == 0 ? p.mean[0] : c == 1 ? p.mean[1] : c == 2 ? p.mean[2] : p.mean[3];
   const float s = c == 0 ? p.std[0] : c == 1 ? p.std[1] : c == 2 ? p.std[2] : p.std[3];
-  table[threadIdx.x] = __fdiv_rn(__fdiv_rn((float)threadIdx.x, 255.0f) - m, s);     // ToTensor, Normalize
+  table[threadIdx.x] = to_tensor_normalize(threadIdx.x, m, s);
   __syncthreads();
   const uint8_t* __restrict__ src = p.src + plane * p.hw;
   float* __restrict__ dst = p.dst + plane * p.hw;

@@ -29,8 +29,15 @@
 // Work split: persistent CTAs, one per SM, each a contiguous range of (image, tile, pooled row) units; the conv row above
 // a range's first pooled row is recomputed (halo). No atomics: an image's result does not depend on its batch.
 // Warps: 0-7 producers (one staged row each, round robin), 8-11 epilogue (TMEM lane quadrants 0-3), 12 MMA issuer.
+//
+// Pixel type: fp32 images, or the uint8 pixels of the loaders (functions.uint8_transform) with ToTensor + Normalize
+// applied in the producers (reference test_...:64-65, train_best_...:42-43). The uint8 kernel builds a [3][256] table
+// of to_tensor_normalize() results in shared memory -- the values gh_normalize_u8 writes -- and looks each byte up, so
+// its staged tf32 operands, and hence its output, are bitwise those of the fp32 kernel on the normalize_u8 batch.
+// Cells outside the image stay 0: conv1's zero padding applies after Normalize. Only the producers' loads differ.
 #pragma once
 #include "common.cuh"
+#include "preprocess.cuh"
 
 namespace gh {
 
@@ -53,16 +60,20 @@ constexpr uint32_t kScXbufOff = kScBiasOff + 64 * 4;
 constexpr uint32_t kScBarOff = kScXbufOff + 2 * 4 * 64 * 4;
 constexpr uint32_t kScBarBytes = 8 * (2 * kScSlots + 2 * kScAccSlots) + 16;
 constexpr uint32_t kScSmemBytes = kScBarOff + kScBarBytes + 1024;
+constexpr uint32_t kScTableOff = kScBarOff + kScBarBytes;        // uint8 pixels: [3][256] fp32 Normalize table
+constexpr uint32_t kScSmemBytesU8 = kScSmemBytes + 3 * 256 * 4;
 
+template <typename T>
 struct StemConvPoolParams {
-  const float* x;
+  const T* x;                          // float or uint8_t pixels
   long long s_img, s_c, s_y, s_x;      // element strides of x
   const float* w;                      // packed tf32 weights, the shared-memory image of the B operands (kScWBytes)
   const float* bias;                   // [64]
   float* out;                          // (B, PH, PW, 64)
   int B, OH, OW, PH, PW, tiles;        // conv size OH x OW = H/2 x W/2; pooled PH x PW; tiles per pooled row
-  int vec2;                            // x-contiguous pixel pairs 8 B aligned: float2 loads
+  int vec2;                            // x-contiguous pixel pairs 2 * sizeof(T) aligned: one load per pair
   long long units;                     // B * tiles * PH
+  float mean[3], std[3];               // uint8 pixels: Normalize's constants
 };
 
 __device__ __forceinline__ float max_nan(float a, float b) { return (b > a || b != b) ? b : a; }
@@ -72,7 +83,8 @@ __device__ __forceinline__ float max_nan(float a, float b) { return (b > a || b 
 struct ScSeg {
   int b, j, py0, py1, y_lo, y_hi;
 };
-__device__ __forceinline__ bool sc_next(const StemConvPoolParams& p, long long& u, long long u1, ScSeg& s) {
+template <typename T>
+__device__ __forceinline__ bool sc_next(const StemConvPoolParams<T>& p, long long& u, long long u1, ScSeg& s) {
   if (u >= u1) return false;
   const long long bj = u / p.PH;
   const long long end = (bj + 1) * p.PH < u1 ? (bj + 1) * p.PH : u1;
@@ -86,7 +98,32 @@ __device__ __forceinline__ bool sc_next(const StemConvPoolParams& p, long long& 
   return true;
 }
 
-__global__ void __launch_bounds__(kScThreads, 1) stem_conv_pool_kernel(const StemConvPoolParams p) {
+// The 2x2 pixel block {(2Y, 2X), (2Y, 2X+1), (2Y+1, 2X), (2Y+1, 2X+1)} of one channel at q, as the fp32 values the
+// convolution sees. table: the channel's 256 Normalize results (uint8 pixels only).
+__device__ __forceinline__ float4 sc_load_block(const StemConvPoolParams<float>& p, const float* q, const float*) {
+  if (p.vec2) {
+    const float2 t0 = __ldg(reinterpret_cast<const float2*>(q));
+    const float2 t1 = __ldg(reinterpret_cast<const float2*>(q + p.s_y));
+    return make_float4(t0.x, t0.y, t1.x, t1.y);
+  }
+  return make_float4(__ldg(q), __ldg(q + p.s_x), __ldg(q + p.s_y), __ldg(q + p.s_y + p.s_x));
+}
+
+__device__ __forceinline__ float4 sc_load_block(const StemConvPoolParams<uint8_t>& p, const uint8_t* q,
+                                                const float* table) {
+  uint32_t b0, b1, b2, b3;
+  if (p.vec2) {
+    const uint32_t t0 = __ldg(reinterpret_cast<const unsigned short*>(q));
+    const uint32_t t1 = __ldg(reinterpret_cast<const unsigned short*>(q + p.s_y));
+    b0 = t0 & 0xffu; b1 = t0 >> 8; b2 = t1 & 0xffu; b3 = t1 >> 8;
+  } else {
+    b0 = __ldg(q); b1 = __ldg(q + p.s_x); b2 = __ldg(q + p.s_y); b3 = __ldg(q + p.s_y + p.s_x);
+  }
+  return make_float4(table[b0], table[b1], table[b2], table[b3]);
+}
+
+template <typename T>
+__global__ void __launch_bounds__(kScThreads, 1) stem_conv_pool_kernel(const StemConvPoolParams<T> p) {
   extern __shared__ uint8_t smem_raw[];
   const uint32_t raw = smem_u32(smem_raw);
   const uint32_t base = (raw + 1023u) & ~1023u;
@@ -108,6 +145,14 @@ __global__ void __launch_bounds__(kScThreads, 1) stem_conv_pool_kernel(const Ste
     if (threadIdx.x < 64) reinterpret_cast<float*>(gbase + kScBiasOff)[threadIdx.x] = __ldg(p.bias + threadIdx.x);
     float4* z = reinterpret_cast<float4*>(gbase + kScAOff + 3 * kScPlaneBytes);
     for (int i = threadIdx.x; i < (int)(kScPlaneBytes / 16); i += kScThreads) z[i] = make_float4(0.f, 0.f, 0.f, 0.f);
+    if constexpr (sizeof(T) == 1) {
+      float* table = reinterpret_cast<float*>(gbase + kScTableOff);
+      for (int i = threadIdx.x; i < 3 * 256; i += kScThreads) {
+        const int c = i >> 8;
+        table[i] = to_tensor_normalize((unsigned)(i & 255), c == 0 ? p.mean[0] : c == 1 ? p.mean[1] : p.mean[2],
+                                       c == 0 ? p.std[0] : c == 1 ? p.std[1] : p.std[2]);
+      }
+    }
     fence_proxy_async_smem();
   }
   if (threadIdx.x == 0) {
@@ -136,7 +181,7 @@ __global__ void __launch_bounds__(kScThreads, 1) stem_conv_pool_kernel(const Ste
     ScSeg sg;
     while (sc_next(p, u, u1, sg)) {
       const int n_stage = sg.y_hi - sg.y_lo + 4;
-      const float* img = p.x + (long long)sg.b * p.s_img;
+      const T* img = p.x + (long long)sg.b * p.s_img;
       for (int k = 0; k < n_stage; ++k) {
         const uint32_t g = gs + (uint32_t)k;
         if ((int)(g % kScProducerWarps) != warp) continue;
@@ -151,14 +196,8 @@ __global__ void __launch_bounds__(kScThreads, 1) stem_conv_pool_kernel(const Ste
           const int X = kScTileCols * 2 * sg.j + s - 3;
           v[it] = make_float4(0.f, 0.f, 0.f, 0.f);
           if (i < kScItems && row_ok && X >= 0 && X < p.OW) {
-            const float* q = img + (long long)c * p.s_c + (long long)(2 * Y) * p.s_y + (long long)(2 * X) * p.s_x;
-            if (p.vec2) {
-              const float2 t0 = __ldg(reinterpret_cast<const float2*>(q));
-              const float2 t1 = __ldg(reinterpret_cast<const float2*>(q + p.s_y));
-              v[it] = make_float4(t0.x, t0.y, t1.x, t1.y);
-            } else {
-              v[it] = make_float4(__ldg(q), __ldg(q + p.s_x), __ldg(q + p.s_y), __ldg(q + p.s_y + p.s_x));
-            }
+            const T* q = img + (long long)c * p.s_c + (long long)(2 * Y) * p.s_y + (long long)(2 * X) * p.s_x;
+            v[it] = sc_load_block(p, q, reinterpret_cast<const float*>(gbase + kScTableOff) + c * 256);
           }
         }
         mbar_wait(bar_empty + 8 * slot, ((g / kScSlots) & 1u) ^ 1u, 300u + slot);

@@ -174,12 +174,20 @@ class FoldedEncoder:
             return ops.maxpool2d_nhwc(x, k, s, pad)
         return p(x)
 
-    def stem_forward(self, x: torch.Tensor) -> torch.Tensor:
+    def _fused_stem_applies(self, x: torch.Tensor) -> bool:
+        return (self.stem_packed is not None and self._stem_fused and torch.backends.cudnn.allow_tf32
+                and x.dim() == 4 and x.shape[1] == 3 and x.shape[2] % 2 == 0 and x.shape[3] % 2 == 0)
+
+    def stem_forward(self, x: torch.Tensor, normalize=None) -> torch.Tensor:
         """Children 0-3: conv1 + bn1 + relu + maxpool. One fused kernel (gh_stem_conv_pool_nhwc) when the chain below
-        would run in TF32 anyway (cudnn.allow_tf32, the torch default) on an fp32 plan; the chain otherwise."""
-        if (self.stem_packed is not None and self._stem_fused and torch.backends.cudnn.allow_tf32
-                and x.dtype == torch.float32 and x.dim() == 4 and x.shape[1] == 3 and x.shape[2] % 2 == 0
-                and x.shape[3] % 2 == 0):
+        would run in TF32 anyway (cudnn.allow_tf32, the torch default) on an fp32 plan; the chain otherwise.
+        normalize: (mean, std) for a uint8 batch, ToTensor + Normalize bit for bit as ops.normalize_u8 -- inside the
+        fused kernel where it applies (gh_stem_conv_pool_u8_nhwc: no fp32 batch), by normalize_u8 before the chain else."""
+        if normalize is not None and x.dtype == torch.uint8:
+            if self._fused_stem_applies(x):
+                return ops.stem_conv_pool_u8(x, *normalize, self.stem_packed, self.stem_s2d[1])
+            x = ops.normalize_u8(x, *normalize)
+        if x.dtype == torch.float32 and self._fused_stem_applies(x):
             return ops.stem_conv_pool(x, self.stem_packed, self.stem_s2d[1])
         if (self.stem_s2d is not None and x.dtype == torch.float32 and x.shape[1] == 3 and x.shape[2] % 2 == 0
                 and x.shape[3] % 2 == 0):
@@ -191,8 +199,8 @@ class FoldedEncoder:
             x = self._conv_relu(x, self.stem)
         return self._pool(x)
 
-    def __call__(self, x: torch.Tensor):
-        x = self.stem_forward(x)
+    def __call__(self, x: torch.Tensor, normalize=None):
+        x = self.stem_forward(x, normalize)
         outs = []
         for blocks in self.stages:
             for c1, c2, c3, down in blocks:

@@ -134,12 +134,7 @@ def _is_uint8_images(t):
     return torch.is_tensor(t) and t.dtype == torch.uint8 and t.dim() == 4 and 1 <= t.shape[1] <= 4
 
 
-def _normalize_host(t, mean, std):
-    """ToTensor's scaling + Normalize for a uint8 batch that stays on the host (CPU runs of the loops): the same op
-    sequence torchvision executes per image (to float32, div 255, sub mean, div std)."""
-    shape = (1, -1, 1, 1)
-    out = t.to(torch.float32).div_(255)
-    return out.sub_(torch.tensor(mean, dtype=torch.float32).view(shape)).div_(torch.tensor(std, dtype=torch.float32).view(shape))
+_normalize_host = ops.normalize_u8_host       # CPU runs of the loops; models with input normalisation use it too
 
 
 def cuda_prefetch(batches, device, reuse_buffers=False, normalize="default"):
@@ -297,6 +292,13 @@ class HostCollector:
         return out
 
 
+def _prefetch_normalize(model):
+    """cuda_prefetch's `normalize` for the loops: None when the model (or the one a DDP wrapper holds) normalises uint8
+    input itself (set_input_normalization), so that the pixels reach it; cuda_prefetch's default otherwise."""
+    inner = getattr(model, "module", model)
+    return None if getattr(inner, "input_normalization", None) is not None else "default"
+
+
 def train_model(model, train_loader, criterion, optimizer, num_epochs=25, writer=None, fold=0):
     """SGD loop of the train script (:123-145): per batch zero_grad / forward / loss / backward / step, a loss print per
     batch, the sample-weighted epoch loss printed and logged as Fold_{fold}/Train/Loss. Returns the model."""
@@ -306,7 +308,8 @@ def train_model(model, train_loader, criterion, optimizer, num_epochs=25, writer
     n_batches = len(train_loader)
     for epoch in range(num_epochs):
         running = 0.0
-        for step, (inputs, labels) in enumerate(cuda_prefetch(train_loader, device, reuse_buffers=True)):
+        for step, (inputs, labels) in enumerate(cuda_prefetch(train_loader, device, reuse_buffers=True,
+                                                              normalize=_prefetch_normalize(model))):
             optimizer.zero_grad()
             loss = criterion(model(inputs), labels)
             loss.backward()
@@ -393,7 +396,8 @@ def evaluate_model(model, val_loader, criterion, writer=None, fold=0):
     model.eval()
     results = HostCollector()
     with torch.no_grad():
-        for inputs, labels in cuda_prefetch(val_loader, device, reuse_buffers=True):
+        for inputs, labels in cuda_prefetch(val_loader, device, reuse_buffers=True,
+                                            normalize=_prefetch_normalize(model)):
             outputs = model(inputs)
             # the reference reads loss.item() and the predictions after every batch (:160-166); here they ride to the
             # host through the pinned ring and are reduced there afterwards, in the same order and precision
@@ -428,7 +432,8 @@ def evaluate_model_test(model, data_loader, device):
     dataset = data_loader.dataset
     results = HostCollector()
     with torch.no_grad():
-        for batch_idx, (inputs, labels) in enumerate(cuda_prefetch(data_loader, device, reuse_buffers=True)):
+        for batch_idx, (inputs, labels) in enumerate(cuda_prefetch(data_loader, device, reuse_buffers=True,
+                                                                   normalize=_prefetch_normalize(model))):
             embeddings, outputs = model(inputs)
             probs = F.softmax(outputs, dim=1)
             preds = outputs.argmax(dim=1)

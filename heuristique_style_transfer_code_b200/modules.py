@@ -62,6 +62,7 @@ class _TruncatedGramAttentionBase(nn.Module):
         self._backbone_mode = "reference"
         self.fold_batchnorm = os.environ.get("GRAMHEAD_FOLD_BN", "1") != "0"
         self._plan = None
+        self._input_normalization = None
         on_cuda = torch.device(self.device).type == "cuda"
         env_mode = os.environ.get("GRAMHEAD_BACKBONE", "")
         if env_mode or on_cuda:
@@ -78,6 +79,30 @@ class _TruncatedGramAttentionBase(nn.Module):
         fmt = torch.channels_last if mode.endswith("channels_last") else torch.contiguous_format
         self.truncated_encoder.to(memory_format=fmt)
         self._backbone_mode = mode
+        return self
+
+    @property
+    def input_normalization(self):
+        """((mean, mean, mean), (std, std, std)) applied to (B, 3, H, W) uint8 input, or None (the default)."""
+        return self._input_normalization
+
+    def set_input_normalization(self, mean, std=None):
+        """Lets forward() take the uint8 pixels of the loaders (functions.uint8_transform): a (B, 3, H, W) uint8 batch is
+        then transformed by ToTensor + Normalize(mean, std) first, bit for bit as ops.normalize_u8 / the host transforms
+        (reference test_...:64-65), so model(x_u8) == model(normalized x_u8). On the fp32 inference plan with the fused
+        stem this happens inside the stem kernel and no fp32 batch is built. Other input is unaffected.
+        set_input_normalization(None) turns it off. A plain attribute: no buffer, no state_dict key. Returns self."""
+        if mean is None:
+            if std is not None:
+                raise ValueError("set_input_normalization(None) takes no std")
+            self._input_normalization = None
+            return self
+        mean, std = tuple(float(v) for v in mean), tuple(float(v) for v in std)
+        if len(mean) != 3 or len(std) != 3:
+            raise ValueError(f"input normalisation needs 3 means and 3 stds, got {len(mean)} and {len(std)}")
+        if not all(s != 0.0 and s == s for s in std):
+            raise ValueError(f"input normalisation: std must be non-zero, got {std}")
+        self._input_normalization = (mean, std)
         return self
 
     def gram_matrix(self, activations):
@@ -124,9 +149,14 @@ class _TruncatedGramAttentionBase(nn.Module):
 
     def _stage_activations(self, x):
         x = x.to(self.device)
+        norm = self._input_normalization
+        if norm is not None and not (x.dtype == torch.uint8 and x.dim() == 4 and x.shape[1] == 3):
+            norm = None
         plan = self._inference_plan(x)
         if plan is not None:
-            return plan(x)
+            return plan(x, normalize=norm)
+        if norm is not None:
+            x = ops.normalize_u8(x, *norm) if x.is_cuda else ops.normalize_u8_host(x, *norm)
         if self._backbone_mode == "reference":
             return self._run_encoder(x)
         if self._backbone_mode.endswith("channels_last"):

@@ -319,6 +319,41 @@ def stem_conv_pool(x: torch.Tensor, packed_weight: torch.Tensor, bias: torch.Ten
     return out
 
 
+def stem_conv_pool_u8(x: torch.Tensor, mean, std, packed_weight: torch.Tensor, bias: torch.Tensor) -> torch.Tensor:
+    """stem_conv_pool(normalize_u8(x, mean, std), packed_weight, bias) bit for bit, in one kernel that reads the (B, 3, H, W)
+    uint8 pixels (any strides, H and W even) and never builds the fp32 batch (gh_stem_conv_pool_u8_nhwc)."""
+    _require_cuda(x, "x")
+    if x.dim() != 4 or x.shape[1] != 3 or x.dtype != torch.uint8 or x.shape[2] % 2 or x.shape[3] % 2:
+        raise GramHeadError("gramhead: stem_conv_pool_u8 takes uint8 (B, 3, H, W) images with even H and W")
+    if (packed_weight.dtype != torch.float32 or packed_weight.numel() != 16384 or not packed_weight.is_contiguous()
+            or bias.dtype != torch.float32 or bias.numel() != 64 or not bias.is_contiguous()
+            or packed_weight.device != x.device or bias.device != x.device):
+        raise GramHeadError("gramhead: stem_conv_pool_u8 takes the packed fp32 stem weights (16384) and bias (64) on x's device")
+    mean, std = [float(v) for v in mean], [float(v) for v in std]
+    if len(mean) != 3 or len(std) != 3:
+        raise GramHeadError("gramhead: stem_conv_pool_u8: 3 channels need 3 means and stds")
+    b, _, h, w = x.shape
+    oh, ow = h // 2, w // 2
+    ph, pw = (oh - 1) // 2 + 1, (ow - 1) // 2 + 1
+    out = torch.empty((b, 64, ph, pw), device=x.device, dtype=torch.float32, memory_format=torch.channels_last)
+    fl = ctypes.c_float * 3
+    work = dict(bytes=x.numel() + out.numel() * 4, flops=2 * b * oh * ow * 64 * 147, kind="stem_conv_pool")
+    with torch.cuda.device(x.device), _Timed(f"stem_conv_pool_u8[HW={h}x{w}]", 1, x.device, **work):
+        rc = _lib.lib().gh_stem_conv_pool_u8_nhwc(x.data_ptr(), x.stride(0), x.stride(1), x.stride(2), x.stride(3), b, h,
+                                                  w, fl(*mean), fl(*std), packed_weight.data_ptr(), bias.data_ptr(),
+                                                  out.data_ptr(), _stream_ptr(x))
+    check(rc, "gh_stem_conv_pool_u8_nhwc")
+    return out
+
+
+def normalize_u8_host(t: torch.Tensor, mean, std) -> torch.Tensor:
+    """ToTensor's scaling + Normalize for a uint8 batch that stays on the host (CPU runs): the same op sequence
+    torchvision executes per image (to float32, div 255, sub mean, div std)."""
+    shape = (1, -1, 1, 1)
+    out = t.to(torch.float32).div_(255)
+    return out.sub_(torch.tensor(mean, dtype=torch.float32).view(shape)).div_(torch.tensor(std, dtype=torch.float32).view(shape))
+
+
 def normalize_u8(x: torch.Tensor, mean, std, out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """(B, C, H, W) uint8 pixels on the device -> the fp32 batch transforms.ToTensor() + transforms.Normalize(mean, std)
     produce on the host (reference test_RESNET50_Truncate_gram_attention.py:64-65), bit for bit (gh_normalize_u8).

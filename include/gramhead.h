@@ -194,6 +194,18 @@ int gh_stem_conv_pool_nhwc(const float* x, long long img_stride, long long c_str
                            long long x_stride, int B, int H, int W, const float* w_packed, const float* bias, float* out,
                            void* stream);
 
+/* gh_stem_conv_pool_nhwc on the uint8 pixels of the loaders (functions.uint8_transform) with ToTensor + Normalize
+ * applied inside it -- the transforms of the reference's loaders, test_RESNET50_Truncate_gram_attention.py:64-65 and
+ * train_best_RESNET50_Truncate_gram_attention.py:42-43, in front of the stem, children 0-3 of `self.truncated_encoder`,
+ * Models/Models_RESNET50_TRUNCATE_GRAM_with_Attention.py:17,37-40 -- in place of gh_normalize_u8 followed by
+ * gh_stem_conv_pool_nhwc, without the fp32 batch. Each pixel becomes (float(b) / 255 - mean[c]) / std[c] exactly as in
+ * gh_normalize_u8, so `out` is bit for bit what those two calls produce. x: uint8 (B, 3, H, W) with the given element
+ * strides; zero padding applies after Normalize. mean3_host / std3_host: HOST pointers to 3 floats each (std neither
+ * zero nor NaN: GH_ERR_BAD_ARG). w_packed, bias, out, H, W: as for gh_stem_conv_pool_nhwc. */
+int gh_stem_conv_pool_u8_nhwc(const unsigned char* x, long long img_stride, long long c_stride, long long y_stride,
+                              long long x_stride, int B, int H, int W, const float* mean3_host, const float* std3_host,
+                              const float* w_packed, const float* bias, float* out, void* stream);
+
 /* ---- Gram head of the Multi-PatchGAN discriminator (the *_test classes of Models/Models_Multi_PatchGAN.py) ----------
  * gh_patch_gram_fwd replaces, for all L collected feature maps of one discriminator in one launch,
  *   F.layer_norm(x_proj, x_proj.shape[1:])                  :198   (only when ln_input != 0; otherwise pass the
