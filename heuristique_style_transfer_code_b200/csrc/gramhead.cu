@@ -523,9 +523,11 @@ static int stem_conv_pool_launch(StemConvPoolParams<T>& p, long long img_stride,
   p.tiles = (p.PW + kScTileCols - 1) / kScTileCols;
   p.vec2 = x_stride == 1 && (uintptr_t)p.x % (2 * sizeof(T)) == 0 && (img_stride % 2 == 0) && (c_stride % 2 == 0) &&
            (y_stride % 2 == 0);
-  p.units = (long long)B * p.tiles * p.PH;
+  const long long units = (long long)B * p.tiles * p.PH;
+  if (units >= (1ll << 30)) return GH_ERR_UNSUPPORTED;          // 256 B of output per unit: 256 GB, more than any GPU
+  p.units = (int)units;
   const int sms = sm_count_cached();
-  const int grid = (int)(p.units < sms ? p.units : sms);
+  const int grid = p.units < sms ? p.units : sms;
   const uint32_t smem = sizeof(T) == 1 ? kScSmemBytesU8 : kScSmemBytes;
   cudaError_t e = cudaFuncSetAttribute(stem_conv_pool_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return (int)e;
@@ -550,6 +552,17 @@ int gh_bp_profile_read(unsigned long long* out) {
   cudaError_t e = cudaDeviceSynchronize();
   if (e == cudaSuccess) e = cudaMemcpyFromSymbol(out, g_bp_prof, sizeof(zero));
   if (e == cudaSuccess) e = cudaMemcpyToSymbol(g_bp_prof, zero, sizeof(zero));
+  return (int)e;
+}
+#endif
+
+#ifdef GH_SC_PROFILE
+// Profile builds only (not part of include/gramhead.h): copies the 16 role counters of stem_conv_pool_kernel and clears them.
+int gh_sc_profile_read(unsigned long long* out) {
+  unsigned long long zero[16] = {0};
+  cudaError_t e = cudaDeviceSynchronize();
+  if (e == cudaSuccess) e = cudaMemcpyFromSymbol(out, g_sc_prof, sizeof(zero));
+  if (e == cudaSuccess) e = cudaMemcpyToSymbol(g_sc_prof, zero, sizeof(zero));
   return (int)e;
 }
 #endif

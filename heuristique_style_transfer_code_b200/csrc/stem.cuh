@@ -11,10 +11,12 @@
 // x[c][2Y+1][2X], x[c][2Y+1][2X+1]} -- a 16-byte "k-chunk" -- and a zero 4th chunk (12 channels padded to 16).
 //
 // Implicit GEMM by descriptor shift. M = 128 consecutive conv columns of one conv row, N = 64 output channels, K = 16
-// taps x 16. The staged image rows live in shared memory K-major without swizzle as [k-chunk plane][row slot][cell][16 B]:
-// one core matrix is 8 consecutive cells (SBO = 128 B between 8-cell groups), the two k-chunks of one tf32 MMA (K = 8)
-// are two planes (LBO = plane stride). Tap (a, b) of the tile is then the same staged rows with the descriptor start moved
-// to row slot y + a and 16 B per cell of b: 16 taps x 2 MMAs of 128 x 64 x 8, no im2col copy.
+// taps x 12 (the zero 4th k-chunk is never multiplied). The staged image rows live in shared memory K-major without
+// swizzle as [k-chunk plane 0..2][row slot][cell][16 B]: one core matrix is 8 consecutive cells (SBO = 128 B between
+// 8-cell groups). Tap (a, b) of the tile is the same staged rows with the descriptor start moved to row slot y + a and
+// 16 B per cell of b, so there is no im2col copy. Per tap row a, six tf32 MMAs of 128 x 64 x 8: one per tap b for
+// k-chunks 0 and 1 (planes 0 and 1, LBO = plane stride), and one per tap pair (b, b + 1) = (0, 1), (2, 3) for k-chunk 2
+// (plane 2 at cell b, LBO = 16 B: the second "k-chunk" of the MMA is the next cell, i.e. tap b + 1). 24 MMAs per conv row.
 //
 // Tiles: 63 pooled columns per tile need the 127 conv columns 126 j - 1 .. 126 j + 125 (lane l = column 126 j - 1 + l),
 // i.e. staged cells 126 j - 1 .. 126 j + 129 of each padded row (131 cells). 224^2 is one tile per row (lanes with no
@@ -28,7 +30,8 @@
 //
 // Work split: persistent CTAs, one per SM, each a contiguous range of (image, tile, pooled row) units; the conv row above
 // a range's first pooled row is recomputed (halo). No atomics: an image's result does not depend on its batch.
-// Warps: 0-7 producers (one staged row each, round robin), 8-11 epilogue (TMEM lane quadrants 0-3), 12 MMA issuer.
+// Warps: 0-6 producers (one staged row each, round robin), 7-14 epilogue (TMEM lane quadrant warp % 4, output channel
+// half (warp - 7) / 4), 15 MMA issuer: 16 warps, so that each thread may hold 128 registers.
 //
 // Pixel type: fp32 images, or the uint8 pixels of the loaders (functions.uint8_transform) with ToTensor + Normalize
 // applied in the producers (reference test_...:64-65, train_best_...:42-43). The uint8 kernel builds a [3][256] table
@@ -41,10 +44,11 @@
 
 namespace gh {
 
-constexpr int kScProducerWarps = 8;
-constexpr int kScEpiWarp0 = 8;
-constexpr int kScMmaWarp = 12;
-constexpr int kScThreads = 13 * 32;
+constexpr int kScProducerWarps = 7;
+constexpr int kScEpiWarp0 = kScProducerWarps;
+constexpr int kScEpiWarps = 8;                         // two per TMEM lane quadrant, 32 output channels each
+constexpr int kScMmaWarp = kScEpiWarp0 + kScEpiWarps;
+constexpr int kScThreads = (kScMmaWarp + 1) * 32;
 constexpr int kScTileCols = 63;                        // pooled columns per tile
 constexpr int kScCells = 131;                          // staged cells per row slot
 constexpr int kScItems = 3 * kScCells;                 // (image channel, cell) k-chunks a producer warp stores per row
@@ -55,7 +59,7 @@ constexpr uint32_t kScSlotBytes = kScCells * 16;       // 2096
 constexpr uint32_t kScPlaneBytes = kScSlots * kScSlotBytes;
 constexpr uint32_t kScWBytes = 16 * 2 * 2048;          // 16 taps x 2 MMAs x (64 rows x 2 k-chunks x 16 B)
 constexpr uint32_t kScAOff = kScWBytes;
-constexpr uint32_t kScBiasOff = kScAOff + 4 * kScPlaneBytes;
+constexpr uint32_t kScBiasOff = kScAOff + 3 * kScPlaneBytes;
 constexpr uint32_t kScXbufOff = kScBiasOff + 64 * 4;
 constexpr uint32_t kScBarOff = kScXbufOff + 2 * 4 * 64 * 4;
 constexpr uint32_t kScBarBytes = 8 * (2 * kScSlots + 2 * kScAccSlots) + 16;
@@ -72,11 +76,38 @@ struct StemConvPoolParams {
   float* out;                          // (B, PH, PW, 64)
   int B, OH, OW, PH, PW, tiles;        // conv size OH x OW = H/2 x W/2; pooled PH x PW; tiles per pooled row
   int vec2;                            // x-contiguous pixel pairs 2 * sizeof(T) aligned: one load per pair
-  long long units;                     // B * tiles * PH
+  int units;                           // B * tiles * PH (the launcher keeps it below 2^30)
   float mean[3], std[3];               // uint8 pixels: Normalize's constants
 };
 
-__device__ __forceinline__ float max_nan(float a, float b) { return (b > a || b != b) ? b : a; }
+// -DGH_SC_PROFILE: per-role cycle accounting (clock64 around every mbarrier wait, the TMEM loads, the epilogue's
+// bar.sync and the store phase of one thread per role, summed over the CTAs into g_sc_prof and read back by
+// gh_sc_profile_read; tools/prof_stem_roles.py). Slots: 0 issuer loop, 1 issuer wait aempty, 2 issuer wait full,
+// 3 conv rows issued, 4 producer (warp 0) loop, 5 producer wait empty, 6 producer store phase (wait for its loads,
+// cvt, STS, arrive), 7 rows staged by warp 0, 8 epilogue (warp kScEpiWarp0) loop, 9 epilogue wait afull, 10 epilogue
+// TMEM loads and row max, 11 epilogue bar.sync, 12 epilogue column max + store, 13 pooled rows, 14 CTAs,
+// 15 CTA lifetime (thread 0, prologue included).
+#ifdef GH_SC_PROFILE
+__device__ unsigned long long g_sc_prof[16];
+#define GH_SC_DECL(var) long long var = 0
+#define GH_SC_CLK(var) const long long var = clock64()
+#define GH_SC_ADD(acc, var) acc += clock64() - var
+#define GH_SC_FLUSH(slot, acc) atomicAdd(&g_sc_prof[slot], (unsigned long long)(acc))
+#define GH_SC_INC(var) ++var
+#else
+#define GH_SC_DECL(var)
+#define GH_SC_CLK(var)
+#define GH_SC_ADD(acc, var)
+#define GH_SC_FLUSH(slot, acc)
+#define GH_SC_INC(var)
+#endif
+
+// max that propagates NaN (one FMNMX.NAN): a NaN operand gives a NaN, as in nn.MaxPool2d and torch.relu.
+__device__ __forceinline__ float max_nan(float a, float b) {
+  float r;
+  asm("max.NaN.f32 %0, %1, %2;" : "=f"(r) : "f"(a), "f"(b));
+  return r;
+}
 
 // A CTA's range of units, cut where (image, tile) changes: one segment = consecutive pooled rows py0..py1-1 of one
 // (image, tile), computed from conv rows y_lo..y_hi, staged from padded rows y_lo..y_hi + 3.
@@ -84,14 +115,14 @@ struct ScSeg {
   int b, j, py0, py1, y_lo, y_hi;
 };
 template <typename T>
-__device__ __forceinline__ bool sc_next(const StemConvPoolParams<T>& p, long long& u, long long u1, ScSeg& s) {
+__device__ __forceinline__ bool sc_next(const StemConvPoolParams<T>& p, int& u, int u1, ScSeg& s) {
   if (u >= u1) return false;
-  const long long bj = u / p.PH;
-  const long long end = (bj + 1) * p.PH < u1 ? (bj + 1) * p.PH : u1;
-  s.b = (int)(bj / p.tiles);
-  s.j = (int)(bj - (long long)s.b * p.tiles);
-  s.py0 = (int)(u - bj * p.PH);
-  s.py1 = s.py0 + (int)(end - u);
+  const int bj = u / p.PH;
+  const int end = (bj + 1) * p.PH < u1 ? (bj + 1) * p.PH : u1;
+  s.b = bj / p.tiles;
+  s.j = bj - s.b * p.tiles;
+  s.py0 = u - bj * p.PH;
+  s.py1 = s.py0 + (end - u);
   s.y_lo = 2 * s.py0 - 1 > 0 ? 2 * s.py0 - 1 : 0;
   s.y_hi = 2 * s.py1 - 1 < p.OH - 1 ? 2 * s.py1 - 1 : p.OH - 1;
   u = end;
@@ -124,6 +155,7 @@ __device__ __forceinline__ float4 sc_load_block(const StemConvPoolParams<uint8_t
 
 template <typename T>
 __global__ void __launch_bounds__(kScThreads, 1) stem_conv_pool_kernel(const StemConvPoolParams<T> p) {
+  GH_SC_CLK(prof_cta0);
   extern __shared__ uint8_t smem_raw[];
   const uint32_t raw = smem_u32(smem_raw);
   const uint32_t base = (raw + 1023u) & ~1023u;
@@ -137,14 +169,12 @@ __global__ void __launch_bounds__(kScThreads, 1) stem_conv_pool_kernel(const Ste
   volatile uint32_t* tmem_slot_ptr = reinterpret_cast<volatile uint32_t*>(gbase + (tmem_slot - base));
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 
-  // Weights and bias for the CTA's life; plane 3 (the zero k-chunk of every cell) once.
+  // Weights and bias for the CTA's life.
   {
     const float4* wg = reinterpret_cast<const float4*>(p.w);
     float4* ws = reinterpret_cast<float4*>(gbase);
     for (int i = threadIdx.x; i < (int)(kScWBytes / 16); i += kScThreads) ws[i] = __ldg(wg + i);
     if (threadIdx.x < 64) reinterpret_cast<float*>(gbase + kScBiasOff)[threadIdx.x] = __ldg(p.bias + threadIdx.x);
-    float4* z = reinterpret_cast<float4*>(gbase + kScAOff + 3 * kScPlaneBytes);
-    for (int i = threadIdx.x; i < (int)(kScPlaneBytes / 16); i += kScThreads) z[i] = make_float4(0.f, 0.f, 0.f, 0.f);
     if constexpr (sizeof(T) == 1) {
       float* table = reinterpret_cast<float*>(gbase + kScTableOff);
       for (int i = threadIdx.x; i < 3 * 256; i += kScThreads) {
@@ -162,7 +192,7 @@ __global__ void __launch_bounds__(kScThreads, 1) stem_conv_pool_kernel(const Ste
     }
     for (int s = 0; s < kScAccSlots; ++s) {
       mbar_init(bar_afull + 8 * s, 1);
-      mbar_init(bar_aempty + 8 * s, 4);
+      mbar_init(bar_aempty + 8 * s, kScEpiWarps);
     }
     mbar_fence_init();
   }
@@ -172,13 +202,18 @@ __global__ void __launch_bounds__(kScThreads, 1) stem_conv_pool_kernel(const Ste
   tc_fence_after_sync();
   const uint32_t tmem_base = *tmem_slot_ptr;
 
-  const long long u0 = p.units * blockIdx.x / gridDim.x, u1 = p.units * (blockIdx.x + 1) / gridDim.x;
+  const int u0 = (int)((long long)p.units * blockIdx.x / gridDim.x);
+  const int u1 = (int)((long long)p.units * (blockIdx.x + 1) / gridDim.x);
 
   if (warp < kScProducerWarps) {
     // =========================== producers: one padded s2d row per warp, round robin ===========================
     uint32_t gs = 0;                                   // staged rows so far (all segments)
-    long long u = u0;
+    int u = u0;
     ScSeg sg;
+    GH_SC_DECL(prof_wait);
+    GH_SC_DECL(prof_store);
+    GH_SC_DECL(prof_n);
+    GH_SC_CLK(prof_t0);
     while (sc_next(p, u, u1, sg)) {
       const int n_stage = sg.y_hi - sg.y_lo + 4;
       const T* img = p.x + (long long)sg.b * p.s_img;
@@ -200,7 +235,11 @@ __global__ void __launch_bounds__(kScThreads, 1) stem_conv_pool_kernel(const Ste
             v[it] = sc_load_block(p, q, reinterpret_cast<const float*>(gbase + kScTableOff) + c * 256);
           }
         }
+        GH_SC_CLK(prof_w0);
         mbar_wait(bar_empty + 8 * slot, ((g / kScSlots) & 1u) ^ 1u, 300u + slot);
+        GH_SC_ADD(prof_wait, prof_w0);
+        GH_SC_CLK(prof_s0);
+        GH_SC_INC(prof_n);
 #pragma unroll
         for (int it = 0; it < kScItemIters; ++it) {
           const int i = it * 32 + lane;
@@ -213,23 +252,44 @@ __global__ void __launch_bounds__(kScThreads, 1) stem_conv_pool_kernel(const Ste
         fence_proxy_async_smem();
         __syncwarp();
         if (lane == 0) mbar_arrive(bar_full + 8 * slot);
+        GH_SC_ADD(prof_store, prof_s0);
       }
       gs += (uint32_t)n_stage;
     }
+#ifdef GH_SC_PROFILE
+    if (warp == 0 && lane == 0) {
+      long long prof_tot = 0;
+      GH_SC_ADD(prof_tot, prof_t0);
+      GH_SC_FLUSH(4, prof_tot);
+      GH_SC_FLUSH(5, prof_wait);
+      GH_SC_FLUSH(6, prof_store);
+      GH_SC_FLUSH(7, prof_n);
+    }
+#endif
   } else if (warp == kScMmaWarp) {
     // =========================== MMA issuer ===========================
     constexpr uint32_t idesc = make_idesc_tf32(128, 64);
-    // k-chunks (0, 1) of the cells are planes 0 and 1 (LBO = one plane); the second MMA of a tap starts 2 planes on
+    // k-chunks (0, 1) of a tap: planes 0 and 1 (LBO = one plane) against packed [a][b][h=0][q=0..1] (LBO = 1024 B).
+    // k-chunk 2 of the taps b and b + 1: cells b and b + 1 of plane 2 (LBO = 16 B, one cell; the last cell read is
+    // 127 + 2 + 1 = 130 < kScCells) against packed [a][b][1][0] and [a][b + 1][1][0] (LBO = 4096 B, one tap).
     const uint64_t adesc0 = make_smem_desc_noswz(a_smem, kScPlaneBytes, 128);
     const uint64_t bdesc0 = make_smem_desc_noswz(w_smem, 1024, 128);
+    const uint64_t adesc2 = make_smem_desc_noswz(a_smem + 2 * kScPlaneBytes, 16, 128);
+    const uint64_t bdesc2 = make_smem_desc_noswz(w_smem + 2048, 4096, 128);
     uint32_t gs = 0, gc = 0;
-    long long u = u0;
+    int u = u0;
     ScSeg sg;
+    GH_SC_DECL(prof_ae);
+    GH_SC_DECL(prof_full);
+    GH_SC_CLK(prof_t0);
     while (sc_next(p, u, u1, sg)) {
       const int n_conv = sg.y_hi - sg.y_lo + 1;
       for (int k = 0; k < n_conv; ++k, ++gc) {
         const uint32_t acc = gc % kScAccSlots;
+        GH_SC_CLK(prof_w0);
         mbar_wait(bar_aempty + 8 * acc, ((gc / kScAccSlots) & 1u) ^ 1u, 400u + acc);
+        GH_SC_ADD(prof_ae, prof_w0);
+        GH_SC_CLK(prof_w1);
         uint32_t slot[4];
 #pragma unroll
         for (int a = 0; a < 4; ++a) {
@@ -237,20 +297,19 @@ __global__ void __launch_bounds__(kScThreads, 1) stem_conv_pool_kernel(const Ste
           slot[a] = g % kScSlots;
           mbar_wait(bar_full + 8 * slot[a], (g / kScSlots) & 1u, 500u + slot[a]);
         }
+        GH_SC_ADD(prof_full, prof_w1);
         tc_fence_after_sync();
         if (elect_one()) {
           const uint32_t d = tmem_base + acc * 64u;
 #pragma unroll
           for (int a = 0; a < 4; ++a) {
-            const uint64_t arow = adesc0 + ((slot[a] * kScSlotBytes) >> 4);
+            const uint32_t row = (slot[a] * kScSlotBytes) >> 4;
 #pragma unroll
             for (int b = 0; b < 4; ++b)
+              umma_tf32(d, adesc0 + row + b, bdesc0 + (((a * 4 + b) * 2 * 2048) >> 4), idesc, (a | b) != 0);
 #pragma unroll
-              for (int h = 0; h < 2; ++h) {
-                const uint64_t da = arow + ((b * 16 + h * 2 * kScPlaneBytes) >> 4);
-                const uint64_t db = bdesc0 + ((((a * 4 + b) * 2 + h) * 2048) >> 4);
-                umma_tf32(d, da, db, idesc, (a | b | h) != 0);
-              }
+            for (int b = 0; b < 4; b += 2)
+              umma_tf32(d, adesc2 + row + b, bdesc2 + (((a * 4 + b) * 2 * 2048) >> 4), idesc, 1u);
           }
           umma_commit(bar_afull + 8 * acc);
           umma_commit(bar_empty + 8 * slot[0]);        // padded row y is not read by conv rows below y
@@ -261,14 +320,34 @@ __global__ void __launch_bounds__(kScThreads, 1) stem_conv_pool_kernel(const Ste
       }
       gs += (uint32_t)(n_conv + 3);
     }
+#ifdef GH_SC_PROFILE
+    if (lane == 0) {
+      long long prof_tot = 0;
+      GH_SC_ADD(prof_tot, prof_t0);
+      GH_SC_FLUSH(0, prof_tot);
+      GH_SC_FLUSH(1, prof_ae);
+      GH_SC_FLUSH(2, prof_full);
+      GH_SC_FLUSH(3, gc);
+    }
+#endif
   } else {
     // =========================== epilogue: TMEM -> 3x3/s2 max -> + bias, ReLU -> NHWC ===========================
-    const int quad = warp - kScEpiWarp0;
-    const uint32_t tlane = tmem_base + ((uint32_t)(32 * quad) << 16);
+    // A warp reads TMEM lane quadrant warp % 4 (the quadrant a warp may access) and output channels 32 half .. + 31.
+    // A window's rows are loaded back to back and waited for once; the window's last row is kept in registers as the
+    // next window's first row, so each conv row leaves TMEM once and its accumulator is released as soon as it is read.
+    const int quad = warp & 3, half = (warp - kScEpiWarp0) >> 2;
+    const uint32_t tlane = tmem_base + ((uint32_t)(32 * quad) << 16) + 32u * (uint32_t)half;
+    const float* bias_h = bias_s + 32 * half;
     const float neg_inf = -__int_as_float(0x7f800000);
     uint32_t gc = 0, xb = 0;
-    long long u = u0;
+    int u = u0;
     ScSeg sg;
+    GH_SC_DECL(prof_af);
+    GH_SC_DECL(prof_ld);
+    GH_SC_DECL(prof_bar);
+    GH_SC_DECL(prof_st);
+    GH_SC_DECL(prof_n);
+    GH_SC_CLK(prof_t0);
     while (sc_next(p, u, u1, sg)) {
       const int x = kScTileCols * 2 * sg.j - 1 + 32 * quad + lane;     // this lane's conv column
       const bool col_ok = x >= 0 && x < p.OW;
@@ -277,76 +356,89 @@ __global__ void __launch_bounds__(kScThreads, 1) stem_conv_pool_kernel(const Ste
         const uint32_t g = gc + (uint32_t)(y - sg.y_lo);
         mbar_wait(bar_afull + 8 * (g % kScAccSlots), (g / kScAccSlots) & 1u, 600u + g % kScAccSlots);
       };
+      uint32_t ra[32];                                                 // conv row 2 py - 1 of the current window
       for (int py = sg.py0; py < sg.py1; ++py) {
         const int ya = 2 * py - 1, yb = 2 * py, yc = 2 * py + 1;
-        const bool ha = ya >= sg.y_lo, hc = yc <= sg.y_hi;
-        if (py == sg.py0 && ha) wait_row(ya);
+        const bool ha = ya >= sg.y_lo, hc = yc <= sg.y_hi, first = py == sg.py0;
+        GH_SC_CLK(prof_w0);
+        if (first && ha) wait_row(ya);
         wait_row(yb);
         if (hc) wait_row(yc);
+        GH_SC_ADD(prof_af, prof_w0);
+        GH_SC_CLK(prof_l0);
+        GH_SC_INC(prof_n);
         tc_fence_after_sync();
-        float m[64];
-#pragma unroll
-        for (int h = 0; h < 2; ++h) {
-          uint32_t r[32];
-          tmem_ld32_nowait(tlane + acc_of(yb) * 64u + 32u * h, r);
-          tmem_ld_wait();
-#pragma unroll
-          for (int i = 0; i < 32; ++i) m[32 * h + i] = __uint_as_float(r[i]);
-          if (ha) {
-            tmem_ld32_nowait(tlane + acc_of(ya) * 64u + 32u * h, r);
-            tmem_ld_wait();
-#pragma unroll
-            for (int i = 0; i < 32; ++i) m[32 * h + i] = max_nan(m[32 * h + i], __uint_as_float(r[i]));
-          }
-          if (hc) {
-            tmem_ld32_nowait(tlane + acc_of(yc) * 64u + 32u * h, r);
-            tmem_ld_wait();
-#pragma unroll
-            for (int i = 0; i < 32; ++i) m[32 * h + i] = max_nan(m[32 * h + i], __uint_as_float(r[i]));
-          }
-        }
-        // rows ya and yb are done; yc is the next window's first row unless the segment ends here
+        uint32_t rb[32], rc[32];
+        if (first && ha) tmem_ld32_nowait(tlane + acc_of(ya) * 64u, ra);
+        tmem_ld32_nowait(tlane + acc_of(yb) * 64u, rb);
+        if (hc) tmem_ld32_nowait(tlane + acc_of(yc) * 64u, rc);
+        tmem_ld_wait();
         tc_fence_before_sync();
         __syncwarp();
         if (lane == 0) {
-          if (ha) mbar_arrive(bar_aempty + 8 * acc_of(ya));
+          if (first && ha) mbar_arrive(bar_aempty + 8 * acc_of(ya));
           mbar_arrive(bar_aempty + 8 * acc_of(yb));
-          if (hc && py == sg.py1 - 1) mbar_arrive(bar_aempty + 8 * acc_of(yc));
+          if (hc) mbar_arrive(bar_aempty + 8 * acc_of(yc));
         }
+        float m[32];
+#pragma unroll
+        for (int i = 0; i < 32; ++i) {
+          m[i] = __uint_as_float(rb[i]);
+          if (ha) m[i] = max_nan(m[i], __uint_as_float(ra[i]));
+          if (hc) m[i] = max_nan(m[i], __uint_as_float(rc[i]));
+          ra[i] = rc[i];
+        }
+        GH_SC_ADD(prof_ld, prof_l0);
         if (!col_ok) {
 #pragma unroll
-          for (int i = 0; i < 64; ++i) m[i] = neg_inf;
+          for (int i = 0; i < 32; ++i) m[i] = neg_inf;
         }
         // column x + 2 of lane 30 is lane 0 of the next quadrant
-        float* xs = xbuf + xb * 256;
+        float* xs = xbuf + xb * 256 + 32 * half;
         if (lane == 0 && quad > 0) {
 #pragma unroll
-          for (int i = 0; i < 64; i += 4)
+          for (int i = 0; i < 32; i += 4)
             *reinterpret_cast<float4*>(xs + quad * 64 + i) = make_float4(m[i], m[i + 1], m[i + 2], m[i + 3]);
         }
-        asm volatile("bar.sync 1, 128;" ::: "memory");
+        GH_SC_CLK(prof_b0);
+        asm volatile("bar.sync %0, 128;" ::"r"(1 + half) : "memory");   // the four warps of this channel half
+        GH_SC_ADD(prof_bar, prof_b0);
+        GH_SC_CLK(prof_s0);
         const bool from_next = lane == 30 && quad < 3;
         const int qx = 16 * quad + (lane >> 1);                         // pooled column within the tile
         const int px = kScTileCols * sg.j + qx;
         const bool store = !(lane & 1) && qx < kScTileCols && px < p.PW;
-        float4* o = reinterpret_cast<float4*>(p.out + (((long long)sg.b * p.PH + py) * p.PW + px) * 64);
+        float4* o = reinterpret_cast<float4*>(p.out + (((long long)sg.b * p.PH + py) * p.PW + px) * 64 + 32 * half);
 #pragma unroll
-        for (int i = 0; i < 64; i += 4) {
+        for (int i = 0; i < 32; i += 4) {
           float r4[4];
 #pragma unroll
           for (int e = 0; e < 4; ++e) {
             const float v1 = __shfl_down_sync(0xffffffffu, m[i + e], 1);
             float v2 = __shfl_down_sync(0xffffffffu, m[i + e], 2);
             if (from_next) v2 = xs[(quad + 1) * 64 + i + e];
-            float t = max_nan(max_nan(m[i + e], v1), v2) + bias_s[i + e];
-            r4[e] = t != t ? t : fmaxf(t, 0.f);
+            float t = max_nan(max_nan(m[i + e], v1), v2) + bias_h[i + e];
+            r4[e] = max_nan(t, 0.f);
           }
           if (store) o[i / 4] = make_float4(r4[0], r4[1], r4[2], r4[3]);
         }
         xb ^= 1u;
+        GH_SC_ADD(prof_st, prof_s0);
       }
       gc += (uint32_t)(sg.y_hi - sg.y_lo + 1);
     }
+#ifdef GH_SC_PROFILE
+    if (warp == kScEpiWarp0 && lane == 0) {
+      long long prof_tot = 0;
+      GH_SC_ADD(prof_tot, prof_t0);
+      GH_SC_FLUSH(8, prof_tot);
+      GH_SC_FLUSH(9, prof_af);
+      GH_SC_FLUSH(10, prof_ld);
+      GH_SC_FLUSH(11, prof_bar);
+      GH_SC_FLUSH(12, prof_st);
+      GH_SC_FLUSH(13, prof_n);
+    }
+#endif
   }
 
   tc_fence_before_sync();
@@ -355,6 +447,14 @@ __global__ void __launch_bounds__(kScThreads, 1) stem_conv_pool_kernel(const Ste
     tc_fence_after_sync();
     tmem_dealloc(tmem_base, 512);
   }
+#ifdef GH_SC_PROFILE
+  if (threadIdx.x == 0) {
+    long long prof_tot = 0;
+    GH_SC_ADD(prof_tot, prof_cta0);
+    GH_SC_FLUSH(14, 1);
+    GH_SC_FLUSH(15, prof_tot);
+  }
+#endif
 }
 
 }  // namespace gh

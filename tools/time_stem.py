@@ -23,7 +23,7 @@ B = int(sys.argv[1]) if len(sys.argv) > 1 else 256
 H = W = 224
 ROUNDS, LAUNCHES, STEPS = 5, 20, 20
 TILE_COLS = 63                                  # csrc/stem.cuh: kScTileCols
-MMA_FLOPS_PER_CONV_ROW = 32 * 2 * 128 * 64 * 8  # 16 taps x 2 MMAs of 128 x 64 x 8 per conv row and tile
+MMA_FLOPS_PER_CONV_ROW = 24 * 2 * 128 * 64 * 8  # 4 tap rows x 6 MMAs of 128 x 64 x 8 per conv row and tile
 dev = torch.device("cuda:0")
 
 
