@@ -128,6 +128,11 @@ __device__ __forceinline__ void fence_proxy_async_smem() {
   asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
 }
 
+// Barrier among a subset of the CTA's warps (nthreads a multiple of 32); id 0 is __syncthreads'.
+__device__ __forceinline__ void named_bar_sync(uint32_t id, uint32_t nthreads) {
+  asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
+}
+
 // ---------------------------------------------------------------------------------------------
 // tcgen05: TMEM allocation, fences, MMA, commit, load
 // ---------------------------------------------------------------------------------------------

@@ -1,33 +1,41 @@
-// Gram backward, second design:  dF_b[c][x] = scale * sum_d M_b[c][d] F_b[d][x],   M = dG + dG^T.
+// Single-CTA Gram backward:  dF_b[c][x] = scale * sum_d M_b[c][d] F_b[d][x],   M = dG + dG^T.
 //
-// Same math as gram_bwd.cuh (reference autograd of Models/...Attention.py:26-30,51-52), different operand roles so that
-// F is consumed exactly as it lies in HBM:
+// This is what autograd derives for the reference's bmm(features, features^T).div(h*w)
+// (Models/Models_RESNET50_TRUNCATE_GRAM_with_Attention.py:26-30) followed, on the classification path, by
+// adaptive_avg_pool2d (:51-52). In POOL mode dG is never materialised: it is the block-constant upsampling of the
+// g x g descriptor gradient, dG[c][d] = dP[c/k][d/k] / k^2, and the symmetrised bf16 operand tile is generated in
+// shared memory from the image's dP. In DENSE mode (gram_matrix() used directly, e.g. style transfer) dG is read from
+// HBM. F is consumed exactly as it lies in HBM:
 //   A tile = M   [128 c][64 d]  K-major SWIZZLE_128B, generated in smem from the image's g x g descriptor gradient
 //                               (POOL) or read from the dense dG (DENSE); two of them per stage (256 output channels)
-//   B tile = F   [64 d][NHW x]  MN-major SWIZZLE_128B: rows of F are contiguous along x, which IS the MN-major
+//   B tile = F   [64 d][256 x]  MN-major SWIZZLE_128B: rows of F are contiguous along x, which IS the MN-major
 //                               canonical layout ([x/64][d/8][d%8][64 x] with 16 B chunks XOR-swizzled by d%8), so the
 //                               producers use the same coalesced ld.global.v4 -> cvt -> st.shared path as the forward
 //                               kernel: no transposing gathers, no scalar loads
-//   D      = dF  [128 c][NHW x] in TMEM: lane = output channel, 32 consecutive x per tcgen05.ld -> 8 x 16 B stores
-//   unit   = (image, NHW-wide x tile, pair of 128-channel output blocks); every CTA owns a contiguous range of units
+//   D      = dF  [128 c][256 x] in TMEM: lane = output channel, 32 consecutive x per tcgen05.ld -> 8 x 16 B stores
+//   unit   = (image, 256-wide x tile, pair of 128-channel output blocks); every CTA owns a contiguous range of units
 //            so the per-image gradient table is rebuilt only at image boundaries
-//   TMEM   = 2 accumulators x NHW columns per unit: double-buffered for NHW = 128 (epilogue of unit i overlaps the MMAs
-//            of unit i+1), single-buffered for NHW = 256
-// Producers double-buffer their loads in registers in batches of 8 x 16 B per thread (one batch per stage for
-// NHW = 128, two for NHW = 256).
+//   TMEM   = one accumulator of 2 x 256 columns per unit
+//   warps  = 8 producers, 4 epilogue warps, 1 MMA warp (TMEM owner + the MMA-issuing thread): 13 warps
+// Producers double-buffer their loads in registers in batches of 8 x 16 B per thread, two batches per stage.
+// At batch 256 on every ResNet stage shape, 256-wide x tiles beat 128-wide ones with two accumulators, and a separate MMA
+// warp beats 16 producer warps with the MMAs issued by an epilogue warp (profiles/r01e_kernel_timings.log).
 #pragma once
 #include "common.cuh"
 #include "gram_fwd.cuh"   // GramMode
-#include "gram_bwd.cuh"   // named_bar_sync
 
 namespace gh {
 
-// Two warp layouts:  NPW = 8 : 8 producer warps, 4 epilogue warps, 1 MMA warp (13 warps; needs the separate issuer
-//                               because the double-buffered accumulators of NHW = 128 let MMAs overlap the epilogue)
-//                    NPW = 16: 16 producer warps, 4 epilogue warps whose first one also issues the MMAs (20 warps,
-//                               96 registers each; only with the single accumulator buffer of NHW = 256)
+constexpr int kB2NHW = 256;                                 // x positions per unit
+constexpr int kB2ProducerWarps = 8;
+constexpr int kB2ProducerThreads = kB2ProducerWarps * 32;
+constexpr int kB2MmaWarp = kB2ProducerWarps + 4;            // after the 4 epilogue warps
+constexpr int kB2Threads = (kB2MmaWarp + 1) * 32;           // 13 warps
+constexpr int kB2Batches = 2 * kB2NHW / kB2ProducerThreads; // register batches (8 x 16 B per thread) per stage
 constexpr uint32_t kB2ATileBytes = 128 * kRowBytes;        // 16 KB
+constexpr uint32_t kB2StageBytes = 2 * kB2ATileBytes + kB2NHW * kRowBytes;   // 64 KB
 constexpr uint32_t kB2RingBytes = 192 * 1024;
+constexpr int kB2Stages = (int)(kB2RingBytes / kB2StageBytes);              // 3
 constexpr int kB2MaxStages = 4;
 constexpr int kB2MaxG = 64;
 constexpr uint32_t kB2SmemBytes = kB2RingBytes + kB2MaxG * kB2MaxG * 4 + 1024 + 256;
@@ -77,7 +85,6 @@ struct Gb2Item {
   GramBwd2Unit w;
 };
 
-template <int NBATCH>
 __device__ __forceinline__ bool gb2_first(Gb2Item& it, const GramBwd2Params& p, int u0, int u1) {
   it.u = u0;
   if (u0 >= u1) return false;
@@ -86,9 +93,8 @@ __device__ __forceinline__ bool gb2_first(Gb2Item& it, const GramBwd2Params& p, 
   it.half = 0;
   return true;
 }
-template <int NBATCH>
 __device__ __forceinline__ bool gb2_next(Gb2Item& it, const GramBwd2Params& p, int u1) {
-  if (++it.half < NBATCH) return true;
+  if (++it.half < kB2Batches) return true;
   it.half = 0;
   if (++it.kb < p.nkb) return true;
   it.kb = 0;
@@ -97,13 +103,13 @@ __device__ __forceinline__ bool gb2_next(Gb2Item& it, const GramBwd2Params& p, i
   return true;
 }
 
-// One batch = 8 segments per thread; a segment = 4 consecutive x of one F row. Segment index s in [0, NHW) per stage:
-// d_local = s / MB, x block = s % MB (MB = NHW / 64), so consecutive segments continue along the same F row.
-template <int SRC, int NHW, int NT>
+// One batch = 8 segments per thread; a segment = 4 consecutive x of one F row. Segment index s in [0, 1024) per stage:
+// d_local = s / MB, x block = s % MB (MB = 256 / 64), so consecutive segments continue along the same F row.
+template <int SRC>
 __device__ __forceinline__ void gb2_load(const GramBwd2Params& p, const Gb2Item& it, uint4 (&r)[8], int tid) {
-  constexpr int MB = NHW / 64, SPP = NT / 16;   // 64-wide x blocks per row; segments per pass
+  constexpr int MB = kB2NHW / 64, SPP = kB2ProducerThreads / 16;   // 64-wide x blocks per row; segments per pass
   const int seg = tid >> 4, q = tid & 15;
-  const int hw0 = it.w.ht * NHW;
+  const int hw0 = it.w.ht * kB2NHW;
 #pragma unroll
   for (int i = 0; i < 8; ++i) {
     const int s = seg + SPP * (i + 8 * it.half);
@@ -143,9 +149,9 @@ __device__ __forceinline__ void gb2_load(const GramBwd2Params& p, const Gb2Item&
   }
 }
 
-template <int SRC, int NHW, int NT>
+template <int SRC>
 __device__ __forceinline__ void gb2_store_b(const Gb2Item& it, const uint4 (&r)[8], uint32_t b_smem, int tid) {
-  constexpr int MB = NHW / 64, SPP = NT / 16;
+  constexpr int MB = kB2NHW / 64, SPP = kB2ProducerThreads / 16;
   const int seg = tid >> 4, q = tid & 15;
 #pragma unroll
   for (int i = 0; i < 8; ++i) {
@@ -162,10 +168,9 @@ __device__ __forceinline__ void gb2_store_b(const Gb2Item& it, const uint4 (&r)[
 }
 
 // A tiles of one stage: rows n in [0, 256) = output channels cp*256 + n, columns = input channels kb*64 .. +63.
-template <int NT>
 __device__ __forceinline__ void gb2_gen_a(const GramBwd2Params& p, const Gb2Item& it, const float* sym, uint32_t a_smem,
                                           int tid) {
-  constexpr int CPT = 8 * 256 / NT;           // 16 B chunks per thread: 8 (256 threads) or 4 (512 threads)
+  constexpr int CPT = 8 * 256 / kB2ProducerThreads;   // 16 B chunks per thread
   const int r256 = tid & 255, j0 = (tid >> 8) * CPT;
   const int c = it.w.cp * 256 + r256;
   const uint32_t tile = a_smem + (uint32_t)(r256 >> 7) * kB2ATileBytes;
@@ -207,73 +212,29 @@ __device__ __forceinline__ void gb2_gen_a(const GramBwd2Params& p, const Gb2Item
   }
 }
 
-// MMAs of one unit (all k-blocks), issued by lane 0 of the calling warp.
-template <int NHW, int kStages, int NACC>
-__device__ __forceinline__ void gb2_issue_unit(const GramBwd2Params& p, uint32_t smem_base, uint32_t stage_bytes,
-                                               uint32_t bar_full, uint32_t bar_empty, uint32_t bar_tfull,
-                                               uint32_t bar_tempty, uint32_t tmem_base, uint32_t& stage, uint32_t& phase,
-                                               uint32_t it, int lane) {
-  const uint32_t idesc = make_idesc_bf16_bmn(128, NHW);
-  const uint32_t ab = (NACC == 2) ? (it & 1u) : 0u;
-  const uint32_t use = (NACC == 2) ? (it >> 1) : it;
-  mbar_wait(bar_tempty + 8 * ab, (use & 1u) ^ 1u, 200u + ab);
-  tc_fence_after_sync();
-  const uint32_t acc_col = ab * (2u * NHW);
-  for (int kb = 0; kb < p.nkb; ++kb) {
-    mbar_wait(bar_full + 8 * stage, phase, 300u + stage);
-    tc_fence_after_sync();
-    if (elect_one()) {   // elect.sync, not a lane test: see gram_fwd_pair.cuh
-      const uint32_t a_smem = smem_base + stage * stage_bytes;
-      const uint32_t b_smem = a_smem + 2 * kB2ATileBytes;
-#pragma unroll
-      for (uint32_t ks = 0; ks < kTileK / kUmmaK; ++ks) {
-        if ((int)(kb * 64 + ks * 16) >= p.C) break;
-        const uint64_t db = make_smem_desc_sw128_mn(b_smem + ks * 2048u);   // 16 k = two 8-row groups of 1 KB
-        for (int a = 0; a < p.nA; ++a)
-          umma_bf16(tmem_base + acc_col + (uint32_t)a * NHW,
-                    make_smem_desc_sw128(a_smem + (uint32_t)a * kB2ATileBytes + ks * 32u), db, idesc, (uint32_t)kb | ks);
-      }
-      umma_commit(bar_empty + 8 * stage);
-      if (kb + 1 == p.nkb) umma_commit(bar_tfull + 8 * ab);
-    }
-    __syncwarp();
-    if ((int)++stage == kStages) { stage = 0; phase ^= 1u; }
-  }
-}
-
-template <int SRC, int NHW, int NPW>
-__global__ void __launch_bounds__((NPW == 8 ? 13 : 20) * 32, 1) gram_bwd2_kernel(const GramBwd2Params p) {
-  constexpr int NT = NPW * 32;
-  constexpr int NB = 2 * NHW / NT;                        // register batches (8 x 16 B per thread) per stage
-  constexpr bool kMerged = (NPW == 16);                   // first epilogue warp issues the MMAs
-  constexpr int kEpiWarp0 = NPW, kMmaWarp = kMerged ? NPW : NPW + 4;
-  static_assert(NB >= 1 && (!kMerged || NHW == 256), "merged MMA/epilogue needs the single-buffer (NHW = 256) layout");
-  constexpr uint32_t kStageBytes = 2 * kB2ATileBytes + NHW * kRowBytes;   // 48 KB | 64 KB
-  constexpr int kStages = (int)(kB2RingBytes / kStageBytes);               // 4 | 3
-  constexpr int NACC = 512 / (2 * NHW);                   // accumulator buffers: 2 | 1
+template <int SRC>
+__global__ void __launch_bounds__(kB2Threads, 1) gram_bwd2_kernel(const GramBwd2Params p) {
   extern __shared__ uint8_t smem_raw[];
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   const uint32_t sym_smem = smem_base + kB2RingBytes;
   float* sym = reinterpret_cast<float*>(smem_raw + (sym_smem - smem_u32(smem_raw)));
   const uint32_t bars = sym_smem + kB2MaxG * kB2MaxG * 4;
   const uint32_t bar_full = bars, bar_empty = bars + 8 * kB2MaxStages;
-  const uint32_t bar_tfull = bars + 16 * kB2MaxStages, bar_tempty = bar_tfull + 16;
-  const uint32_t tmem_slot = bar_tempty + 16;
+  const uint32_t bar_tfull = bars + 16 * kB2MaxStages, bar_tempty = bar_tfull + 8;
+  const uint32_t tmem_slot = bar_tempty + 8;
   volatile uint32_t* tmem_slot_ptr = reinterpret_cast<volatile uint32_t*>(smem_raw + (tmem_slot - smem_u32(smem_raw)));
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   if (threadIdx.x == 0) {
     for (int s = 0; s < kB2MaxStages; ++s) {
-      mbar_init(bar_full + 8 * s, NPW);
+      mbar_init(bar_full + 8 * s, kB2ProducerWarps);
       mbar_init(bar_empty + 8 * s, 1);
     }
-    for (int a = 0; a < 2; ++a) {
-      mbar_init(bar_tfull + 8 * a, 1);
-      mbar_init(bar_tempty + 8 * a, 4);
-    }
+    mbar_init(bar_tfull, 1);
+    mbar_init(bar_tempty, 4);
     mbar_fence_init();
   }
-  if (warp == kMmaWarp) tmem_alloc(tmem_slot, 512);
+  if (warp == kB2MmaWarp) tmem_alloc(tmem_slot, 512);
   tc_fence_before_sync();
   __syncthreads();
   tc_fence_after_sync();
@@ -283,81 +244,100 @@ __global__ void __launch_bounds__((NPW == 8 ? 13 : 20) * 32, 1) gram_bwd2_kernel
   const int u0 = blockIdx.x * p.units_per_cta;
   const int u1 = min(u0 + p.units_per_cta, p.total_units);
 
-  if (warp < NPW) {
+  if (warp < kB2ProducerWarps) {
     // =========================== producers ===========================
     const int tid = threadIdx.x;
     uint32_t stage = 0, phase = 0;
     int cur_b = -1;
     uint4 ra[8], rb[8];
     Gb2Item cur;
-    bool have = gb2_first<NB>(cur, p, u0, u1);
-    if (have) gb2_load<SRC, NHW, NT>(p, cur, ra, tid);
+    bool have = gb2_first(cur, p, u0, u1);
+    if (have) gb2_load<SRC>(p, cur, ra, tid);
 
     auto publish = [&](const Gb2Item& it, const uint4 (&r)[8]) {
       if (it.half == 0) {
         if (p.mode == GRAM_POOL && it.w.b != cur_b) {
           // per-image table sym[i][j] = dP[i][j] + dP[j][i]; every producer is done reading the previous image's
-          named_bar_sync(1, NT);
+          named_bar_sync(1, kB2ProducerThreads);
           const float* dp = p.dP + (long long)it.w.b * p.dp_img_stride;
           const int gg = p.g * p.g;
-          for (int i = tid; i < gg; i += NT) {
+          for (int i = tid; i < gg; i += kB2ProducerThreads) {
             const int rr = i / p.g, cc = i - rr * p.g;
             sym[i] = __ldg(dp + i) + __ldg(dp + cc * p.g + rr);
           }
-          named_bar_sync(1, NT);
+          named_bar_sync(1, kB2ProducerThreads);
           cur_b = it.w.b;
         }
         mbar_wait(bar_empty + 8 * stage, phase ^ 1u, 100u + stage);
-        gb2_gen_a<NT>(p, it, sym, smem_base + stage * kStageBytes, tid);
+        gb2_gen_a(p, it, sym, smem_base + stage * kB2StageBytes, tid);
       }
-      gb2_store_b<SRC, NHW, NT>(it, r, smem_base + stage * kStageBytes + 2 * kB2ATileBytes, tid);
-      if (it.half == NB - 1) {
+      gb2_store_b<SRC>(it, r, smem_base + stage * kB2StageBytes + 2 * kB2ATileBytes, tid);
+      if (it.half == kB2Batches - 1) {
         fence_proxy_async_smem();
         __syncwarp();
         if (lane == 0) mbar_arrive(bar_full + 8 * stage);
-        if ((int)++stage == kStages) { stage = 0; phase ^= 1u; }
+        if ((int)++stage == kB2Stages) { stage = 0; phase ^= 1u; }
       }
     };
     while (have) {
       Gb2Item n1 = cur;
-      const bool h1 = gb2_next<NB>(n1, p, u1);
-      if (h1) gb2_load<SRC, NHW, NT>(p, n1, rb, tid);
+      const bool h1 = gb2_next(n1, p, u1);
+      if (h1) gb2_load<SRC>(p, n1, rb, tid);
       publish(cur, ra);
       if (!h1) break;
       cur = n1;
-      have = gb2_next<NB>(cur, p, u1);
-      if (have) gb2_load<SRC, NHW, NT>(p, cur, ra, tid);
+      have = gb2_next(cur, p, u1);
+      if (have) gb2_load<SRC>(p, cur, ra, tid);
       publish(n1, rb);
     }
-  } else if (!kMerged && warp == kMmaWarp) {
-    // =========================== MMA issuer (separate warp) ===========================
+  } else if (warp == kB2MmaWarp) {
+    // =========================== MMA issuer: all k-blocks of a unit ===========================
+    const uint32_t idesc = make_idesc_bf16_bmn(128, kB2NHW);
     uint32_t stage = 0, phase = 0, it = 0;
-    for (int u = u0; u < u1; ++u, ++it) gb2_issue_unit<NHW, kStages, NACC>(p, smem_base, kStageBytes, bar_full, bar_empty, bar_tfull, bar_tempty, tmem_base, stage, phase, it, lane);
+    for (int u = u0; u < u1; ++u, ++it) {
+      mbar_wait(bar_tempty, (it & 1u) ^ 1u, 200u);
+      tc_fence_after_sync();
+      for (int kb = 0; kb < p.nkb; ++kb) {
+        mbar_wait(bar_full + 8 * stage, phase, 300u + stage);
+        tc_fence_after_sync();
+        if (elect_one()) {   // elect.sync, not a lane test: see gram_fwd_pair.cuh
+          const uint32_t a_smem = smem_base + stage * kB2StageBytes;
+          const uint32_t b_smem = a_smem + 2 * kB2ATileBytes;
+#pragma unroll
+          for (uint32_t ks = 0; ks < kTileK / kUmmaK; ++ks) {
+            if ((int)(kb * 64 + ks * 16) >= p.C) break;
+            const uint64_t db = make_smem_desc_sw128_mn(b_smem + ks * 2048u);   // 16 k = two 8-row groups of 1 KB
+            for (int a = 0; a < p.nA; ++a)
+              umma_bf16(tmem_base + (uint32_t)a * kB2NHW,
+                        make_smem_desc_sw128(a_smem + (uint32_t)a * kB2ATileBytes + ks * 32u), db, idesc, (uint32_t)kb | ks);
+          }
+          umma_commit(bar_empty + 8 * stage);
+          if (kb + 1 == p.nkb) umma_commit(bar_tfull);
+        }
+        __syncwarp();
+        if ((int)++stage == kB2Stages) { stage = 0; phase ^= 1u; }
+      }
+    }
   } else {
     // =========================== epilogue ===========================
-    const int q = warp - kEpiWarp0;
+    const int q = warp - kB2ProducerWarps;
     uint32_t it = 0;
-    uint32_t mstage = 0, mphase = 0;
     for (int u = u0; u < u1; ++u, ++it) {
       const GramBwd2Unit w = gb2_decode(p, u);
-      if (kMerged && q == 0)
-        gb2_issue_unit<NHW, kStages, NACC>(p, smem_base, kStageBytes, bar_full, bar_empty, bar_tfull, bar_tempty, tmem_base, mstage, mphase, it, lane);
-      const uint32_t ab = (NACC == 2) ? (it & 1u) : 0u;
-      const uint32_t use = (NACC == 2) ? (it >> 1) : it;
-      mbar_wait(bar_tfull + 8 * ab, use & 1u, 400u + ab);
+      mbar_wait(bar_tfull, it & 1u, 400u);
       tc_fence_after_sync();
-      const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + ab * (2u * NHW);
-      const int x0 = w.ht * NHW;
+      const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16);
+      const int x0 = w.ht * kB2NHW;
 #pragma unroll 1
       for (int a = 0; a < p.nA; ++a) {
         const int c = w.cp * 256 + a * 128 + q * 32 + lane;
         float* orow = p.dF + (long long)w.b * p.df_img_stride + (long long)c * p.df_row_stride;
 #pragma unroll 1
-        for (int n0 = 0; n0 < NHW; n0 += 32) {
+        for (int n0 = 0; n0 < kB2NHW; n0 += 32) {
           const int x = x0 + n0;
           if (x >= p.HW) break;   // warp-uniform
           float v[32];
-          tmem_ld32(taddr + (uint32_t)(a * NHW + n0), v);
+          tmem_ld32(taddr + (uint32_t)(a * kB2NHW + n0), v);
           if (c < p.C) {
             if (p.df_vec_ok && x + 32 <= p.HW) {
 #pragma unroll
@@ -374,13 +354,13 @@ __global__ void __launch_bounds__((NPW == 8 ? 13 : 20) * 32, 1) gram_bwd2_kernel
       }
       tc_fence_before_sync();
       __syncwarp();
-      if (lane == 0) mbar_arrive(bar_tempty + 8 * ab);
+      if (lane == 0) mbar_arrive(bar_tempty);
     }
   }
 
   tc_fence_before_sync();
   __syncthreads();
-  if (warp == kMmaWarp) {
+  if (warp == kB2MmaWarp) {
     tc_fence_after_sync();
     tmem_dealloc(tmem_base, 512);
   }

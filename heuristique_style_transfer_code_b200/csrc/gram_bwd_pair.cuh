@@ -24,7 +24,6 @@
 #pragma once
 #include "pair.cuh"
 #include "gram_fwd.cuh"   // GramMode
-#include "gram_bwd.cuh"   // named_bar_sync
 
 namespace gh {
 

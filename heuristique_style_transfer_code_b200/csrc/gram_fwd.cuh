@@ -8,7 +8,7 @@
 // Work decomposition
 //   unit      = (image b, 256x256 super-tile (I <= J) of the Gram, K-range kp of ksplit)
 //   CTA       = persistent, walks units blockIdx.x, +gridDim.x, ...
-//   producers = NPW (8 or 16) warps: ld.global fp32/bf16 (coalesced along HW) -> cvt.rn.bf16x2 -> st.shared into the
+//   producers = 16 warps: ld.global fp32/bf16 (coalesced along HW) -> cvt.rn.bf16x2 -> st.shared into the
 //               UMMA K-major SWIZZLE_128B layout (no separate cast pass over HBM, any HW, any pitch); the loads of
 //               stage s+1 are issued before stage s is converted and stored (register double buffering)
 //   epilogue  = 4 warps: tcgen05.ld -> in-register k x k block sums -> descriptor (mirrored for off-diagonal
@@ -28,6 +28,9 @@ constexpr uint32_t kGfStageRows = 256;
 constexpr uint32_t kGfStageBytes = kGfStageRows * kRowBytes;   // 32 KB
 constexpr uint32_t kGfSmemBytes = kGfStages * kGfStageBytes + 1024 /*align*/ + 256 /*barriers*/;
 constexpr uint32_t kGfTmemCols = 512;
+constexpr int kGfProducerWarps = 16;
+constexpr int kGfProducerThreads = kGfProducerWarps * 32;
+constexpr int kGfThreads = (kGfProducerWarps + 4) * 32;   // + 4 epilogue warps
 
 enum GramMode : int { GRAM_POOL = 0, GRAM_DENSE = 1 };
 
@@ -69,7 +72,7 @@ __device__ __forceinline__ GramUnit gram_decode_unit(const GramFwdParams& p, int
 
 // ---- producers ----------------------------------------------------------------------------------------------------
 // One stage = rows [blk*256, blk*256+256) x k in [kb*64, kb*64+64) of image b.
-// 16 threads cover one row (64 elements, 4 each); NT producer threads cover NT/16 rows per pass, 4096/NT passes.
+// 16 threads cover one row (64 elements, 4 each); the 512 producer threads cover 32 rows per pass, 8 passes.
 // Loading (global -> registers) and storing (registers -> swizzled smem) are separate steps so that the loads of the
 // NEXT stage are in flight while the current one is converted and stored (register double buffering): the memory
 // pipe never drains between stages, units or images.
@@ -106,9 +109,11 @@ struct GfRegs {
   uint2 h[SRC == 0 ? 1 : NL];
 };
 
-template <int SRC, int NT>
-__device__ __forceinline__ void gf_load(const GramFwdParams& p, const GfItem& it, GfRegs<SRC, 4096 / NT>& r, int tid) {
-  constexpr int NL = 4096 / NT, RPP = NT / 16;
+constexpr int kGfLoads = 4096 / kGfProducerThreads;   // 16 B loads per producer thread and stage
+
+template <int SRC>
+__device__ __forceinline__ void gf_load(const GramFwdParams& p, const GfItem& it, GfRegs<SRC, kGfLoads>& r, int tid) {
+  constexpr int NL = kGfLoads, RPP = kGfProducerThreads / 16;
   const int sub = tid >> 4, q = tid & 15;
   const int k = it.kb * 64 + q * 4;
   const int blk = it.h == 0 ? it.w.I : it.w.J;
@@ -162,10 +167,10 @@ __device__ __forceinline__ void gf_load(const GramFwdParams& p, const GfItem& it
   }
 }
 
-template <int SRC, int NT>
-__device__ __forceinline__ void gf_store(const GramFwdParams& p, const GfItem& it, const GfRegs<SRC, 4096 / NT>& r,
+template <int SRC>
+__device__ __forceinline__ void gf_store(const GramFwdParams& p, const GfItem& it, const GfRegs<SRC, kGfLoads>& r,
                                          uint32_t stage_smem, int tid) {
-  constexpr int NL = 4096 / NT, RPP = NT / 16;
+  constexpr int NL = kGfLoads, RPP = kGfProducerThreads / 16;
   const int sub = tid >> 4, q = tid & 15;
   // a 16-wide k-step that lies entirely beyond HW is never issued to the tensor core, so it need not be written
   if (it.kb * 64 + (q >> 2) * 16 >= p.HW) return;
@@ -178,12 +183,12 @@ __device__ __forceinline__ void gf_store(const GramFwdParams& p, const GfItem& i
   }
 }
 
-template <int SRC, int NT>
-__device__ __forceinline__ void gf_publish(const GramFwdParams& p, const GfItem& it, const GfRegs<SRC, 4096 / NT>& r,
+template <int SRC>
+__device__ __forceinline__ void gf_publish(const GramFwdParams& p, const GfItem& it, const GfRegs<SRC, kGfLoads>& r,
                                            uint32_t smem_base, uint32_t bar_full, uint32_t bar_empty, uint32_t& stage,
                                            uint32_t& phase, int tid, int lane) {
   mbar_wait(bar_empty + 8 * stage, phase ^ 1u, 100u + stage);
-  gf_store<SRC, NT>(p, it, r, smem_base + stage * kGfStageBytes, tid);
+  gf_store<SRC>(p, it, r, smem_base + stage * kGfStageBytes, tid);
   fence_proxy_async_smem();
   __syncwarp();
   if (lane == 0) mbar_arrive(bar_full + 8 * stage);
@@ -414,11 +419,10 @@ __device__ __forceinline__ void gf_issue_unit(const GramFwdParams& p, const Gram
   }
 }
 
-// Drains the accumulators of one unit. q = TMEM lane quarter of this warp, hc / nhc = which of the nhc warps sharing a
-// quarter this is (they alternate 128-column groups).
+// Drains the accumulators of one unit. q = TMEM lane quarter of this warp.
 template <int KP>
 __device__ __forceinline__ void gf_epilogue_unit(const GramFwdParams& p, const GramUnit& w, uint32_t tmem_base, int q,
-                                                 int hc, int nhc, bool atomics, int lane) {
+                                                 bool atomics, int lane) {
   const bool diag = (w.I == w.J);
   float* outp = p.out + (long long)w.b * p.out_img_stride;
   const uint32_t lane_addr = tmem_base + ((uint32_t)(q * 32) << 16);
@@ -429,9 +433,8 @@ __device__ __forceinline__ void gf_epilogue_unit(const GramFwdParams& p, const G
     const int colbase = w.J * 256 + ((a == 1 && diag) ? 128 : 0);
     if (w.I * 256 + a * 128 >= p.C) break;   // whole accumulator is padding (C <= 128)
 #pragma unroll 1
-    for (int g0 = hc * 128; g0 < ncols; g0 += 128 * nhc) {
+    for (int g0 = 0; g0 < ncols && colbase + g0 < p.C; g0 += 128) {   // columns >= C are padding
       const int c_grp = colbase + g0;
-      if (c_grp >= p.C) break;              // padding columns
       // a 128x128 block strictly above the diagonal is mirrored; diagonal blocks are complete on their own
       const bool mirror = (c_grp >> 7) > (c_row >> 7);
       if constexpr (KP >= 8) {
@@ -453,17 +456,16 @@ __device__ __forceinline__ void gf_epilogue_unit(const GramFwdParams& p, const G
   }
 }
 
-// SRC: see gf_load.  KP = pool factor (POOL) or 0 (DENSE).  NPW = producer warps (8 or 16).
-// NEW = epilogue warps (4 or 8).
-// Warp roles: [0, NPW) producers, [NPW, NPW+NEW) epilogue (NPW % 4 == 0 so warp % 4 is the TMEM lane quarter). The first
-// epilogue warp also owns TMEM and issues the MMAs of a unit before joining its epilogue: with one accumulator set in
-// TMEM (384-512 of the 512 columns) the two phases of a unit cannot overlap anyway, and NPW + 4 warps (a multiple of
-// the 4 SM sub-partitions) leaves every thread 96 (NPW = 16) / 168 (NPW = 8) registers for the double-buffered loads.
-template <int SRC, int KP, int NPW, int NEW>
-__global__ void __launch_bounds__((NPW + NEW) * 32, 1) gram_fwd_kernel(const GramFwdParams p) {
-  constexpr int NT = NPW * 32;
-  constexpr int kEpiWarp0 = NPW, kMmaWarp = NPW;
-  static_assert(NEW == 4 || NEW == 8, "4 or 8 epilogue warps");
+// SRC: see gf_load.  KP = pool factor (POOL) or 0 (DENSE).
+// Warp roles: [0, 16) producers, [16, 20) epilogue (warp % 4 is the TMEM lane quarter). The first epilogue warp also
+// owns TMEM and issues the MMAs of a unit before joining its epilogue: with one accumulator set in TMEM (384-512 of the
+// 512 columns) the two phases of a unit cannot overlap anyway, and 20 warps (a multiple of the 4 SM sub-partitions)
+// leave every thread 96 registers for the double-buffered loads. Measured on every ResNet stage shape
+// (profiles/r01e_kernel_timings.log), 16 producer warps are as fast as 8 or faster, and 8 epilogue warps (24 warps -> 80
+// registers per thread) spill in the producer loop and lose.
+template <int SRC, int KP>
+__global__ void __launch_bounds__(kGfThreads, 1) gram_fwd_kernel(const GramFwdParams p) {
+  constexpr int kEpiWarp0 = kGfProducerWarps, kMmaWarp = kGfProducerWarps;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   const uint32_t bars = smem_base + kGfStages * kGfStageBytes;
@@ -478,11 +480,11 @@ __global__ void __launch_bounds__((NPW + NEW) * 32, 1) gram_fwd_kernel(const Gra
 
   if (threadIdx.x == 0) {
     for (int s = 0; s < kGfStages; ++s) {
-      mbar_init(bar_full + 8 * s, NPW);
+      mbar_init(bar_full + 8 * s, kGfProducerWarps);
       mbar_init(bar_empty + 8 * s, 1);
     }
     mbar_init(bar_tfull, 1);
-    mbar_init(bar_tempty, NEW);
+    mbar_init(bar_tempty, 4);
     mbar_fence_init();
   }
   if (warp == kMmaWarp) tmem_alloc(tmem_slot, kGfTmemCols);
@@ -491,30 +493,29 @@ __global__ void __launch_bounds__((NPW + NEW) * 32, 1) gram_fwd_kernel(const Gra
   tc_fence_after_sync();
   const uint32_t tmem_base = *tmem_slot_ptr;
 
-  if (warp < NPW) {
+  if (warp < kGfProducerWarps) {
     // =========================== producers ===========================
     uint32_t stage = 0, phase = 0;
     const int tid = threadIdx.x;
-    GfRegs<SRC, 4096 / NT> ra, rb;
+    GfRegs<SRC, kGfLoads> ra, rb;
     GfItem cur;
     bool have = gf_item_first(cur, p);
-    if (have) gf_load<SRC, NT>(p, cur, ra, tid);
+    if (have) gf_load<SRC>(p, cur, ra, tid);
     while (have) {
       GfItem n1 = cur;
       const bool h1 = gf_item_next(n1, p);
-      if (h1) gf_load<SRC, NT>(p, n1, rb, tid);    // next stage's loads fly while this one is stored
-      gf_publish<SRC, NT>(p, cur, ra, smem_base, bar_full, bar_empty, stage, phase, tid, lane);
+      if (h1) gf_load<SRC>(p, n1, rb, tid);    // next stage's loads fly while this one is stored
+      gf_publish<SRC>(p, cur, ra, smem_base, bar_full, bar_empty, stage, phase, tid, lane);
       if (!h1) break;
       cur = n1;
       have = gf_item_next(cur, p);
-      if (have) gf_load<SRC, NT>(p, cur, ra, tid);
-      gf_publish<SRC, NT>(p, n1, rb, smem_base, bar_full, bar_empty, stage, phase, tid, lane);
+      if (have) gf_load<SRC>(p, cur, ra, tid);
+      gf_publish<SRC>(p, n1, rb, smem_base, bar_full, bar_empty, stage, phase, tid, lane);
     }
   } else {
     // =========================== MMA issue (first epilogue warp) + epilogue (all of them) ===========================
     const int ew = warp - kEpiWarp0;
     const int q = ew & 3;             // TMEM lane quarter this warp may read (= warp % 4)
-    const int hc = ew >> 2;           // with 8 epilogue warps, the two warps of a quarter alternate 128-column groups
     uint32_t acc_phase = 0, stage = 0, phase = 0;
     const bool atomics = p.use_atomics != 0;
     for (int u = blockIdx.x; u < p.total_units; u += gridDim.x) {
@@ -523,7 +524,7 @@ __global__ void __launch_bounds__((NPW + NEW) * 32, 1) gram_fwd_kernel(const Gra
         gf_issue_unit(p, w, smem_base, bar_full, bar_empty, bar_tfull, bar_tempty, tmem_base, stage, phase, acc_phase, lane);
       mbar_wait(bar_tfull, acc_phase, 400u);
       tc_fence_after_sync();
-      gf_epilogue_unit<KP>(p, w, tmem_base, q, hc, NEW / 4, atomics, lane);
+      gf_epilogue_unit<KP>(p, w, tmem_base, q, atomics, lane);
       tc_fence_before_sync();
       __syncwarp();
       if (lane == 0) mbar_arrive(bar_tempty);

@@ -4,7 +4,6 @@
 #include "common.cuh"
 #include "gram_fwd.cuh"
 #include "gram_fwd_pair.cuh"
-#include "gram_bwd.cuh"
 #include "gram_bwd2.cuh"
 #include "gram_bwd_pair.cuh"
 #include "attn_head.cuh"
@@ -60,19 +59,11 @@ static int choose_ksplit(long long base_units, int nkb, int ctas, bool balance =
   return ks < 1 ? 1 : (int)ks;
 }
 
-// Tuning knobs (gh_set_option)
-static int g_opt_fwd_producer_warps = 0;    // 0 = auto
-static int g_opt_fwd_epilogue_warps = 0;    // 0 = auto
-static int g_opt_bwd_variant = 2;   // 1 = transposed product (gram_bwd.cuh), 2 = MN-major F operand (gram_bwd2.cuh)
-static int g_opt_bwd_nhw = 0;       // 0 = auto, 128, 256
-static int g_opt_bwd_producer_warps = 8;    // NHW = 256 only; measured: 8 (separate MMA warp) beats 16 (merged) on every shape
-static int g_opt_attn_gemm = 1;     // 1 = tcgen05 split-bf16 GEMM for the attention linear layers, 0 = fp32 SIMT
-
 // D = A B (+ bias) with strided fp32 operands: tensor-core path when the layout allows it, fp32 FMA kernel otherwise.
 static cudaError_t gemm_auto(const float* A, long long a_sm, long long a_sk, const float* Bm, long long b_sk,
                              long long b_sn, const float* bias, float* D, long long ldd, int M, int N, int K,
                              int accumulate, cudaStream_t st) {
-  if (g_opt_attn_gemm == 1 && !accumulate && (a_sk == 1 || a_sm == 1) && (b_sk == 1 || b_sn == 1)) {
+  if (!accumulate && (a_sk == 1 || a_sm == 1) && (b_sk == 1 || b_sn == 1)) {
     const bool a_mn = (a_sk != 1), b_mn = (b_sk != 1);
     cudaError_t e = launch_umma_gemm(A, a_mn, a_mn ? a_sk : a_sm, Bm, b_mn, b_mn ? b_sk : b_sn, bias, D, ldd, M, N, K,
                                      sm_count_cached(), st);
@@ -81,37 +72,26 @@ static cudaError_t gemm_auto(const float* A, long long a_sm, long long a_sk, con
   return launch_sgemm(A, a_sm, a_sk, Bm, b_sk, b_sn, bias, D, ldd, M, N, K, accumulate, st);
 }
 
-template <int SRC, int KP, int NPW, int NEW>
+template <int SRC, int KP>
 static cudaError_t launch_gram_fwd_one(const GramFwdParams& p, int grid, cudaStream_t st) {
-  cudaError_t e = cudaFuncSetAttribute(gram_fwd_kernel<SRC, KP, NPW, NEW>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+  cudaError_t e = cudaFuncSetAttribute(gram_fwd_kernel<SRC, KP>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                        (int)kGfSmemBytes);
   if (e != cudaSuccess) return e;
-  gram_fwd_kernel<SRC, KP, NPW, NEW><<<grid, (NPW + NEW) * 32, kGfSmemBytes, st>>>(p);
+  gram_fwd_kernel<SRC, KP><<<grid, kGfThreads, kGfSmemBytes, st>>>(p);
   return cudaGetLastError();
 }
 
 template <int SRC>
 static cudaError_t launch_gram_fwd_kp(const GramFwdParams& p, int kp, int grid, cudaStream_t st) {
-  // Warp mix: 16 producer + 4 epilogue warps measured best on every ResNet stage shape (profiles/r01e_kernel_timings.log);
-  // 8 epilogue warps (24 warps -> 80 registers/thread) spill in the producer loop and lose. gh_set_option overrides.
-  const int npw = g_opt_fwd_producer_warps ? g_opt_fwd_producer_warps : 16;
-  const int nepi = g_opt_fwd_epilogue_warps ? g_opt_fwd_epilogue_warps : 4;
-#define GH_LAUNCH_GF(KP)                                                                  \
-  {                                                                                       \
-    if (npw == 8) return launch_gram_fwd_one<SRC, KP, 8, 4>(p, grid, st);                 \
-    if (nepi == 4) return launch_gram_fwd_one<SRC, KP, 16, 4>(p, grid, st);               \
-    return launch_gram_fwd_one<SRC, KP, 16, 8>(p, grid, st);                              \
-  }
   switch (kp) {
-    case 0: GH_LAUNCH_GF(0)
-    case 8: GH_LAUNCH_GF(8)
-    case 16: GH_LAUNCH_GF(16)
-    case 32: GH_LAUNCH_GF(32)
-    case 64: GH_LAUNCH_GF(64)
-    case 128: GH_LAUNCH_GF(128)
+    case 0: return launch_gram_fwd_one<SRC, 0>(p, grid, st);
+    case 8: return launch_gram_fwd_one<SRC, 8>(p, grid, st);
+    case 16: return launch_gram_fwd_one<SRC, 16>(p, grid, st);
+    case 32: return launch_gram_fwd_one<SRC, 32>(p, grid, st);
+    case 64: return launch_gram_fwd_one<SRC, 64>(p, grid, st);
+    case 128: return launch_gram_fwd_one<SRC, 128>(p, grid, st);
     default: return cudaErrorInvalidValue;
   }
-#undef GH_LAUNCH_GF
 }
 
 // Pair (cta_group::2, TMA-staged) kernels. -1 = auto, 0 = never, 1 = whenever TMA can describe the tensors.
@@ -124,7 +104,6 @@ static int g_opt_bwd_ats = -1;      // pooled pair backward with the generated g
                                     // TMEM columns beside the two accumulators hold the A ring, -1 = auto (C >= 512)
 static int g_opt_bwd_ch = 0;        // K chunks per ring stage of the tensor-memory form, at most: 1, 2 (8 MMAs per iteration
                                     // of the issuing thread, when the widened A ring fits TMEM), 0 = auto (2)
-static int g_opt_tma_f32_type = 1;  // tensor-map data type for fp32 features: 0 = FLOAT32, 1 = TFLOAT32
 
 template <int KIND, int KP, bool NHWC>
 static cudaError_t launch_gram_fwd_pair_one(const GramFwdParams& p, const CUtensorMap& map, int npairs, cudaStream_t st) {
@@ -190,9 +169,9 @@ static int gram_fwd_common(const void* F, int f_dtype, long long img_stride, lon
     CUtensorMap map;
     const int kb_elems = is_bf16 ? 64 : 32;
     const bool mapped = nhwc ? make_tensor_map_nhwc_mn(&map, F, is_bf16, img_stride, x_stride, B, C, HW, kb_elems, 128,
-                                                       g_opt_tma_f32_type)
+                                                       /*tf32=*/true)
                              : make_tensor_map_xcb(&map, F, is_bf16, img_stride, row_stride, B, C, HW, kb_elems, 128,
-                                                   g_opt_tma_f32_type);
+                                                   /*tf32=*/true);
     if (mapped) {
       GramFwdParams q = p;
       q.nkb = (HW + kb_elems - 1) / kb_elems;
@@ -300,6 +279,14 @@ static bool plan_bwd_pair(int C, int HW, int g, int mode, bool is_bf16, bool nhw
   return q.b_stages >= 2;
 }
 
+template <int SRC>
+static cudaError_t launch_gram_bwd2(const GramBwd2Params& q, int grid, cudaStream_t st) {
+  cudaError_t e = cudaFuncSetAttribute(gram_bwd2_kernel<SRC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kB2SmemBytes);
+  if (e != cudaSuccess) return e;
+  gram_bwd2_kernel<SRC><<<grid, kB2Threads, kB2SmemBytes, st>>>(q);
+  return cudaGetLastError();
+}
+
 static int gram_bwd_common(const void* F, int f_dtype, long long img_stride, long long row_stride, long long x_stride,
                            int B, int C, int HW, int mode, int g, const float* dP, long long dp_img_stride,
                            const float* dG, void* dF_any, int df_dtype, long long df_img_stride, long long df_row_stride,
@@ -313,20 +300,18 @@ static int gram_bwd_common(const void* F, int f_dtype, long long img_stride, lon
   if (x_stride <= 0 || row_stride <= 0 || df_x_stride <= 0 || df_row_stride <= 0) return GH_ERR_BAD_ARG;
   if (nhwc != (df_x_stride != 1) || (nhwc && (row_stride != 1 || df_row_stride != 1))) return GH_ERR_BAD_ARG;
   if (C % 16 != 0) return GH_ERR_UNSUPPORTED;
-  GramBwdParams p;
-  p.F = F; p.img_stride = img_stride; p.row_stride = row_stride;
-  p.B = B; p.C = C; p.HW = HW; p.mode = mode;
-  p.dP = dP; p.dp_img_stride = dp_img_stride; p.g = g; p.kshift = 0; p.dG = dG;
+  int kshift = 0;           // POOL: pool factor k = 1 << kshift
+  float scale;
   if (mode == GRAM_POOL) {
     if (!dP) return GH_ERR_BAD_ARG;
-    if (g <= 0 || g > kGbMaxG || C % g != 0) return GH_ERR_UNSUPPORTED;
+    if (g <= 0 || g > kB2MaxG || C % g != 0) return GH_ERR_UNSUPPORTED;
     const int k = C / g;
-    p.kshift = ilog2_exact(k);
-    if (p.kshift < 0) return GH_ERR_UNSUPPORTED;
-    p.scale = 1.0f / ((float)HW * (float)k * (float)k);
+    kshift = ilog2_exact(k);
+    if (kshift < 0) return GH_ERR_UNSUPPORTED;
+    scale = 1.0f / ((float)HW * (float)k * (float)k);
   } else {
     if (!dG) return GH_ERR_BAD_ARG;
-    p.scale = 1.0f / (float)HW;
+    scale = 1.0f / (float)HW;
   }
   // ---- CTA-pair kernel: F TMA-staged as the MN-major operand, dF written with TMA stores ----
   {
@@ -345,17 +330,19 @@ static int gram_bwd_common(const void* F, int f_dtype, long long img_stride, lon
     if (want_pair && planned) {
       if (nhwc)     // F: K-major tiles [NT/2 position rows][128 B of channels]; dF: [32 x][32 c] tiles
         mapped = make_tensor_map_nhwc_cxb(&tmF, F, is_bf16, img_stride, x_stride, B, C, HW, kc_elems, q.NT / 2,
-                                          g_opt_tma_f32_type) &&
-                 make_tensor_map_nhwc_cxb(&tmD, dF, df16, df_img_stride, df_x_stride, B, C, HW, 32, 32, 0, /*swizzle64=*/df16);
+                                          /*tf32=*/true) &&
+                 make_tensor_map_nhwc_cxb(&tmD, dF, df16, df_img_stride, df_x_stride, B, C, HW, 32, 32, /*tf32=*/false,
+                                          /*swizzle64=*/df16);
       else
         mapped = make_tensor_map_xcb(&tmF, F, is_bf16, img_stride, row_stride, B, C, HW, kc_elems, kc_elems,
-                                     g_opt_tma_f32_type, /*atom32=*/!is_bf16) &&
-                 make_tensor_map_xcb(&tmD, dF, df16, df_img_stride, df_row_stride, B, C, HW, 32, 32, 0, false, /*swizzle64=*/df16);
+                                     /*tf32=*/true, /*atom32=*/!is_bf16) &&
+                 make_tensor_map_xcb(&tmD, dF, df16, df_img_stride, df_row_stride, B, C, HW, 32, 32, /*tf32=*/false, false,
+                                     /*swizzle64=*/df16);
     }
     if (mapped) {
       q.B = B; q.C = C; q.HW = HW; q.mode = mode;
-      q.dP = dP; q.dp_img_stride = dp_img_stride; q.g = g; q.kshift = p.kshift; q.dG = dG;
-      q.scale = p.scale;
+      q.dP = dP; q.dp_img_stride = dp_img_stride; q.g = g; q.kshift = kshift; q.dG = dG;
+      q.scale = scale;
       q.df_bf16 = df16 ? 1 : 0;
       const long long tot = (long long)B * q.nHT * q.nCB;
       if (tot <= 0x7fffffffLL) {
@@ -389,80 +376,32 @@ static int gram_bwd_common(const void* F, int f_dtype, long long img_stride, lon
       }
     }
   }
-  if (nhwc || df16) return GH_ERR_UNSUPPORTED;   // the ld.global kernels read / write fp32 NCHW rows only
-  if (g_opt_bwd_variant == 2) {
-    GramBwd2Params q;
-    q.F = F; q.img_stride = img_stride; q.row_stride = row_stride;
-    q.B = B; q.C = C; q.HW = HW; q.mode = mode;
-    q.dP = dP; q.dp_img_stride = dp_img_stride; q.g = g; q.kshift = p.kshift; q.dG = dG;
-    q.dF = dF; q.df_img_stride = df_img_stride; q.df_row_stride = df_row_stride; q.scale = p.scale;
-    const int nhw = g_opt_bwd_nhw ? g_opt_bwd_nhw : 256;   // measured: 256 wins on every ResNet stage shape
-    q.nHT = (HW + nhw - 1) / nhw;
-    q.nCP = (C + 255) / 256;
-    q.nkb = (C + 63) / 64;
-    q.nA = (C > 128) ? 2 : 1;
-    const long long total2 = (long long)B * q.nHT * q.nCP;
-    if (total2 > 0x7fffffffLL) return GH_ERR_UNSUPPORTED;
-    q.total_units = (int)total2;
-    const int sms2 = sm_count_cached();
-    const int ctas2 = (max_ctas > 0 && max_ctas < sms2) ? max_ctas : sms2;
-    int grid2 = (int)(total2 < ctas2 ? total2 : ctas2);
-    q.units_per_cta = (int)((total2 + grid2 - 1) / grid2);
-    grid2 = (int)((total2 + q.units_per_cta - 1) / q.units_per_cta);
-    q.df_vec_ok = (HW % 4 == 0 && df_img_stride % 4 == 0 && df_row_stride % 4 == 0 && ((uintptr_t)dF) % 16 == 0) ? 1 : 0;
-    const bool s4 = (HW % 4 == 0) && (row_stride % 4 == 0) && (img_stride % 4 == 0);
-    int src;
-    if (f_dtype == GH_DTYPE_F32) src = (s4 && ((uintptr_t)F) % 16 == 0) ? 0 : 1;
-    else src = (s4 && ((uintptr_t)F) % 8 == 0) ? 2 : 3;
-    cudaError_t e2 = cudaErrorInvalidValue;
-#define GH_LAUNCH_B2(SRC, NHW, NPW)                                                                                    \
-    {                                                                                                                  \
-      e2 = cudaFuncSetAttribute(gram_bwd2_kernel<SRC, NHW, NPW>, cudaFuncAttributeMaxDynamicSharedMemorySize,          \
-                                (int)kB2SmemBytes);                                                                    \
-      if (e2 == cudaSuccess) {                                                                                         \
-        gram_bwd2_kernel<SRC, NHW, NPW><<<grid2, (NPW == 8 ? 13 : 20) * 32, kB2SmemBytes, st>>>(q);                    \
-        e2 = cudaGetLastError();                                                                                       \
-      }                                                                                                                \
-    }
-    if (nhw == 128) {
-      if (src == 0) GH_LAUNCH_B2(0, 128, 8) else if (src == 1) GH_LAUNCH_B2(1, 128, 8)
-      else if (src == 2) GH_LAUNCH_B2(2, 128, 8) else GH_LAUNCH_B2(3, 128, 8)
-    } else if (g_opt_bwd_producer_warps == 8) {
-      if (src == 0) GH_LAUNCH_B2(0, 256, 8) else if (src == 1) GH_LAUNCH_B2(1, 256, 8)
-      else if (src == 2) GH_LAUNCH_B2(2, 256, 8) else GH_LAUNCH_B2(3, 256, 8)
-    } else {
-      if (src == 0) GH_LAUNCH_B2(0, 256, 16) else if (src == 1) GH_LAUNCH_B2(1, 256, 16)
-      else if (src == 2) GH_LAUNCH_B2(2, 256, 16) else GH_LAUNCH_B2(3, 256, 16)
-    }
-#undef GH_LAUNCH_B2
-    return (int)e2;
-  }
-  p.dF = dF; p.df_img_stride = df_img_stride; p.df_row_stride = df_row_stride;
-  p.NB = (C > 256) ? 2 : 1;
-  p.nHT = (HW + 127) / 128;
-  p.nCB = (C + 256 * p.NB - 1) / (256 * p.NB);
-  p.nkb = (C + 63) / 64;
-  p.stage_bytes = kGbATileBytes + (uint32_t)p.NB * kGbBBlkBytes;
-  p.stages = (int)(kGbRingBytes / p.stage_bytes);
-  if (p.stages > kGbMaxStages) p.stages = kGbMaxStages;
-  p.nacc = (p.NB == 1) ? 2 : 1;
-  const long long total = (long long)B * p.nHT * p.nCB;
+  if (nhwc || df16) return GH_ERR_UNSUPPORTED;   // the ld.global kernel reads / writes fp32 NCHW rows only
+  GramBwd2Params q;
+  q.F = F; q.img_stride = img_stride; q.row_stride = row_stride;
+  q.B = B; q.C = C; q.HW = HW; q.mode = mode;
+  q.dP = dP; q.dp_img_stride = dp_img_stride; q.g = g; q.kshift = kshift; q.dG = dG;
+  q.dF = dF; q.df_img_stride = df_img_stride; q.df_row_stride = df_row_stride; q.scale = scale;
+  q.nHT = (HW + kB2NHW - 1) / kB2NHW;
+  q.nCP = (C + 255) / 256;
+  q.nkb = (C + 63) / 64;
+  q.nA = (C > 128) ? 2 : 1;
+  const long long total = (long long)B * q.nHT * q.nCP;
   if (total > 0x7fffffffLL) return GH_ERR_UNSUPPORTED;
-  p.total_units = (int)total;
+  q.total_units = (int)total;
   const int sms = sm_count_cached();
   const int ctas = (max_ctas > 0 && max_ctas < sms) ? max_ctas : sms;
-  const int grid = (int)(total < ctas ? total : ctas);
+  int grid = (int)(total < ctas ? total : ctas);
+  q.units_per_cta = (int)((total + grid - 1) / grid);
+  grid = (int)((total + q.units_per_cta - 1) / q.units_per_cta);
+  q.df_vec_ok = (HW % 4 == 0 && df_img_stride % 4 == 0 && df_row_stride % 4 == 0 && ((uintptr_t)dF) % 16 == 0) ? 1 : 0;
+  const bool s4 = (HW % 4 == 0) && (row_stride % 4 == 0) && (img_stride % 4 == 0);
   cudaError_t e;
-  if (f_dtype == GH_DTYPE_F32) {
-    e = cudaFuncSetAttribute(gram_bwd_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kGbSmemBytes);
-    if (e != cudaSuccess) return (int)e;
-    gram_bwd_kernel<0><<<grid, kGbThreads, kGbSmemBytes, st>>>(p);
-  } else {
-    e = cudaFuncSetAttribute(gram_bwd_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kGbSmemBytes);
-    if (e != cudaSuccess) return (int)e;
-    gram_bwd_kernel<2><<<grid, kGbThreads, kGbSmemBytes, st>>>(p);
-  }
-  return (int)cudaGetLastError();
+  if (f_dtype == GH_DTYPE_F32)
+    e = (s4 && ((uintptr_t)F) % 16 == 0) ? launch_gram_bwd2<0>(q, grid, st) : launch_gram_bwd2<1>(q, grid, st);
+  else
+    e = (s4 && ((uintptr_t)F) % 8 == 0) ? launch_gram_bwd2<2>(q, grid, st) : launch_gram_bwd2<3>(q, grid, st);
+  return (int)e;
 }
 
 // ---- general-bin adaptive pooling (torch rule), used when C % g != 0 ------------------------------------------------
@@ -583,11 +522,6 @@ int gh_gram_bwd_plan(int C, int HW, int g, int f_dtype, int channels_last, int* 
 int gh_set_option(const char* name, int value) {
   if (!name) return GH_ERR_BAD_ARG;
   const std::string key(name);
-  if (key == "gram_fwd_producer_warps") {
-    if (value != 0 && value != 8 && value != 16) return GH_ERR_BAD_ARG;
-    g_opt_fwd_producer_warps = value;
-    return 0;
-  }
   if (key == "gram_fwd_pair") {
     if (value < -1 || value > 1) return GH_ERR_BAD_ARG;
     g_opt_fwd_pair = value;
@@ -619,16 +553,6 @@ int gh_set_option(const char* name, int value) {
     g_opt_bwd_ch = value;
     return 0;
   }
-  if (key == "tma_f32_type") {
-    if (value != 0 && value != 1) return GH_ERR_BAD_ARG;
-    g_opt_tma_f32_type = value;
-    return 0;
-  }
-  if (key == "gram_fwd_epilogue_warps") {
-    if (value != 0 && value != 4 && value != 8) return GH_ERR_BAD_ARG;
-    g_opt_fwd_epilogue_warps = value;
-    return 0;
-  }
   if (key == "tgemm_tn") {
     if (value != 0 && value != 128 && value != 256) return GH_ERR_BAD_ARG;
     g_opt_tg_tn = value;
@@ -637,26 +561,6 @@ int gh_set_option(const char* name, int value) {
   if (key == "pdl") {
     if (value != 0 && value != 1) return GH_ERR_BAD_ARG;
     g_opt_pdl = value;
-    return 0;
-  }
-  if (key == "attn_gemm") {
-    if (value != 0 && value != 1) return GH_ERR_BAD_ARG;
-    g_opt_attn_gemm = value;
-    return 0;
-  }
-  if (key == "gram_bwd_variant") {
-    if (value != 1 && value != 2) return GH_ERR_BAD_ARG;
-    g_opt_bwd_variant = value;
-    return 0;
-  }
-  if (key == "gram_bwd_producer_warps") {
-    if (value != 8 && value != 16) return GH_ERR_BAD_ARG;
-    g_opt_bwd_producer_warps = value;
-    return 0;
-  }
-  if (key == "gram_bwd_nhw") {
-    if (value != 0 && value != 128 && value != 256) return GH_ERR_BAD_ARG;
-    g_opt_bwd_nhw = value;
     return 0;
   }
   return GH_ERR_BAD_ARG;

@@ -255,12 +255,12 @@ inline PFN_encodeTiled get_encode_tiled() {
 // map (x, c, b) with a box of box_x x box_c x 1 elements and 128 B swizzle (box_x * elem_bytes must be 128).
 // Out-of-bounds box elements read as zero and are not written. Returns false when TMA cannot describe the layout
 // (base or pitches not multiples of 16 B, extents out of range): the caller then uses a non-TMA kernel.
-// f32_type: 0 = CU_TENSOR_MAP_DATA_TYPE_FLOAT32 (bits copied; the tensor core then truncates to tf32),
-//           1 = ..._TFLOAT32 (the TMA unit rounds fp32 to the nearest tf32 on the way in: measured on B200, normwise
-//               Gram error 4e-6..7e-6 against 7e-4 for the truncating path).
+// tf32: fp32 elements as CU_TENSOR_MAP_DATA_TYPE_TFLOAT32, for tensor-core operands: the TMA unit rounds fp32 to the
+//       nearest tf32 on the way in (measured on B200: normwise Gram error 4e-6..7e-6, against 7e-4 for FLOAT32 bits
+//       that the tensor core truncates). Otherwise FLOAT32: bits copied (gradient stores).
 // atom32: 128 B swizzle with a 32 B atom (MN-major tf32 operands) instead of the plain 128 B swizzle.
 inline bool make_tensor_map_xcb(CUtensorMap* map, const void* base, bool is_bf16, long long img_stride,
-                                long long row_stride, int B, int C, int HW, int box_x, int box_c, int f32_type = 0,
+                                long long row_stride, int B, int C, int HW, int box_x, int box_c, bool tf32,
                                 bool atom32 = false, bool swizzle64 = false) {
   PFN_encodeTiled enc = get_encode_tiled();
   if (!enc) return false;
@@ -273,7 +273,7 @@ inline bool make_tensor_map_xcb(CUtensorMap* map, const void* base, bool is_bf16
   cuuint32_t box[3] = {(cuuint32_t)box_x, (cuuint32_t)box_c, 1};
   cuuint32_t estr[3] = {1, 1, 1};
   const CUtensorMapDataType dt = is_bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16
-                                 : (f32_type == 1 ? CU_TENSOR_MAP_DATA_TYPE_TFLOAT32 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32);
+                                 : (tf32 ? CU_TENSOR_MAP_DATA_TYPE_TFLOAT32 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32);
   CUresult r = enc(map, dt, 3,
                    const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                    swizzle64 ? CU_TENSOR_MAP_SWIZZLE_64B
@@ -286,9 +286,9 @@ inline bool make_tensor_map_xcb(CUtensorMap* map, const void* base, bool is_bf16
 // Operand tiles whose MN index is the channel (the Gram forward): 128 B rows run along c, so the canonical MN-major tile
 // of R channels x K positions is R/E atoms of [K positions][E channels] (E = 128 B of elements). One 4-D box fetches
 // all atoms of a tile: dims (c within atom, x, atom, b), box E x box_x x (R/E) x 1, landing as [atom][x][E].
-// tf32 MN-major operands need the 32 B-atom flavour of the 128 B swizzle.
+// tf32 MN-major operands need the 32 B-atom flavour of the 128 B swizzle. tf32: as for make_tensor_map_xcb.
 inline bool make_tensor_map_nhwc_mn(CUtensorMap* map, const void* base, bool is_bf16, long long img_stride,
-                                    long long x_stride, int B, int C, int HW, int box_x, int rows, int f32_type) {
+                                    long long x_stride, int B, int C, int HW, int box_x, int rows, bool tf32) {
   PFN_encodeTiled enc = get_encode_tiled();
   if (!enc) return false;
   const long long es = is_bf16 ? 2 : 4;
@@ -301,7 +301,7 @@ inline bool make_tensor_map_nhwc_mn(CUtensorMap* map, const void* base, bool is_
   cuuint32_t box[4] = {(cuuint32_t)E, (cuuint32_t)box_x, (cuuint32_t)(rows / E), 1};
   cuuint32_t estr[4] = {1, 1, 1, 1};
   const CUtensorMapDataType dt = is_bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16
-                                 : (f32_type == 1 ? CU_TENSOR_MAP_DATA_TYPE_TFLOAT32 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32);
+                                 : (tf32 ? CU_TENSOR_MAP_DATA_TYPE_TFLOAT32 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32);
   CUresult r = enc(map, dt, 4, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                    is_bf16 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B,
                    CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
@@ -310,7 +310,7 @@ inline bool make_tensor_map_nhwc_mn(CUtensorMap* map, const void* base, bool is_
 // The same tensor as a 3-D map (c, x, b) with a box of box_c x box_x x 1 and the plain 128 B swizzle: K-major operand
 // tiles whose K index is the channel (the backward's F operand: [x rows][128 B of channels]) and the NHWC gradient store.
 inline bool make_tensor_map_nhwc_cxb(CUtensorMap* map, const void* base, bool is_bf16, long long img_stride,
-                                     long long x_stride, int B, int C, int HW, int box_c, int box_x, int f32_type,
+                                     long long x_stride, int B, int C, int HW, int box_c, int box_x, bool tf32,
                                      bool swizzle64 = false) {
   PFN_encodeTiled enc = get_encode_tiled();
   if (!enc) return false;
@@ -323,7 +323,7 @@ inline bool make_tensor_map_nhwc_cxb(CUtensorMap* map, const void* base, bool is
   cuuint32_t box[3] = {(cuuint32_t)box_c, (cuuint32_t)box_x, 1};
   cuuint32_t estr[3] = {1, 1, 1};
   const CUtensorMapDataType dt = is_bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16
-                                 : (f32_type == 1 ? CU_TENSOR_MAP_DATA_TYPE_TFLOAT32 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32);
+                                 : (tf32 ? CU_TENSOR_MAP_DATA_TYPE_TFLOAT32 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32);
   CUresult r = enc(map, dt, 3, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                    swizzle64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);

@@ -35,10 +35,6 @@ int gh_sm_count(void);
 /* Launch tuning, process-wide. Known names (unknown name or value outside the allowed set: GH_ERR_BAD_ARG):
  *   "gram_fwd_pair", "gram_bwd_pair"   -1 = CTA-pair (TMA-staged) kernels whenever TMA can describe the tensors (default),
  *                                      0 = never (ld.global-fed kernels), 1 = same as -1
- *   "gram_fwd_producer_warps"          0 = auto, 8, 16        "gram_fwd_epilogue_warps"   0 = auto, 4, 8   (ld.global family)
- *   "gram_bwd_variant"                 1 = transposed product with gathered F^T tiles, 2 = F as an MN-major operand (default)
- *   "gram_bwd_nhw"                     x-tile width of variant 2: 0 = auto, 128, 256
- *   "gram_bwd_producer_warps"          8 or 16 (variant 2, x-tile width 256)
  *   "gram_bwd_nt"                      0 = plan the x-tile width of the pair backward; 64..256 (multiple of 16) forces it
  *   "gram_bwd_stages"                  0 = by shape; a*16 + b = A / F ring depths of the pair backward (a >= 4)
  *   "gram_bwd_ats"                     pooled pair backward with the generated gradient tile in tensor memory (the MMAs read
@@ -46,8 +42,6 @@ int gh_sm_count(void);
  *                                      accumulators hold the A ring, -1 = for C >= 512 only (default)
  *   "gram_bwd_ch"                      K chunks per ring stage of that form (MMAs per iteration of the issuing thread / 4):
  *                                      0 = as many as fit, at most 2 (default), 1, 2
- *   "tma_f32_type"                     tensor-map type for fp32 features: 1 = TFLOAT32 (round to nearest, default), 0 = FLOAT32
- *   "attn_gemm"                        ld.global attention family: 1 = tcgen05 split-bf16 GEMMs (default), 0 = fp32 FMA kernels
  *   "tgemm_tn"                         tile width of the TMA-fed attention GEMMs: 0 = planned (default), 128, 256
  *   "pdl"                              1 = programmatic dependent launch along the attention kernel chain (default), 0 = off */
 int gh_set_option(const char* name, int value);
@@ -155,8 +149,7 @@ int gh_normalize_u8(const unsigned char* src, float* dst, long long images, int 
 /* The GEMM the attention entry points are built from, exposed for testing and reuse:
  *   D[m*ldd + n] = sum_k A[m*a_sm + k*a_sk] * B[k*b_sk + n*b_sn] (+ bias[n]),   fp32 in, fp32 out.
  * Runs on tcgen05 with split-bf16 operands (hi*hi + hi*lo + lo*hi, fp32 accumulate: ~1e-5 relative) when each operand
- * is contiguous along one of its two axes with 16 B aligned rows and N >= 64; otherwise (and with option
- * "attn_gemm" = 0) on the fp32 FMA kernel. Stands in for the F.linear / matmul calls inside
+ * is contiguous along one of its two axes with 16 B aligned rows and N >= 64; otherwise on the fp32 FMA kernel. Stands in for the F.linear / matmul calls inside
  * torch.nn.functional.multi_head_attention_forward that the reference reaches through self.attention (:58). */
 int gh_gemm_f32(const float* A, long long a_sm, long long a_sk, const float* B, long long b_sk, long long b_sn,
                 const float* bias, float* D, long long ldd, int M, int N, int K, void* stream);

@@ -53,7 +53,11 @@ def test_argument_validation_without_gpu(library):
     # a layout that is neither x-contiguous nor c-contiguous is refused
     assert library.gh_gram_pool_fwd(dummy, 0, 256 * 64 * 2, 128, 2, 1, 256, 64, 32, dummy, 0, 1, 0, 0, None) == _lib.GH_ERR_BAD_ARG
     assert library.gh_set_option(b"no_such_option", 1) == _lib.GH_ERR_BAD_ARG
-    assert library.gh_set_option(b"gram_fwd_producer_warps", 12) == _lib.GH_ERR_BAD_ARG
+    assert library.gh_set_option(b"gram_bwd_ch", 3) == _lib.GH_ERR_BAD_ARG
+    # retired knobs are unknown names now, even with the value that used to be their default
+    for name, value in ((b"gram_fwd_producer_warps", 0), (b"gram_fwd_epilogue_warps", 0), (b"gram_bwd_variant", 2),
+                        (b"gram_bwd_nhw", 0), (b"gram_bwd_producer_warps", 8), (b"tma_f32_type", 1), (b"attn_gemm", 1)):
+        assert library.gh_set_option(name, value) == _lib.GH_ERR_BAD_ARG, name
     assert library.gh_attn_head_bwd_workspace(4, 3, 64) == 2 * 4 * 64 + 3 * 4 * 3 * 64
     # Multi-PatchGAN head and inference-plan entries
     assert library.gh_patch_gram_workspace(6, 256, 64) == 6 * 256 * 64 * 20

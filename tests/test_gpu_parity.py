@@ -147,47 +147,6 @@ def test_split_bf16_gemm_all_layouts(ops, M, N, K):
             assert float((got.double() - ref).norm() / ref.norm()) <= 2e-5, (a_t, b_t)
 
 
-def test_gram_backward_variants_agree(ops):
-    from heuristique_style_transfer_code_b200 import _lib
-    torch.manual_seed(0)
-    x = torch.relu(torch.randn(3, 512, 784, device="cuda"))
-    dd = torch.randn(3, 1, 1024, device="cuda")
-    ref = O.gram_pool_backward(npf(x), 32, npf(dd[:, 0]))
-    try:
-        _lib.lib().gh_set_option(b"gram_bwd_pair", 0)
-        for variant, nhw, npw in [(1, 0, 16), (2, 128, 8), (2, 256, 8), (2, 256, 16)]:
-            lib = _lib.lib()
-            assert lib.gh_set_option(b"gram_bwd_variant", variant) == 0
-            assert lib.gh_set_option(b"gram_bwd_nhw", nhw) == 0
-            assert lib.gh_set_option(b"gram_bwd_producer_warps", npw) == 0
-            df = ops.gram_pool_bwd(x, 32, dd, 0)
-            assert O.rel_err(npf(df), ref) <= 6e-3, (variant, nhw, npw)
-    finally:
-        _lib.lib().gh_set_option(b"gram_bwd_variant", 2)
-        _lib.lib().gh_set_option(b"gram_bwd_nhw", 0)
-        _lib.lib().gh_set_option(b"gram_bwd_producer_warps", 8)
-        _lib.lib().gh_set_option(b"gram_bwd_pair", -1)
-
-
-def test_producer_warp_variants_agree(ops):
-    from heuristique_style_transfer_code_b200 import _lib
-    torch.manual_seed(0)
-    x = torch.relu(torch.randn(4, 512, 784, device="cuda"))
-    outs = []
-    for npw, nepi in ((8, 0), (16, 4), (16, 8)):
-        assert _lib.lib().gh_set_option(b"gram_fwd_producer_warps", npw) == 0
-        assert _lib.lib().gh_set_option(b"gram_fwd_epilogue_warps", nepi) == 0
-        desc = torch.empty((4, 1, 1024), device="cuda")
-        ops.KSPLIT = 1
-        with kernel_path("ldg"):
-            ops.gram_pool_fwd_(x, 32, desc, 0)
-        ops.KSPLIT = 0
-        outs.append(desc.clone())
-    _lib.lib().gh_set_option(b"gram_fwd_producer_warps", 0)
-    _lib.lib().gh_set_option(b"gram_fwd_epilogue_warps", 0)
-    assert torch.equal(outs[0], outs[1]) and torch.equal(outs[0], outs[2])   # same summation order -> bit identical
-
-
 @pytest.mark.parametrize("B,C,HW,ksplit", [(1, 64, 3136, 1), (2, 256, 784, 1), (2, 512, 196, 1), (1, 64, 3136, 0),
                                            (2, 320, 100, 1), (1, 256, 196, 1)])
 @pytest.mark.parametrize("path", PATHS)

@@ -288,15 +288,12 @@ def timing():
     import torch
     from heuristique_style_transfer_code_b200 import ops
     peaks = json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json"))) if os.path.exists(os.path.join(ROOT, "MEASURED_PEAKS.json")) else {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0}
-    from heuristique_style_transfer_code_b200 import _lib
     g = 32
     for (B, C, HW) in [(256, 256, 3136), (256, 512, 784), (256, 1024, 196), (16, 256, 3136), (1, 256, 12544)]:
         x = torch.relu(torch.randn(B, C, HW, device="cuda"))
         desc = torch.empty(B, 3, g * g, device="cuda")
         dd = torch.randn(B, 3, g * g, device="cuda")
-        for (npw, nepi, ks) in [(16, 4, 1), (16, 8, 1), (8, 0, 1), (0, 0, 0)]:
-            _lib.lib().gh_set_option(b"gram_fwd_producer_warps", npw)
-            _lib.lib().gh_set_option(b"gram_fwd_epilogue_warps", nepi)
+        for ks in (1, 0):
             ops.KSPLIT = ks
             for _ in range(3):
                 ops.gram_pool_fwd_(x, g, desc, 0)
@@ -310,32 +307,23 @@ def timing():
             ms = ev[0].elapsed_time(ev[1]) / n
             by = B * C * HW * 4 + B * g * g * 4
             fl = B * C * (C + 1) * HW
-            print(f"fwd B={B} C={C} HW={HW} npw={npw} nepi={nepi} ksplit={ks}: {ms*1e3:8.1f} us  {by/ms/1e6:8.1f} GB/s ({by/ms/1e6/peaks['hbm_gbs']:.2f} of HBM)"
+            print(f"fwd B={B} C={C} HW={HW} ksplit={ks}: {ms*1e3:8.1f} us  {by/ms/1e6:8.1f} GB/s ({by/ms/1e6/peaks['hbm_gbs']:.2f} of HBM)"
                   f"  {fl/ms/1e9:8.1f} TFLOP/s sym ({fl/ms/1e9/peaks['bf16_tflops']:.2f} of tensor)")
         ops.KSPLIT = 0
-        _lib.lib().gh_set_option(b"gram_fwd_producer_warps", 0)
-        _lib.lib().gh_set_option(b"gram_fwd_epilogue_warps", 0)
-        for (variant, nhw, bnpw) in [(2, 128, 8), (2, 256, 8), (2, 256, 16)]:
-            _lib.lib().gh_set_option(b"gram_bwd_variant", variant)
-            _lib.lib().gh_set_option(b"gram_bwd_nhw", nhw)
-            _lib.lib().gh_set_option(b"gram_bwd_producer_warps", bnpw)
-            for _ in range(3):
-                ops.gram_pool_bwd(x, g, dd, 0)
-            torch.cuda.synchronize()
-            ev = [torch.cuda.Event(enable_timing=True) for _ in range(2)]
-            n = 10
-            ev[0].record()
-            for _ in range(n):
-                ops.gram_pool_bwd(x, g, dd, 0)
-            ev[1].record(); torch.cuda.synchronize()
-            ms = ev[0].elapsed_time(ev[1]) / n
-            by = 2 * B * C * HW * 4
-            fl = 2 * B * C * C * HW
-            print(f"bwd B={B} C={C} HW={HW} variant={variant} nhw={nhw} npw={bnpw}: {ms*1e3:8.1f} us  {by/ms/1e6:8.1f} GB/s ({by/ms/1e6/peaks['hbm_gbs']:.2f} of HBM)"
-                  f"  {fl/ms/1e9:8.1f} TFLOP/s ({fl/ms/1e9/peaks['bf16_tflops']:.2f} of tensor)")
-        _lib.lib().gh_set_option(b"gram_bwd_variant", 2)
-        _lib.lib().gh_set_option(b"gram_bwd_nhw", 0)
-        _lib.lib().gh_set_option(b"gram_bwd_producer_warps", 8)
+        for _ in range(3):
+            ops.gram_pool_bwd(x, g, dd, 0)
+        torch.cuda.synchronize()
+        ev = [torch.cuda.Event(enable_timing=True) for _ in range(2)]
+        n = 10
+        ev[0].record()
+        for _ in range(n):
+            ops.gram_pool_bwd(x, g, dd, 0)
+        ev[1].record(); torch.cuda.synchronize()
+        ms = ev[0].elapsed_time(ev[1]) / n
+        by = 2 * B * C * HW * 4
+        fl = 2 * B * C * C * HW
+        print(f"bwd B={B} C={C} HW={HW}: {ms*1e3:8.1f} us  {by/ms/1e6:8.1f} GB/s ({by/ms/1e6/peaks['hbm_gbs']:.2f} of HBM)"
+              f"  {fl/ms/1e9:8.1f} TFLOP/s ({fl/ms/1e9/peaks['bf16_tflops']:.2f} of tensor)")
         # torch reference ops on the same GPU (fp32 bmm + div + pool), for scale
         xf = x
         for _ in range(2):
@@ -347,32 +335,29 @@ def timing():
         ev[1].record(); torch.cuda.synchronize()
         print(f"torch fp32 bmm+div+pool C={C} HW={HW}: {ev[0].elapsed_time(ev[1])/3*1e3:8.1f} us")
         del x, desc, dd, G, P
-    # attention head, both GEMM back ends
+    # attention head (tcgen05 split-bf16 GEMMs)
     for Bq in (256, 512, 1):
         E, L, nc = 1024, 3, 4
         desc = torch.randn(Bq, L, E, device="cuda", requires_grad=True)
         mha = torch.nn.MultiheadAttention(E, 1).cuda(); lin = torch.nn.Linear(E, nc).cuda()
         ps = [mha.in_proj_weight, mha.in_proj_bias, mha.out_proj.weight, mha.out_proj.bias, lin.weight, lin.bias]
-        for mode in (1, 0):
-            _lib.lib().gh_set_option(b"attn_gemm", mode)
-            def fb():
-                emb, logits = ops.attention_head(desc, *ps)
-                return emb, logits
-            for _ in range(2):
-                e_, l_ = fb(); (l_.sum() + e_.sum()).backward()
-            torch.cuda.synchronize()
-            ev = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
-            ev[0].record()
-            for _ in range(5):
-                e_, l_ = fb()
-            ev[1].record()
-            for _ in range(5):
-                e_, l_ = fb(); (l_.sum() + e_.sum()).backward()
-            ev[2].record(); torch.cuda.synchronize()
-            f_us = ev[0].elapsed_time(ev[1]) / 5 * 1e3
-            fb_us = ev[1].elapsed_time(ev[2]) / 5 * 1e3
-            print(f"attn B={Bq} gemm={'tcgen05 split-bf16' if mode else 'fp32 SIMT'}: fwd {f_us:8.1f} us   fwd+bwd {fb_us:8.1f} us")
-        _lib.lib().gh_set_option(b"attn_gemm", 1)
+        def fb():
+            emb, logits = ops.attention_head(desc, *ps)
+            return emb, logits
+        for _ in range(2):
+            e_, l_ = fb(); (l_.sum() + e_.sum()).backward()
+        torch.cuda.synchronize()
+        ev = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
+        ev[0].record()
+        for _ in range(5):
+            e_, l_ = fb()
+        ev[1].record()
+        for _ in range(5):
+            e_, l_ = fb(); (l_.sum() + e_.sum()).backward()
+        ev[2].record(); torch.cuda.synchronize()
+        f_us = ev[0].elapsed_time(ev[1]) / 5 * 1e3
+        fb_us = ev[1].elapsed_time(ev[2]) / 5 * 1e3
+        print(f"attn B={Bq}: fwd {f_us:8.1f} us   fwd+bwd {fb_us:8.1f} us")
     return True
 
 
@@ -382,7 +367,7 @@ def _opt(name, value):
     assert rc == 0, (name, value, rc)
 
 
-def _pair_fwd_case(B, C, HW, g, dtype="f32", ksplit=0, f32_type=0, relu=True):
+def _pair_fwd_case(B, C, HW, g, dtype="f32", ksplit=0, relu=True):
     import torch
     from heuristique_style_transfer_code_b200 import ops
     from oracle import head_fp64 as O
@@ -393,7 +378,6 @@ def _pair_fwd_case(B, C, HW, g, dtype="f32", ksplit=0, f32_type=0, relu=True):
     if dtype == "bf16":
         x = x.bfloat16()
     _opt("gram_fwd_pair", 1)
-    _opt("tma_f32_type", f32_type)
     desc = torch.full((B, 2, g * g), float("nan"), device="cuda")
     ops.KSPLIT = ksplit
     ops.gram_pool_fwd_(x, g, desc, 1)
@@ -406,7 +390,7 @@ def _pair_fwd_case(B, C, HW, g, dtype="f32", ksplit=0, f32_type=0, relu=True):
         errs[model] = O.rel_err(got, O.descriptors([xf], g, operand_rounding=model)[:, 0])
     untouched = bool(torch.isnan(desc[:, 0]).all())
     best = min(v for k, v in errs.items() if k != "exact") if dtype != "bf16" else errs["exact"]
-    print(f"pair-fwd B={B} C={C} HW={HW} g={g} {dtype} ksplit={ksplit} f32_type={f32_type}: " +
+    print(f"pair-fwd B={B} C={C} HW={HW} g={g} {dtype} ksplit={ksplit}: " +
           " ".join(f"{k}={v:.2e}" for k, v in errs.items()) + f" other-slice-untouched={untouched}", flush=True)
     return errs["exact"] < 1e-3 and best < 2e-5 and untouched
 
@@ -421,10 +405,9 @@ def pair_fwd_min():
 @case
 def pair_fwd():
     ok = True
-    for f32_type in (0, 1):
-        ok &= _pair_fwd_case(2, 256, 3136, 32, f32_type=f32_type)
-        ok &= _pair_fwd_case(3, 512, 784, 32, f32_type=f32_type)
-        ok &= _pair_fwd_case(2, 1024, 196, 32, f32_type=f32_type)
+    ok &= _pair_fwd_case(2, 256, 3136, 32)
+    ok &= _pair_fwd_case(3, 512, 784, 32)
+    ok &= _pair_fwd_case(2, 1024, 196, 32)
     ok &= _pair_fwd_case(2, 256, 3136, 32, dtype="bf16")
     ok &= _pair_fwd_case(3, 512, 784, 32, dtype="bf16")
     ok &= _pair_fwd_case(2, 1024, 200, 32, dtype="bf16")
@@ -465,7 +448,7 @@ def pair_fwd_dense():
     return ok
 
 
-def _pair_bwd_case(B, C, HW, g, dtype="f32", f32_type=0):
+def _pair_bwd_case(B, C, HW, g, dtype="f32"):
     import torch
     from heuristique_style_transfer_code_b200 import ops
     from oracle import head_fp64 as O
@@ -475,7 +458,6 @@ def _pair_bwd_case(B, C, HW, g, dtype="f32", f32_type=0):
         x = x.bfloat16()
     dd = torch.randn(B, 2, g * g, device="cuda")
     _opt("gram_bwd_pair", 1)
-    _opt("tma_f32_type", f32_type)
     df = ops.gram_pool_bwd(x, g, dd, 1)
     torch.cuda.synchronize()
     xf = _np(x)
@@ -485,7 +467,7 @@ def _pair_bwd_case(B, C, HW, g, dtype="f32", f32_type=0):
     df_old = ops.gram_pool_bwd(x, g, dd, 1)
     torch.cuda.synchronize()
     e2 = O.rel_err(_np(df), _np(df_old))
-    print(f"pair-bwd B={B} C={C} HW={HW} g={g} {dtype} f32_type={f32_type}: rel_err vs fp64={e0:.3e} vs tf32-trunc-F fp64={e1:.3e} vs legacy kernel={e2:.3e}", flush=True)
+    print(f"pair-bwd B={B} C={C} HW={HW} g={g} {dtype}: rel_err vs fp64={e0:.3e} vs tf32-trunc-F fp64={e1:.3e} vs legacy kernel={e2:.3e}", flush=True)
     return e0 < 3e-3
 
 
@@ -499,10 +481,9 @@ def pair_bwd_min():
 @case
 def pair_bwd():
     ok = True
-    for f32_type in (0, 1):
-        ok &= _pair_bwd_case(2, 256, 3136, 32, f32_type=f32_type)
-        ok &= _pair_bwd_case(2, 512, 784, 32, f32_type=f32_type)
-        ok &= _pair_bwd_case(2, 1024, 196, 32, f32_type=f32_type)
+    ok &= _pair_bwd_case(2, 256, 3136, 32)
+    ok &= _pair_bwd_case(2, 512, 784, 32)
+    ok &= _pair_bwd_case(2, 1024, 196, 32)
     ok &= _pair_bwd_case(2, 256, 3136, 32, dtype="bf16")
     ok &= _pair_bwd_case(2, 1024, 200, 32, dtype="bf16")
     ok &= _pair_bwd_case(40, 256, 784, 32)
