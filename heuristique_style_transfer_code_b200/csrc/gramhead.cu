@@ -784,8 +784,8 @@ int gh_gram_mse_blocks(long long n) {
 
 int gh_gram_mse(const float* G, const float* G_target, long long n, float* dG, float* partial, void* stream) {
   if (!G || !G_target || !dG || !partial || n <= 0) return GH_ERR_BAD_ARG;
-  if (n % 4 != 0 || ((uintptr_t)G | (uintptr_t)G_target | (uintptr_t)dG) % 16 != 0) return GH_ERR_UNSUPPORTED;
-  gram_mse_kernel<<<gh_gram_mse_blocks(n), kMseThreads, 0, (cudaStream_t)stream>>>(G, G_target, dG, partial, n / 4,
+  if (((uintptr_t)G | (uintptr_t)G_target | (uintptr_t)dG) % 16 != 0) return GH_ERR_UNSUPPORTED;
+  gram_mse_kernel<<<gh_gram_mse_blocks(n), kMseThreads, 0, (cudaStream_t)stream>>>(G, G_target, dG, partial, n,
                                                                                    1.0f / (float)n);
   return (int)cudaGetLastError();
 }

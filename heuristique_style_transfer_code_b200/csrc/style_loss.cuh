@@ -13,19 +13,27 @@ namespace gh {
 constexpr int kMseThreads = 256;
 constexpr int kMseMaxBlocks = 1024;      // partial sums (the caller adds them up in a fixed order)
 
-// partial[blockIdx.x] = sum over this block's elements of (G - Gt)^2 * inv_n ;  dG = 2 * inv_n * (G - Gt).  n4 = n / 4.
+// partial[blockIdx.x] = sum over this block's elements of (G - Gt)^2 * inv_n ;  dG = 2 * inv_n * (G - Gt).
+// float4 steps over the first 4 * (n / 4) elements; the n % 4 left (B*C*C with odd C and B) are block 0's.
 __global__ void __launch_bounds__(kMseThreads) gram_mse_kernel(const float* __restrict__ G, const float* __restrict__ Gt,
                                                                float* __restrict__ dG, float* __restrict__ partial,
-                                                               long long n4, float inv_n) {
+                                                               long long n, float inv_n) {
   __shared__ float red[kMseThreads / 32];
   float acc = 0.f;
   const float coef = 2.f * inv_n;
+  const long long n4 = n >> 2;
   for (long long i = (long long)blockIdx.x * kMseThreads + threadIdx.x; i < n4; i += (long long)gridDim.x * kMseThreads) {
     const float4 a = *reinterpret_cast<const float4*>(G + 4 * i);
     const float4 b = *reinterpret_cast<const float4*>(Gt + 4 * i);
     const float4 d = make_float4(a.x - b.x, a.y - b.y, a.z - b.z, a.w - b.w);
     acc = fmaf(d.x, d.x, fmaf(d.y, d.y, fmaf(d.z, d.z, fmaf(d.w, d.w, acc))));
     *reinterpret_cast<float4*>(dG + 4 * i) = make_float4(coef * d.x, coef * d.y, coef * d.z, coef * d.w);
+  }
+  if (blockIdx.x == 0 && threadIdx.x < (int)(n - 4 * n4)) {
+    const long long i = 4 * n4 + threadIdx.x;
+    const float d = G[i] - Gt[i];
+    acc = fmaf(d, d, acc);
+    dG[i] = coef * d;
   }
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);

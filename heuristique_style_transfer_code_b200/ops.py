@@ -223,7 +223,26 @@ def gram_pool_bwd(x: torch.Tensor, g: int, d_desc: torch.Tensor, l: int) -> torc
 
 
 def gram_dense_bwd(x: torch.Tensor, d_gram: torch.Tensor) -> torch.Tensor:
+    """-> dF = (dG + dG^T) F / HW, in the layout gram_pool_bwd returns.
+
+    The backward kernels take C % 16 == 0 only (gh_gram_dense_bwd refuses other C). For other C (e.g. 3, 17, 100) F's
+    channels and dG's rows and columns are zero-padded to the next multiple of 16 here, and the first C channels of the
+    padded gradient are returned: padded channels add exact zeros to every sum of (dG + dG^T) F, so the result is the
+    unpadded one. This costs a copy of F and dG; the ResNet stages (C a multiple of 64) never take it. The pooled backward
+    is not padded (extra channels would move the pooling bins): style_descriptor sends such stages here through
+    adaptive_pool_bwd."""
     d_gram = d_gram.contiguous().float()
+    c = x.shape[1]
+    if c % 16:
+        b, cp = x.shape[0], (c + 15) // 16 * 16
+        xp = torch.zeros((b, cp, x[0, 0].numel()), device=x.device, dtype=x.dtype)
+        xp[:, :c] = x.reshape(b, c, -1)
+        dgp = torch.zeros((b, cp, cp), device=d_gram.device, dtype=torch.float32)
+        dgp[:, :c, :c] = d_gram
+        df = gram_dense_bwd(xp, dgp)[:, :c]
+        if x.dim() == 4 and is_channels_last(x):       # the layout _grad_buffer gives channels_last features
+            return df.reshape(x.shape).contiguous(memory_format=torch.channels_last)
+        return df.contiguous()
     rc, df = _gram_bwd_call(_lib.lib().gh_gram_dense_bwd, "gram_dense_bwd", x, (d_gram.data_ptr(),), d_gram.numel() * 4)
     check(rc, "gh_gram_dense_bwd")
     return df

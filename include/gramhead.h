@@ -247,7 +247,7 @@ int gh_attn_head_bwd(const float* desc, const float* W_in, const float* W_out, c
  * element-wise part of `loss.backward()` (functions/functions_RESNET50_Truncate_Gram_Attention.py:291-295):
  *   partial[i] = sum over block i's elements of (G - G_target)^2 / n     (loss = sum_i partial[i], i < gh_gram_mse_blocks(n))
  *   dG         = 2 (G - G_target) / n                                      (d loss / d G; feed it to gh_gram_dense_bwd)
- * G, G_target, dG: n = B*C*C fp32 elements, 16 B aligned, n % 4 == 0. */
+ * G, G_target, dG: n = B*C*C fp32 elements, 16 B aligned (any n). */
 int gh_gram_mse_blocks(long long n);
 int gh_gram_mse(const float* G, const float* G_target, long long n, float* dG, float* partial, void* stream);
 

@@ -55,7 +55,7 @@ def gram(features: np.ndarray) -> np.ndarray:
     f = np.asarray(features, dtype=np.float64)
     b, c = f.shape[:2]
     f = f.reshape(b, c, -1)
-    return np.einsum("bck,bdk->bcd", f, f) / f.shape[2]
+    return np.einsum("bck,bdk->bcd", f, f, optimize=True) / f.shape[2]
 
 
 def pool_bins(c: int, g: int):
@@ -76,7 +76,7 @@ def pool_matrix(c: int, g: int) -> np.ndarray:
 def adaptive_pool(gmat: np.ndarray, g: int) -> np.ndarray:
     """(B, C, C) -> (B, g, g)."""
     m = pool_matrix(gmat.shape[-1], g)
-    return np.einsum("ic,bcd,jd->bij", m, np.asarray(gmat, dtype=np.float64), m)
+    return np.einsum("ic,bcd,jd->bij", m, np.asarray(gmat, dtype=np.float64), m, optimize=True)
 
 
 def descriptors(features: Sequence[np.ndarray], g: int, operand_rounding: Optional[str] = None) -> np.ndarray:
@@ -156,8 +156,8 @@ def gram_pool_backward(features: np.ndarray, g: int, d_pooled: np.ndarray) -> np
     f = f.reshape(b, c, -1)
     m = pool_matrix(c, g)
     dp = np.asarray(d_pooled, dtype=np.float64).reshape(b, g, g)
-    dg = np.einsum("ic,bij,jd->bcd", m, dp, m)
-    df = np.einsum("bcd,bdk->bck", dg + dg.transpose(0, 2, 1), f) / f.shape[2]
+    dg = np.einsum("ic,bij,jd->bcd", m, dp, m, optimize=True)
+    df = np.einsum("bcd,bdk->bck", dg + dg.transpose(0, 2, 1), f, optimize=True) / f.shape[2]
     return df.reshape(shape)
 
 
@@ -167,7 +167,7 @@ def gram_dense_backward(features: np.ndarray, d_gram: np.ndarray) -> np.ndarray:
     b, c = shape[:2]
     f = f.reshape(b, c, -1)
     dg = np.asarray(d_gram, dtype=np.float64)
-    return (np.einsum("bcd,bdk->bck", dg + dg.transpose(0, 2, 1), f) / f.shape[2]).reshape(shape)
+    return (np.einsum("bcd,bdk->bck", dg + dg.transpose(0, 2, 1), f, optimize=True) / f.shape[2]).reshape(shape)
 
 
 def style_loss_and_grad(features: np.ndarray, target_gram: np.ndarray):

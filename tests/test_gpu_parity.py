@@ -1,10 +1,13 @@
 """Parity of the sm_100a kernels against the oracle, through the C ABI (ops.py is a thin ctypes layer over it).
 
-Two kernel families sit behind every Gram entry point and both are tested explicitly (`path`):
-  * "ldg"  - single-CTA kernels whose producer warps convert fp32 -> bf16 (round to nearest even) on the way to smem;
+Behind every Gram entry point sit two kernel families, forced here one at a time (`path`):
+  * "ldg"  - single-CTA kernels whose producer warps convert fp32 -> bf16 (round to nearest even) on the way to smem,
+             with four loaders (fp32 / bf16, vector / scalar loads) chosen by the tensor's alignment;
   * "pair" - CTA-pair (cta_group::2) kernels with TMA-staged operands: bf16 features feed kind::f16 as they are,
              fp32 features feed kind::tf32, rounded to the nearest tf32 by the TMA unit (TFLOAT32 tensor maps);
   * "auto" - whatever the library picks for the shape (the shipped default).
+This file feeds fresh tensors at the shipped shapes. tests/test_gpu_gram_routes.py covers the routes a tensor's layout
+selects (strided and misaligned views, every loader, ragged channel counts) and checks which kernel ran.
 
 Tolerances (written next to each assert):
   * Gram / descriptor vs the fp64 oracle on fp32 inputs:            normwise rel. err <= 1e-3  (task statement)
