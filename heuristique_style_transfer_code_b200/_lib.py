@@ -49,6 +49,8 @@ _SIGNATURES = {
     "gh_attn_head_bwd": (c_int, [_P] * 10 + [c_int] * 4 + [_P] * 8 + [_P]),
     "gh_gram_mse_blocks": (c_int, [c_longlong]),
     "gh_gram_mse": (c_int, [_P, _P, c_longlong, _P, _P, _P]),
+    "gh_gram_mse_images_blocks": (c_int, [c_longlong]),
+    "gh_gram_mse_images": (c_int, [_P, _P, c_int, c_longlong, _P, _P, _P]),
     "gh_split_bf16": (c_int, [_P, _P, c_longlong, c_longlong, _P]),
     "gh_gemm_planes": (c_int, [_P, c_longlong, c_longlong, c_int, _P, c_longlong, c_longlong, c_int, _P, _P, _P,
                                 c_longlong, c_longlong, c_int, c_int, c_int, c_int, _P]),

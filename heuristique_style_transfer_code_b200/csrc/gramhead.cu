@@ -790,6 +790,18 @@ int gh_gram_mse(const float* G, const float* G_target, long long n, float* dG, f
   return (int)cudaGetLastError();
 }
 
+int gh_gram_mse_images_blocks(long long n_img) { return gh_gram_mse_blocks(n_img); }
+
+int gh_gram_mse_images(const float* G, const float* G_target, int B, long long n_img, float* dG, float* partial,
+                       void* stream) {
+  if (!G || !G_target || !dG || !partial || B <= 0 || n_img <= 0) return GH_ERR_BAD_ARG;
+  if (B > 65535) return GH_ERR_UNSUPPORTED;                                  // gridDim.y
+  const dim3 grid(gh_gram_mse_blocks(n_img), B);
+  gram_mse_images_kernel<<<grid, kMseThreads, 0, (cudaStream_t)stream>>>(G, G_target, dG, partial, n_img,
+                                                                         1.0f / (float)n_img);
+  return (int)cudaGetLastError();
+}
+
 long long gh_patch_gram_workspace(int L, int B, int D) {
   if (L <= 0 || B <= 0 || D <= 0) return 0;
   return (long long)L * B * D * (kPatchBins + 4);      // bin means (16 floats) + two doubles per plane

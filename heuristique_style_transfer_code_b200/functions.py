@@ -478,27 +478,34 @@ class _StyleIteration:
     At batch 1 the step is ~400 small kernels (cuDNN encoder forward + backward, the dense tcgen05 Gram forward and
     backward, the loss, Adam) and is bound by launch latency, not by any kernel; replaying it as one graph removes
     that. The image, the target Gram and the optimiser state live in static buffers: a new image only copies into them.
-    The arithmetic and its order are the eager loop's (reference functions/...:283-299)."""
+    The arithmetic and its order are the eager loop's (reference functions/...:283-299).
 
-    def __init__(self, model, encoder, device, learning_rate, use_graph=True):
+    `images` = N > 1 optimises N independent images in one step: the loss is the sum of the per-image losses
+    (ops.gram_mse_loss_per_image), so each image gets exactly its own batch-1 d loss / d G; the eval-mode encoder and
+    Adam act on each image separately."""
+
+    def __init__(self, model, encoder, device, learning_rate, use_graph=True, images=1):
         self.model, self.encoder, self.device = model, encoder, torch.device(device)
-        self.noise = torch.zeros((1, 3, 224, 224), device=self.device, requires_grad=True)
+        self.noise = torch.zeros((images, 3, 224, 224), device=self.device, requires_grad=True)
         self.use_graph = bool(use_graph) and self.device.type == 'cuda'
         self.optimizer = torch.optim.Adam([self.noise], lr=learning_rate, capturable=self.use_graph)
         self.mse = nn.MSELoss()
         self.target = None
         self.loss = None
+        self.losses = None
         self.graph = None
 
     def _step(self):
         features = self.encoder(self.noise)
-        if features.is_cuda:       # Gram forward, fused loss + dG pass, Gram backward (ops.gram_mse_loss; reference :286-295)
-            loss = ops.gram_mse_loss(features, self.target)
+        if features.is_cuda:       # Gram forward, fused loss + dG pass, Gram backward (ops.gram_mse_loss_per_image; reference :286-295)
+            losses = ops.gram_mse_loss_per_image(features, self.target)
         else:
-            loss = self.mse(self.model.gram_matrix(features), self.target)
+            gram = self.model.gram_matrix(features)
+            losses = torch.stack([self.mse(gram[b], self.target[b]) for b in range(gram.shape[0])])
+        loss = losses.sum()
         loss.backward()
         self.optimizer.step()
-        return loss
+        return loss, losses
 
     def _reset_optimizer(self):
         for state in self.optimizer.state.values():
@@ -507,7 +514,8 @@ class _StyleIteration:
                     v.zero_()
 
     def start(self, target, noise_init):
-        """New image: target Gram and a fresh noise image; Adam restarts from zero moments (a new optimiser upstream)."""
+        """New images: target Grams (N, C, C) and fresh noise (N, 3, 224, 224); Adam restarts from zero moments (a new
+        optimiser upstream)."""
         if self.target is None:
             self.target = target.detach().clone()
         else:
@@ -524,53 +532,114 @@ class _StyleIteration:
             self.optimizer.zero_grad(set_to_none=True)
             self.graph = torch.cuda.CUDAGraph()
             with torch.cuda.graph(self.graph):
-                self.loss = self._step()
+                self.loss, self.losses = self._step()
         with torch.no_grad():
             self.noise.copy_(noise_init)
         self._reset_optimizer()
 
-    def step(self):
-        """Runs one iteration and returns the loss as a Python float (the only synchronisation, as upstream)."""
+    def _run(self):
         if self.graph is not None:
             self.graph.replay()
-            return self.loss.item()
-        self.optimizer.zero_grad()
-        return self._step().item()
+        else:
+            self.optimizer.zero_grad()
+            self.loss, self.losses = self._step()
+
+    def step(self):
+        """Runs one iteration and returns the loss (summed over the images) as a Python float (the only
+        synchronisation, as upstream)."""
+        self._run()
+        return self.loss.item()
+
+    def step_losses(self):
+        """Runs one iteration and returns the N per-image losses (before the Adam step) as Python floats, from one
+        synchronisation."""
+        self._run()
+        return self.losses.tolist()
+
+
+def _style_images_per_step(images_per_step, device):
+    """images_per_step, or $GRAMHEAD_STYLE_IMAGES when it is None (1 when that is unset too)."""
+    if images_per_step is None:
+        env = os.environ.get("GRAMHEAD_STYLE_IMAGES", "").strip()
+        try:
+            images_per_step = int(env) if env else 1
+        except ValueError:
+            raise ValueError(f"GRAMHEAD_STYLE_IMAGES={env!r} is not an integer") from None
+    images_per_step = int(images_per_step)
+    if images_per_step < 1:
+        raise ValueError(f"images_per_step must be >= 1, got {images_per_step}")
+    if images_per_step > 1 and torch.device(device).type != 'cuda':
+        raise ValueError("images_per_step > 1 needs a CUDA device")
+    return images_per_step
+
+
+def _optimise_chunk(runner, target, noise0, threshold, num_iterations):
+    """Steps runner's N images from noise0 until each one's loss has gone below `threshold` or `num_iterations` ran out.
+    -> (results (N, 3, 224, 224), reached): reached[b] is the iteration at which image b's pre-step loss was first below
+    threshold (None if never) and results[b] the noise after that step -- what upstream saves after its `break` -- or
+    after the last step. A converged image keeps being stepped with the others; its result is copied out on the stream
+    before the next step, so it no longer changes."""
+    runner.start(target, noise0)
+    noise = runner.noise.detach()
+    result = torch.empty_like(noise)
+    reached = [None] * noise.shape[0]
+    for iteration in range(num_iterations):
+        for b, loss in enumerate(runner.step_losses()):
+            if reached[b] is None and loss < threshold:
+                reached[b] = iteration
+                result[b].copy_(noise[b])
+        if None not in reached:
+            break
+    for b, it in enumerate(reached):
+        if it is None:
+            result[b].copy_(noise[b])
+    return result, reached
 
 
 def style_transfer(model, data_loader, device, save_dir, layers=None, threshold=1e-4, num_iterations=500,
-                   learning_rate=0.01, use_graph=True):
+                   learning_rate=0.01, use_graph=True, images_per_step=None):
     """For every image: optimise a noise image with Adam so that the dense Gram of the first `layers` encoder children
     matches the image's (MSE), stop below `threshold`, save original|result under save_dir/style_transfer_<date>/<label>
     (:247-314). Both Gram evaluations and the gradient through them go through model.gram_matrix(), i.e. the dense
     tcgen05 forward/backward kernels; on a CUDA device the whole iteration is replayed from one CUDA graph
-    (`use_graph=False` runs the eager loop, same arithmetic)."""
+    (`use_graph=False` runs the eager loop, same arithmetic).
+
+    `images_per_step` (default: $GRAMHEAD_STYLE_IMAGES, else 1) optimises that many images of a loader batch together,
+    each with its own loss, Adam state and stopping point: image b's result is the noise after the first iteration whose
+    loss was below `threshold`, as in the one-image loop, and the chunk runs until every image got there or
+    `num_iterations` ran out. The random noise, the printed lines and the files are those of the one-image loop; the
+    images differ from it only by the encoder's batch-size-dependent rounding."""
+    per_step = _style_images_per_step(images_per_step, device)
     model.eval()
     out_root = os.path.join(save_dir, f'style_transfer_{datetime.now().strftime("%Y-%m-%d")}')
     os.makedirs(out_root, exist_ok=True)
     mean = torch.tensor([0.485, 0.456, 0.406], device=device)
     std = torch.tensor([0.229, 0.224, 0.225], device=device)
     encoder = nn.Sequential(*list(model.truncated_encoder.children())[:layers]).to(device)
-    runner = _StyleIteration(model, encoder, device, learning_rate, use_graph=use_graph)
+    runners = {}                                      # one per chunk size: the full chunk and a smaller last one
     for inputs, labels in data_loader:
         inputs, labels = inputs.to(device), labels.to(device)
-        for i, image in enumerate(inputs):
-            image = image.unsqueeze(0)
+        # file names use the index within the loader batch (as upstream), so a chunk never spans two batches
+        for first in range(0, inputs.size(0), per_step):
+            chunk = inputs[first:first + per_step]
+            n = chunk.size(0)
             with torch.no_grad():
-                target = model.gram_matrix(encoder(image))
-            class_dir = os.path.join(out_root, str(labels[i].item()))
-            os.makedirs(class_dir, exist_ok=True)
-            runner.start(target, torch.randn((1, 3, 224, 224), device=device))
-            for iteration in range(num_iterations):
-                if runner.step() < threshold:
-                    print(f"Seuil atteint pour l'image {i}, itération {iteration}")
-                    break
-            noise = runner.noise
-            result = denormalize(noise.detach().cpu().squeeze(), mean, std).clamp_(0, 1).numpy().transpose(1, 2, 0)
-            original = denormalize(image.detach().cpu().squeeze(), mean, std).clamp_(0, 1).numpy().transpose(1, 2, 0)
-            save_path = os.path.join(class_dir, f'style_transfer_{i}.png')
-            _save_side_by_side(save_path, np.hstack((original, result)))
-            print(f"Style transféré pour l'image {i}, sauvegardée à {save_path}")
+                target = model.gram_matrix(encoder(chunk))
+            noise0 = torch.cat([torch.randn((1, 3, 224, 224), device=device) for _ in range(n)])   # upstream's draws
+            if n not in runners:
+                runners[n] = _StyleIteration(model, encoder, device, learning_rate, use_graph=use_graph, images=n)
+            result, reached = _optimise_chunk(runners[n], target, noise0, threshold, num_iterations)
+            for b in range(n):
+                i = first + b
+                if reached[b] is not None:
+                    print(f"Seuil atteint pour l'image {i}, itération {reached[b]}")
+                class_dir = os.path.join(out_root, str(labels[i].item()))
+                os.makedirs(class_dir, exist_ok=True)
+                res = denormalize(result[b].cpu(), mean, std).clamp_(0, 1).numpy().transpose(1, 2, 0)
+                original = denormalize(chunk[b].detach().cpu(), mean, std).clamp_(0, 1).numpy().transpose(1, 2, 0)
+                save_path = os.path.join(class_dir, f'style_transfer_{i}.png')
+                _save_side_by_side(save_path, np.hstack((original, res)))
+                print(f"Style transféré pour l'image {i}, sauvegardée à {save_path}")
 
 
 # ---------------------------------------------------------------------------------------------------------------------

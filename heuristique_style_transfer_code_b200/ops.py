@@ -523,6 +523,48 @@ def gram_mse_loss(x: torch.Tensor, target: torch.Tensor) -> torch.Tensor:
     return _GramMSE.apply(x, target)
 
 
+class _GramMSEPerImage(torch.autograd.Function):
+    """[mse_loss(gram_matrix(x[b]), target[b]) for b] as one differentiable op: dense Gram forward, one pass for the B
+    losses and d (sum_b loss_b) / d G (gh_gram_mse_images), dense Gram backward. Image b's dG is the one a batch-1
+    gram_mse_loss computes for it, so several style-transfer images step together with their own gradients."""
+
+    @staticmethod
+    def forward(ctx, x, target):
+        ctx.meta = (tuple(x.shape), x.dtype, is_channels_last(x) and not nhwc_native(x))
+        if ctx.meta[2]:
+            x = nhwc_to_nchw(x)
+        gram = gram_dense_fwd(x)
+        target = target.detach().contiguous().float()
+        if target.shape != gram.shape:
+            raise GramHeadError(f"gramhead: target Gram {tuple(target.shape)} does not match {tuple(gram.shape)}")
+        b, c, _ = gram.shape
+        n = c * c
+        lib = _lib.lib()
+        k = lib.gh_gram_mse_images_blocks(n)
+        d_gram = torch.empty_like(gram)
+        partial = torch.empty((b, k), device=gram.device, dtype=torch.float32)
+        with torch.cuda.device(x.device), _Timed(f"gram_mse_images[B={b},n={n}]", 1, x.device, bytes=3 * b * n * 4,
+                                                 flops=3 * b * n, kind="style"):
+            rc = lib.gh_gram_mse_images(gram.data_ptr(), target.data_ptr(), b, n, d_gram.data_ptr(), partial.data_ptr(),
+                                        _stream_ptr(x))
+        check(rc, "gh_gram_mse_images")
+        ctx.save_for_backward(x, d_gram)
+        return partial.sum(1)
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        x, d_gram = ctx.saved_tensors
+        df = gram_dense_bwd(x, d_gram * grad_out.view(-1, 1, 1))   # all ones under losses.sum().backward()
+        if df.dim() == 4:
+            return df.to(ctx.meta[1]), None
+        return grad_like_activation(df, *ctx.meta), None
+
+
+def gram_mse_loss_per_image(x: torch.Tensor, target: torch.Tensor) -> torch.Tensor:
+    """(B,) losses mean((gram_matrix(x)[b] - target[b])^2): x (B, C, H, W) activations, target (B, C, C)."""
+    return _GramMSEPerImage.apply(x, target)
+
+
 class _StyleDescriptor(torch.autograd.Function):
     """L stage activations -> (B, L, g*g) pooled-Gram descriptors (the attention's input, batch-major)."""
 

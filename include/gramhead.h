@@ -251,6 +251,18 @@ int gh_attn_head_bwd(const float* desc, const float* W_in, const float* W_out, c
 int gh_gram_mse_blocks(long long n);
 int gh_gram_mse(const float* G, const float* G_target, long long n, float* dG, float* partial, void* stream);
 
+/* The same loss with one value per image, for several style-transfer images optimised in one step (the reference's loop
+ * of functions/functions_RESNET50_Truncate_Gram_Attention.py:283-299 runs each image's `mse_loss(noise_gram,
+ * original_gram)` and `loss.backward()` on its own, :291-295). G, G_target, dG: (B, C, C) fp32, n_img = C*C, k =
+ * gh_gram_mse_images_blocks(n_img) (= gh_gram_mse_blocks(n_img)):
+ *   partial[b*k + i] = sum over block i of image b of (G - G_target)^2 / n_img     (mse_b = sum_i partial[b*k + i])
+ *   dG               = 2 (G - G_target) / n_img                                    (d (sum_b mse_b) / d G)
+ * Image b's partials and dG slice are bitwise what gh_gram_mse gives on a 16 B-aligned copy of that image alone. Any
+ * n_img: images that do not start on a 16 B boundary (n_img % 4 != 0) are read with scalar loads. B <= 65535. */
+int gh_gram_mse_images_blocks(long long n_img);
+int gh_gram_mse_images(const float* G, const float* G_target, int B, long long n_img, float* dG, float* partial,
+                       void* stream);
+
 /* ---- Attention head on TMA-fed tensor-core GEMMs (the default whenever E % 64 == 0, E <= 1024, L <= 8, nc <= 16) -------
  * Same reference lines as gh_attn_head_fwd / gh_attn_head_bwd (Models/...Attention.py:56-61 and its autograd), other
  * operand format: every matrix that feeds a linear layer travels as "split planes" -- two bf16 matrices of the same
