@@ -681,6 +681,33 @@ int gh_preprocess_frame(const unsigned char* frame, long long pitch_bytes, int H
   return (int)cudaGetLastError();
 }
 
+static_assert(sizeof(GhFrameDesc) == 80, "GhFrameDesc is mirrored by streaming.FRAME_DESC_DTYPE");
+
+int gh_preprocess_frames_smem(int OW, int span_rows) {
+  if (OW <= 0 || span_rows <= 0) return GH_ERR_BAD_ARG;
+  const long long bytes = 3LL * OW * span_rows;
+  return bytes > kFramesMaxSmem ? GH_ERR_UNSUPPORTED : (int)bytes;
+}
+
+int gh_preprocess_frames(const GhFrameDesc* frames, int N, int OH, int OW, int band_rows, int span_rows, const int* tables,
+                         int hkmax, int vkmax, unsigned char* out, void* stream) {
+  if (!frames || !tables || !out) return GH_ERR_BAD_ARG;
+  if (N <= 0 || OH <= 0 || OW <= 0 || band_rows <= 0 || hkmax <= 0 || vkmax <= 0 || span_rows < vkmax) return GH_ERR_BAD_ARG;
+  const int smem = gh_preprocess_frames_smem(OW, span_rows);
+  if (smem < 0) return smem;
+  const int bands = (int)((OH + (long long)band_rows - 1) / band_rows);
+  if (N > 65535 || bands > 65535) return GH_ERR_UNSUPPORTED;
+  if (smem > 48 * 1024) {
+    const cudaError_t e = cudaFuncSetAttribute(preprocess_frames_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    if (e != cudaSuccess) return (int)e;
+  }
+  FramesParams p;
+  p.frames = frames; p.tables = tables; p.out = out;
+  p.OH = OH; p.OW = OW; p.band_rows = band_rows; p.span_rows = span_rows; p.hkmax = hkmax; p.vkmax = vkmax;
+  preprocess_frames_kernel<<<dim3(bands, N), kFramesThreads, smem, (cudaStream_t)stream>>>(p);
+  return (int)cudaGetLastError();
+}
+
 int gh_normalize_u8(const unsigned char* src, float* dst, long long images, int channels, long long hw,
                     const float* mean_host, const float* std_host, void* stream) {
   if (!src || !dst || !mean_host || !std_host || images <= 0 || hw <= 0) return GH_ERR_BAD_ARG;

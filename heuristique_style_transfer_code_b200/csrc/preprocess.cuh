@@ -13,6 +13,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include "../../include/gramhead.h"
 
 namespace gh {
 
@@ -71,6 +72,90 @@ __global__ void __launch_bounds__(256) preprocess_frame_kernel(const PreprocPara
     const int src = p.bgr ? 2 - c : c;
     const float v = (float)preproc_clip8(acc[src]) / 255.0f;          // ToTensor
     o[c * plane] = (v - p.mean[c]) / p.std[c];                        // Normalize (IEEE division: no fast-math)
+  }
+}
+
+// ---- several frames per launch, into one uint8 batch (streaming.FrameBatchPipeline) ------------------------------------
+// N frames, each with its own size, pitch, channel order and tables (GhFrameDesc, include/gramhead.h), resampled to one
+// common (OH, OW) and written as a dense (N, 3, OH, OW) uint8 batch in RGB order: clip8 of the vertical sum, the byte that
+// preprocess_frame_kernel divides by 255 and normalises. The model applies ToTensor + Normalize to it bit for bit as that
+// kernel does (to_tensor_normalize), so the batch carries the same information in a quarter of the bytes.
+// preprocess_frame_kernel recomputes every horizontal tap sum once per output row that uses its input row (vy_size of
+// them: ~6 at 1080p -> 448, ~17 at 2160p -> Resize(256)). Here a CTA owns (band of `band_rows` output rows, frame): it
+// filters the band's input rows horizontally once, rounds them to uint8 into shared memory, then filters those vertically.
+// Same integer operations in the same order as preprocess_frame_kernel, so the same bytes. A band whose input rows exceed
+// the `span_rows` rows of shared memory is done as several runs of consecutive output rows, each of which fits (one
+// output row always does: span_rows >= vkmax), so the host's choice of band height is a matter of speed only.
+struct FramesParams {
+  const GhFrameDesc* frames;    // [N]
+  const int* tables;            // the packed tables the descriptors' offsets point into
+  uint8_t* out;                 // (N, 3, OH, OW)
+  int OH, OW, band_rows, span_rows, hkmax, vkmax;
+};
+
+constexpr int kFramesThreads = 256;
+constexpr int kFramesMaxSmem = 227 * 1024;
+
+__global__ void __launch_bounds__(kFramesThreads) preprocess_frames_kernel(const FramesParams p) {
+  extern __shared__ uint8_t hrows[];     // [span_rows][3][OW]: horizontally filtered input rows, output channel order
+  const GhFrameDesc d = p.frames[blockIdx.y];
+  const int OW = p.OW;
+  const int* __restrict__ hx_min = p.tables + d.hx_min;
+  const int* __restrict__ hx_size = p.tables + d.hx_size;
+  const int* __restrict__ vy_min = p.tables + d.vy_min;
+  const int* __restrict__ vy_size = p.tables + d.vy_size;
+  const long long plane = (long long)p.OH * OW;
+  uint8_t* __restrict__ out = p.out + (long long)blockIdx.y * 3 * plane;
+  const int band_end = min(p.OH, (int)(blockIdx.x + 1) * p.band_rows);
+  for (int r = blockIdx.x * p.band_rows; r < band_end;) {
+    // output rows [r, re) and the input rows [ylo, yhi) they read: the longest run that fits in shared memory
+    int ylo = __ldg(vy_min + r), yhi = ylo + __ldg(vy_size + r), re = r + 1;
+    for (; re < band_end; ++re) {
+      const int y0 = __ldg(vy_min + re);
+      const int lo = min(ylo, y0), hi = max(yhi, y0 + __ldg(vy_size + re));
+      if (hi - lo > p.span_rows) break;
+      ylo = lo;
+      yhi = hi;
+    }
+    const int items = (yhi - ylo) * OW;
+    for (int i = threadIdx.x; i < items; i += kFramesThreads) {
+      const int yy = i / OW, ox = i - yy * OW;
+      const int x0 = __ldg(hx_min + ox), nx = __ldg(hx_size + ox);
+      const int* __restrict__ hk = p.tables + d.hk + (long long)ox * p.hkmax;
+      const uint8_t* __restrict__ row = d.frame + (long long)(ylo + yy) * d.pitch + (long long)x0 * 3;
+      int h0 = 1 << (kPreprocPrecisionBits - 1), h1 = h0, h2 = h0;
+      for (int k = 0; k < nx; ++k) {
+        const int c = __ldg(hk + k);
+        h0 += (int)__ldg(row + 3 * k) * c;
+        h1 += (int)__ldg(row + 3 * k + 1) * c;
+        h2 += (int)__ldg(row + 3 * k + 2) * c;
+      }
+      uint8_t* s = hrows + (long long)yy * 3 * OW + ox;
+      s[0] = (uint8_t)preproc_clip8(d.bgr ? h2 : h0);     // output channel c holds input channel bgr ? 2 - c : c
+      s[OW] = (uint8_t)preproc_clip8(h1);
+      s[2 * OW] = (uint8_t)preproc_clip8(d.bgr ? h0 : h2);
+    }
+    __syncthreads();
+    const int outs = (re - r) * OW;
+    for (int i = threadIdx.x; i < outs; i += kFramesThreads) {
+      const int dy = i / OW, ox = i - dy * OW, oy = r + dy;
+      const int y0 = __ldg(vy_min + oy) - ylo, ny = __ldg(vy_size + oy);
+      const int* __restrict__ vk = p.tables + d.vk + (long long)oy * p.vkmax;
+      int a0 = 1 << (kPreprocPrecisionBits - 1), a1 = a0, a2 = a0;
+      for (int j = 0; j < ny; ++j) {
+        const int kv = __ldg(vk + j);
+        const uint8_t* s = hrows + (long long)(y0 + j) * 3 * OW + ox;
+        a0 += (int)s[0] * kv;
+        a1 += (int)s[OW] * kv;
+        a2 += (int)s[2 * OW] * kv;
+      }
+      uint8_t* o = out + (long long)oy * OW + ox;
+      o[0] = (uint8_t)preproc_clip8(a0);
+      o[plane] = (uint8_t)preproc_clip8(a1);
+      o[2 * plane] = (uint8_t)preproc_clip8(a2);
+    }
+    __syncthreads();
+    r = re;
   }
 }
 

@@ -754,3 +754,124 @@ def run_camera(model, transform, class_names, save_video, save_dir, prob_thresho
     if display:
         cv2.destroyAllWindows()
     return times
+
+
+def _frame_batch_spec(model, transform, who):
+    """The transform as the batched frame kernel reproduces it; ValueError when it cannot (there is no host fallback)."""
+    from .streaming import parse_transform
+    if torch.device(model.device).type != "cuda":
+        raise ValueError(f"{who} needs the model on a CUDA device")
+    if parse_transform(transform) is None:
+        raise ValueError(f"{who} needs a Resize [+ CenterCrop] + ToTensor + Normalize transform")
+
+
+def run_cameras(model, transform, class_names, captures, save_video, save_dir, prob_threshold, measure_time,
+                display=False, max_frames=None):
+    """run_camera for several cameras in one process: each step reads one frame from every capture, classifies them all
+    in one forward (streaming.FrameBatchPipeline: one slot per capture, shaped by its first frame) and overlays the label
+    on each frame as run_camera does. save_video writes save_dir/camera_<i>_output.avi per stream; measure_time writes
+    save_dir/times_cameras.json, the time of each step (all streams). Stops when any capture fails to read, after
+    `max_frames` steps, or on 'q' when displaying. Returns the step times.
+    Only the GPU path exists: a model off CUDA or a transform the kernel cannot reproduce raises ValueError."""
+    captures = list(captures)
+    if not captures:
+        raise ValueError("run_cameras needs at least one capture")
+    if max_frames is not None and max_frames < 0:
+        raise ValueError(f"max_frames must be >= 0, got {max_frames}")
+    _frame_batch_spec(model, transform, "run_cameras")
+    import cv2
+    from .streaming import FrameBatchPipeline
+    model.eval()
+    times = []
+    if not all(cap.isOpened() for cap in captures):
+        print("Error: Unable to open the cameras")
+        for cap in captures:
+            cap.release()
+        return times
+    pipe, writers, steps = None, [], 0
+    with torch.no_grad():
+        while max_frames is None or steps < max_frames:
+            frames = []
+            for cap in captures:
+                ok, frame = cap.read()
+                if not ok:
+                    break
+                frames.append(frame)
+            if len(frames) < len(captures):
+                print(f"Error: Unable to read the image from camera {len(frames)}")
+                break
+            if pipe is None:
+                pipe = FrameBatchPipeline.from_transform(model, transform, [f.shape for f in frames])
+                if save_video:
+                    os.makedirs(save_dir, exist_ok=True)
+                    writers = [cv2.VideoWriter(os.path.join(save_dir, f"camera_{i}_output.avi"),
+                                               cv2.VideoWriter_fourcc(*'XVID'), 20.0, (f.shape[1], f.shape[0]))
+                               for i, f in enumerate(frames)]
+            start = time.time()
+            probabilities = pipe(frames)
+            times.append(time.time() - start)
+            steps += 1
+            for i, (frame, probs) in enumerate(zip(frames, probabilities)):
+                best = int(np.argmax(probs))
+                prob = probs[best]
+                name = class_names[best] if prob >= prob_threshold else "Unknown"
+                cv2.putText(frame, f"Pred: {name}, Prob: {prob:.4f}", (10, 25), cv2.FONT_HERSHEY_SIMPLEX, 0.7,
+                            (0, 255, 0), 2)
+                if display:
+                    cv2.imshow(f'Camera {i}', frame)
+                if writers:
+                    writers[i].write(frame)
+            if display and (cv2.waitKey(1) & 0xFF == ord('q')):
+                break
+    if measure_time:
+        os.makedirs(save_dir, exist_ok=True)
+        with open(os.path.join(save_dir, "times_cameras.json"), "w") as f:
+            json.dump(times, f, indent=4)
+        if times:
+            print(f"Average processing time per step ({len(captures)} frames): {np.mean(times)} seconds")
+            print(f"Total processing time: {np.sum(times)} seconds")
+    for cap in captures:
+        cap.release()
+    for w in writers:
+        w.release()
+    if display:
+        cv2.destroyAllWindows()
+    return times
+
+
+def classify_video(model, transform, capture, frames_per_call=16, max_frames=None):
+    """Classifies the frames of `capture` (anything with read(), e.g. cv2.VideoCapture("file.mp4")) `frames_per_call` at a
+    time, in one forward per group (streaming.FrameBatchPipeline; a shorter last group gets a pipeline of its own).
+    Reads until the capture ends or `max_frames` frames. Returns (predictions int64 (F,), probabilities float32 (F,)):
+    the arg-max class of each frame and its softmax probability, in frame order. The capture is not released.
+    Only the GPU path exists: a model off CUDA or a transform the kernel cannot reproduce raises ValueError."""
+    if isinstance(frames_per_call, bool) or not isinstance(frames_per_call, int) or frames_per_call < 1:
+        raise ValueError(f"frames_per_call must be a positive integer, got {frames_per_call!r}")
+    if max_frames is not None and max_frames < 0:
+        raise ValueError(f"max_frames must be >= 0, got {max_frames}")
+    _frame_batch_spec(model, transform, "classify_video")
+    from .streaming import FrameBatchPipeline
+    model.eval()
+    pipes, preds, probs, count = {}, [], [], 0
+    while max_frames is None or count < max_frames:
+        group = []
+        while len(group) < frames_per_call and (max_frames is None or count + len(group) < max_frames):
+            ok, frame = capture.read()
+            if not ok:
+                break
+            group.append(frame)
+        if not group:
+            break
+        n = len(group)
+        if n not in pipes:
+            pipes[n] = FrameBatchPipeline.from_transform(model, transform, [group[0].shape] * n)
+        p = pipes[n](group)
+        best = p.argmax(axis=1)
+        preds.append(best.astype(np.int64))
+        probs.append(p[np.arange(n), best].astype(np.float32))
+        count += n
+        if n < frames_per_call:
+            break
+    if not preds:
+        return np.zeros(0, np.int64), np.zeros(0, np.float32)
+    return np.concatenate(preds), np.concatenate(probs)

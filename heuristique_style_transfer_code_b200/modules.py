@@ -147,9 +147,11 @@ class _TruncatedGramAttentionBase(nn.Module):
             self._plan = plan
         return plan
 
-    def _stage_activations(self, x):
+    def _stage_activations(self, x, *, normalize=None):
+        """normalize: (mean, std) to use in place of input_normalization for this call (streaming.FrameBatchPipeline
+        feeds uint8 batches without changing the model)."""
         x = x.to(self.device)
-        norm = self._input_normalization
+        norm = self._input_normalization if normalize is None else normalize
         if norm is not None and not (x.dtype == torch.uint8 and x.dim() == 4 and x.shape[1] == 3):
             norm = None
         plan = self._inference_plan(x)
@@ -179,8 +181,8 @@ class _TruncatedGramAttentionBase(nn.Module):
             stages.append(x)
         return x, stages
 
-    def _head(self, x):
-        x, stages = self._stage_activations(x)
+    def _head(self, x, *, normalize=None):
+        x, stages = self._stage_activations(x, normalize=normalize)
         if not stages:
             return None, torch.zeros((x.size(0), self.num_classes), requires_grad=True).to(self.device)
         return GramAttentionHead.apply(stages, self.gram_matrix_size, self.attention, self.classifier)

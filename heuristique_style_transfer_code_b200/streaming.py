@@ -197,3 +197,208 @@ class CameraPipeline:
         if spec is None:
             return None
         return cls(model, frame_shape, spec["resize"], spec["crop"], spec["mean"], spec["std"], bgr=bgr, use_graph=use_graph)
+
+
+# ---- several frames per forward ---------------------------------------------------------------------------------------
+# GhFrameDesc of include/gramhead.h, one record per frame slot; the table offsets count int32 elements.
+FRAME_DESC_DTYPE = np.dtype([("frame", "<u8"), ("pitch", "<i8"), ("H", "<i4"), ("W", "<i4"), ("bgr", "<i4"),
+                             ("reserved", "<i4"), ("hx_min", "<i8"), ("hx_size", "<i8"), ("hk", "<i8"), ("vy_min", "<i8"),
+                             ("vy_size", "<i8"), ("vk", "<i8")])
+_TABLE_FIELDS = ("hx_min", "hx_size", "hk", "vy_min", "vy_size", "vk")
+# shared memory a band of gh_preprocess_frames may use when the host picks its height: several CTAs stay resident per SM
+_BAND_SMEM_BUDGET = 48 * 1024
+
+
+def pack_frame_tables(frame_shapes, resize, crop=None):
+    """Resample tables of N frame slots, packed for gh_preprocess_frames.
+
+    Returns dict(out_hw=(oh, ow), tables=int32 array, offsets=(N, 6) int64 (start of hx_min, hx_size, hk, vy_min,
+    vy_size, vk of each slot in `tables`), hkmax, vkmax, rows=[(vy_min, vy_size)] per slot). Coefficient rows are padded
+    with zeros to the largest kmax of the batch. Every slot must resize [and crop] to the same size."""
+    geometry = []
+    for shape in frame_shapes:
+        if len(shape) != 3 or int(shape[2]) != 3 or int(shape[0]) <= 0 or int(shape[1]) <= 0:
+            raise GramHeadError(f"gramhead: frames must be (H, W, 3) uint8, got shape {tuple(shape)}")
+        h, w = int(shape[0]), int(shape[1])
+        rh, rw = _resize_output_size(h, w, resize)
+        top, left, oh, ow = 0, 0, rh, rw
+        if crop is not None:
+            oh, ow = (int(crop), int(crop)) if not isinstance(crop, (tuple, list)) else (int(crop[0]), int(crop[-1]))
+            if oh > rh or ow > rw:
+                raise GramHeadError("gramhead: CenterCrop larger than the resized frame is not supported on the GPU path")
+            top, left = int(round((rh - oh) / 2.0)), int(round((rw - ow) / 2.0))
+        geometry.append((h, w, rh, rw, top, left, oh, ow))
+    if not geometry:
+        raise GramHeadError("gramhead: a frame batch needs at least one frame slot")
+    sizes = sorted({g[6:] for g in geometry})
+    if len(sizes) != 1:
+        raise GramHeadError(f"gramhead: the frames come out of the transform at different sizes {sizes}; one batch needs "
+                            "one size (Resize((h, w)), or a CenterCrop)")
+    oh, ow = sizes[0]
+    hx = [resample_tables(w, rw, left, ow) for h, w, rh, rw, top, left, _, _ in geometry]
+    vy = [resample_tables(h, rh, top, oh) for h, w, rh, rw, top, left, _, _ in geometry]
+    hkmax = max(t[2].shape[1] for t in hx)
+    vkmax = max(t[2].shape[1] for t in vy)
+    parts, offsets, pos = [], [], 0
+    for (x0, xn, xk), (y0, yn, yk) in zip(hx, vy):
+        xk = np.pad(xk, ((0, 0), (0, hkmax - xk.shape[1])))
+        yk = np.pad(yk, ((0, 0), (0, vkmax - yk.shape[1])))
+        row = []
+        for a in (x0, xn, xk, y0, yn, yk):
+            row.append(pos)
+            parts.append(a.ravel())
+            pos += a.size
+        offsets.append(row)
+    return dict(out_hw=(oh, ow), tables=np.concatenate(parts).astype(np.int32), offsets=np.array(offsets, np.int64),
+                hkmax=hkmax, vkmax=vkmax, rows=[(t[0], t[1]) for t in vy])
+
+
+def band_span(rows, band_rows: int) -> int:
+    """The most input rows a band of `band_rows` consecutive output rows (bands start at multiples of band_rows) reads,
+    over every slot; rows: pack_frame_tables(...)["rows"]."""
+    span = 0
+    for y0, yn in rows:
+        starts = np.arange(0, len(y0), band_rows)
+        lo, hi = np.minimum.reduceat(y0, starts), np.maximum.reduceat(y0 + yn, starts)
+        span = max(span, int((hi - lo).max()))
+    return span
+
+
+def max_band_rows(rows, ow: int, budget: int = _BAND_SMEM_BUDGET) -> int:
+    """The tallest band whose input rows fit in `budget` bytes of shared memory (gh_preprocess_frames_smem); 1 when even
+    one output row needs more (one row always runs if the kernel can hold it at all)."""
+    lib = _lib.lib()
+    best = 1
+    for r in range(2, len(rows[0][0]) + 1):
+        smem = lib.gh_preprocess_frames_smem(ow, band_span(rows, r))
+        if smem < 0 or smem > budget:
+            break
+        best = r
+    return best
+
+
+class FrameBatchPipeline:
+    """N frames (H_i, W_i, 3) uint8 numpy -> probabilities (N, num_classes) numpy, one forward for all of them: the
+    CameraPipeline of several cameras or of consecutive video frames. Slot i takes frames of shape frame_shapes[i]; every
+    slot must come out of resize [+ crop] at the same size. The model (either model class, on a CUDA device) is unchanged:
+    it gets the uint8 batch with this transform's Normalize for this call only (the fused uint8 stem on the fp32 inference
+    plan), which is bit for bit the fp32 batch CameraPipeline would give it.
+
+      frames --memcpy--> one pinned arena --one H2D--> gh_preprocess_frames (N frames -> (N, 3, oh, ow) uint8)
+      --> model --> softmax --D2H--> pinned (N, num_classes)
+
+    Everything between the two host buffers is one CUDA graph (use_graph=True), replayed per call."""
+
+    def __init__(self, model, frame_shapes, resize, crop=None, mean=(0.485, 0.456, 0.406), std=(0.229, 0.224, 0.225),
+                 bgr: bool = True, use_graph: bool = True):
+        self.model = model
+        self.device = torch.device(model.device)
+        if self.device.type != "cuda":
+            raise GramHeadError("gramhead: FrameBatchPipeline needs the model on a CUDA device (there is no CPU path)")
+        mean, std = tuple(float(v) for v in mean), tuple(float(v) for v in std)
+        if len(mean) != 3 or len(std) != 3:
+            raise GramHeadError(f"gramhead: Normalize needs 3 means and 3 stds, got {len(mean)} and {len(std)}")
+        self._normalize = (mean, std)
+        packed = pack_frame_tables(frame_shapes, resize, crop)
+        self.frame_shapes = [(int(s[0]), int(s[1]), 3) for s in frame_shapes]
+        self.out_hw, self.bgr = packed["out_hw"], bool(bgr)
+        self._hkmax, self._vkmax, self._rows = packed["hkmax"], packed["vkmax"], packed["rows"]
+        n, dev = len(self.frame_shapes), self.device
+        sizes = [h * w * 3 for h, w, _ in self.frame_shapes]
+        starts = np.concatenate([[0], np.cumsum(sizes)]).astype(np.int64)
+        self._frames_pin = torch.empty(int(starts[-1]), dtype=torch.uint8).pin_memory()
+        arena = self._frames_pin.numpy()
+        self._slots = [arena[starts[i]:starts[i + 1]].reshape(self.frame_shapes[i]) for i in range(n)]
+        self._frames_dev = torch.empty(int(starts[-1]), dtype=torch.uint8, device=dev)
+        desc = np.zeros(n, dtype=FRAME_DESC_DTYPE)
+        desc["frame"] = self._frames_dev.data_ptr() + starts[:-1]
+        desc["pitch"] = [w * 3 for _, w, _ in self.frame_shapes]
+        desc["H"] = [h for h, _, _ in self.frame_shapes]
+        desc["W"] = [w for _, w, _ in self.frame_shapes]
+        desc["bgr"] = int(self.bgr)
+        for j, name in enumerate(_TABLE_FIELDS):
+            desc[name] = packed["offsets"][:, j]
+        self._desc = torch.from_numpy(desc.view(np.uint8).copy()).to(dev)
+        self._tables = torch.from_numpy(packed["tables"]).to(dev)
+        oh, ow = self.out_hw
+        self.max_band_rows = max_band_rows(self._rows, ow)
+        sms = torch.cuda.get_device_properties(dev).multi_processor_count
+        # as tall a band as the budget allows, but not so tall that the grid leaves SMs without two CTAs
+        self.band_rows = max(1, min(self.max_band_rows, -(-n * oh // (2 * sms))))
+        self._input = torch.empty((n, 3, oh, ow), dtype=torch.uint8, device=dev)
+        self._probs_dev = None
+        self._probs_pin = None
+        self._graph = None
+        self._done = torch.cuda.Event()
+        model.eval()
+        with torch.cuda.device(dev), torch.no_grad():
+            self._body()                                  # allocates the output buffers, loads every kernel
+            torch.cuda.synchronize(dev)
+            if use_graph:
+                side = torch.cuda.Stream(device=dev)
+                side.wait_stream(torch.cuda.current_stream(dev))
+                with torch.cuda.stream(side):
+                    for _ in range(2):
+                        self._body()
+                torch.cuda.current_stream(dev).wait_stream(side)
+                torch.cuda.synchronize(dev)
+                graph = torch.cuda.CUDAGraph()
+                with torch.cuda.graph(graph):
+                    self._body()
+                self._graph = graph
+                # the graph holds raw addresses of the model's folded inference plan: keep it alive with the pipeline
+                self._captured_plan = getattr(model, "_plan", None)
+
+    def preprocess_(self, band_rows: Optional[int] = None):
+        """Runs gh_preprocess_frames on the uploaded frames; result in self._input (N, 3, oh, ow) uint8, RGB.
+        band_rows: output rows per CTA, 1 .. max_band_rows (default: self.band_rows)."""
+        r = self.band_rows if band_rows is None else int(band_rows)
+        if not 1 <= r <= self.max_band_rows:
+            raise GramHeadError(f"gramhead: band_rows must be in [1, {self.max_band_rows}], got {band_rows}")
+        oh, ow = self.out_hw
+        span = max(band_span(self._rows, r), self._vkmax)
+        rc = _lib.lib().gh_preprocess_frames(
+            self._desc.data_ptr(), len(self.frame_shapes), oh, ow, r, span, self._tables.data_ptr(), self._hkmax,
+            self._vkmax, self._input.data_ptr(), torch.cuda.current_stream(self.device).cuda_stream)
+        check(rc, "gh_preprocess_frames")
+        return self._input
+
+    def _body(self):
+        self._frames_dev.copy_(self._frames_pin, non_blocking=True)
+        self.preprocess_()
+        out = self.model._head(self._input, normalize=self._normalize)
+        logits = out[1] if isinstance(out, (tuple, list)) else out
+        probs = torch.softmax(logits, dim=1)
+        if self._probs_dev is None:
+            self._probs_dev = torch.empty_like(probs)
+            self._probs_pin = torch.empty(probs.shape, dtype=probs.dtype).pin_memory()
+        self._probs_dev.copy_(probs)
+        self._probs_pin.copy_(self._probs_dev, non_blocking=True)
+
+    def __call__(self, frames) -> np.ndarray:
+        if len(frames) != len(self._slots):
+            raise GramHeadError(f"gramhead: FrameBatchPipeline was built for {len(self._slots)} frames, got {len(frames)}")
+        for i, (frame, shape) in enumerate(zip(frames, self.frame_shapes)):
+            if not isinstance(frame, np.ndarray) or frame.dtype != np.uint8 or frame.shape != shape:
+                got = (getattr(frame, "dtype", type(frame).__name__), tuple(getattr(frame, "shape", ())))
+                raise GramHeadError(f"gramhead: frame {i}: slot {i} takes uint8 frames of shape {shape}, got {got}")
+        for slot, frame in zip(self._slots, frames):
+            np.copyto(slot, frame)
+        with torch.cuda.device(self.device), torch.no_grad():
+            if self._graph is not None:
+                self._graph.replay()
+            else:
+                self._body()
+            self._done.record(torch.cuda.current_stream(self.device))
+        self._done.synchronize()
+        return self._probs_pin.numpy().copy()
+
+    @classmethod
+    def from_transform(cls, model, transform, frame_shapes, bgr: bool = True, use_graph: bool = True):
+        """Pipeline equivalent to `transform` applied to a PIL image of each frame, or None when the transform is not the
+        Resize [+ CenterCrop] + ToTensor + Normalize chain the GPU kernel reproduces."""
+        spec = parse_transform(transform)
+        if spec is None:
+            return None
+        return cls(model, frame_shapes, spec["resize"], spec["crop"], spec["mean"], spec["std"], bgr=bgr,
+                   use_graph=use_graph)

@@ -137,6 +137,35 @@ int gh_preprocess_frame(const unsigned char* frame, long long pitch_bytes, int H
                         int vkmax, const float* mean3_host, const float* std3_host, float* out, int OH, int OW,
                         void* stream);
 
+/* Several camera or video frames per call: the resize [+ centre crop] of gh_preprocess_frame for N frames of any sizes
+ * at once, written as one dense (N, 3, OH, OW) uint8 batch in RGB order -- the rounded bytes gh_preprocess_frame divides
+ * by 255 and normalises, so that ToTensor + Normalize applied to this batch (gh_normalize_u8, or the uint8 stem
+ * gh_stem_conv_pool_u8_nhwc) gives its fp32 output bit for bit. One record per frame, in DEVICE memory (it does not
+ * change between calls, so a CUDA graph can hold it); the table offsets count int elements from `tables`: */
+typedef struct GhFrameDesc {
+  const unsigned char* frame;   /* (H, W, 3) uint8 on the device, `pitch` bytes between rows */
+  long long pitch;
+  int H, W;
+  int bgr;                      /* != 0: channels are B,G,R (OpenCV); the output is RGB either way */
+  int reserved;                 /* 0 */
+  long long hx_min, hx_size;    /* [OW] first contributing input column and their number */
+  long long hk;                 /* [OW][hkmax] 22-bit fixed-point coefficients, rows padded with zeros to hkmax */
+  long long vy_min, vy_size;    /* [OH] the same for rows */
+  long long vk;                 /* [OH][vkmax] */
+} GhFrameDesc;                  /* 80 bytes */
+
+/* frames: [N] descriptors (device). tables: the packed int tables (device). Each CTA resamples `band_rows` output rows of
+ * one frame, holding the horizontally filtered input rows they read in shared memory, at most `span_rows` of them at a
+ * time: span_rows >= vkmax (one output row always fits); a band that needs more input rows is done in several runs, so
+ * any band_rows is correct and the caller picks it for speed (streaming.py: the most input rows any band of that height
+ * needs). out: (N, 3, OH, OW) uint8. N <= 65535 and ceil(OH / band_rows) <= 65535 (GH_ERR_UNSUPPORTED beyond); the
+ * shared memory gh_preprocess_frames_smem(OW, span_rows) must be available (GH_ERR_UNSUPPORTED otherwise). */
+int gh_preprocess_frames(const GhFrameDesc* frames, int N, int OH, int OW, int band_rows, int span_rows, const int* tables,
+                         int hkmax, int vkmax, unsigned char* out, void* stream);
+/* Host-only: the shared-memory bytes of one gh_preprocess_frames CTA holding span_rows filtered rows of width OW;
+ * GH_ERR_BAD_ARG for non-positive sizes, GH_ERR_UNSUPPORTED above what one CTA can have. No GPU needed. */
+int gh_preprocess_frames_smem(int OW, int span_rows);
+
 /* Loader-side counterpart of gh_preprocess_frame: a dense (images, channels, H, W) uint8 batch -> the fp32 batch the
  * reference's loader transforms produce on the host, transforms.ToTensor() + transforms.Normalize(mean, std)
  * (test_RESNET50_Truncate_gram_attention.py:64-65, train_best_RESNET50_Truncate_gram_attention.py:42-43):
