@@ -37,6 +37,8 @@ _SIGNATURES = {
                                      c_int, c_int, _P]),
     "gh_preprocess_frames": (c_int, [_P, c_int, c_int, c_int, c_int, c_int, _P, c_int, c_int, _P, _P]),
     "gh_preprocess_frames_smem": (c_int, [c_int, c_int]),
+    "gh_frame_tables": (c_int, [_P, c_int, _P, c_int, c_int, c_int, c_int, _P, _P, _P]),
+    "gh_frame_tables_stride": (c_longlong, [c_int, c_int, c_int, c_int]),
     "gh_normalize_u8": (c_int, [_P, _P, c_longlong, c_int, c_longlong, _P, _P, _P]),
     "gh_gemm_f32": (c_int, [_P, c_longlong, c_longlong, _P, c_longlong, c_longlong, _P, _P, c_longlong, c_int, c_int,
                              c_int, _P]),

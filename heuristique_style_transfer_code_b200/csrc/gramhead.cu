@@ -708,6 +708,25 @@ int gh_preprocess_frames(const GhFrameDesc* frames, int N, int OH, int OW, int b
   return (int)cudaGetLastError();
 }
 
+long long gh_frame_tables_stride(int OH, int OW, int hkmax, int vkmax) {
+  if (OH <= 0 || OW <= 0 || hkmax <= 0 || vkmax <= 0) return GH_ERR_BAD_ARG;
+  return frame_tables_stride(OH, OW, hkmax, vkmax);
+}
+
+int gh_frame_tables(const long long* geom, int N, const unsigned char* base, int OH, int OW, int hkmax, int vkmax,
+                    int* tables, GhFrameDesc* frames, void* stream) {
+  if (!geom || !base || !tables || !frames) return GH_ERR_BAD_ARG;
+  if (N <= 0 || OH <= 0 || OW <= 0 || hkmax <= 0 || vkmax <= 0) return GH_ERR_BAD_ARG;
+  const long long coords = (long long)OH + OW;
+  if (N > 65535 || coords > 0x7fffffffLL - kFrameTablesThreads) return GH_ERR_UNSUPPORTED;
+  FrameTablesParams p;
+  p.geom = geom; p.base = base; p.tables = tables; p.frames = frames;
+  p.OH = OH; p.OW = OW; p.hkmax = hkmax; p.vkmax = vkmax; p.stride = frame_tables_stride(OH, OW, hkmax, vkmax);
+  const dim3 grid((unsigned)((coords + kFrameTablesThreads - 1) / kFrameTablesThreads), (unsigned)N);
+  frame_tables_kernel<<<grid, kFrameTablesThreads, 0, (cudaStream_t)stream>>>(p);
+  return (int)cudaGetLastError();
+}
+
 int gh_normalize_u8(const unsigned char* src, float* dst, long long images, int channels, long long hw,
                     const float* mean_host, const float* std_host, void* stream) {
   if (!src || !dst || !mean_host || !std_host || images <= 0 || hw <= 0) return GH_ERR_BAD_ARG;

@@ -159,6 +159,78 @@ __global__ void __launch_bounds__(kFramesThreads) preprocess_frames_kernel(const
   }
 }
 
+// ---- the tables of a loader batch, built on the device (functions.gpu_resize_transform) ---------------------------------
+// A loader hands over N decoded images of new sizes in every batch, so the tables preprocess_frames_kernel reads change
+// per batch; streaming.resample_tables builds them in Python one output coordinate at a time (over half a second for 256
+// mixed images). Here one thread owns one output coordinate of one image -- its column (c < OW) or row (c - OW) -- and
+// evaluates Pillow's precompute_coeffs for it in fp64, in Pillow's order of operations, every operation correctly rounded
+// and none contracted (__d*_rn: a fused 1 - |t| * ss or center - support + 0.5 rounds differently), so the int tables are
+// resample_tables' bit for bit. Each image's tables sit at a fixed stride (frame_tables_stride), laid out as the offsets
+// of its GhFrameDesc, which the same launch writes.
+struct FrameTablesParams {
+  const long long* geom;        // [N][7]: H, W, byte offset of the image in `base`, resized rh, rw, crop top, left
+  const uint8_t* base;
+  int* tables;                  // [N][stride]
+  GhFrameDesc* frames;          // [N]
+  int OH, OW, hkmax, vkmax;
+  long long stride;
+};
+
+constexpr int kFrameTablesThreads = 128;
+
+__host__ __device__ inline long long frame_tables_stride(int OH, int OW, int hkmax, int vkmax) {
+  return (2LL + hkmax) * OW + (2LL + vkmax) * OH;
+}
+
+// Pillow's bilinear filter at input index `x` for an output coordinate centred at `center`: max(0, 1 - |(x - center + 0.5) * ss|)
+__device__ __forceinline__ double resample_tap(int x, double center, double ss) {
+  const double w = __dsub_rn(1.0, fabs(__dmul_rn(__dadd_rn(__dsub_rn((double)x, center), 0.5), ss)));
+  return w > 0.0 ? w : 0.0;
+}
+
+__global__ void __launch_bounds__(kFrameTablesThreads) frame_tables_kernel(const FrameTablesParams p) {
+  const long long* g = p.geom + 7LL * blockIdx.y;
+  const int H = (int)g[0], W = (int)g[1];
+  int* t = p.tables + p.stride * blockIdx.y;
+  if (blockIdx.x == 0 && threadIdx.x == 0) {
+    GhFrameDesc d;
+    d.frame = p.base + g[2];
+    d.pitch = 3LL * W;
+    d.H = H; d.W = W; d.bgr = 0; d.reserved = 0;
+    const long long t0 = p.stride * blockIdx.y, v0 = t0 + (2LL + p.hkmax) * p.OW;
+    d.hx_min = t0; d.hx_size = t0 + p.OW; d.hk = t0 + 2LL * p.OW;
+    d.vy_min = v0; d.vy_size = v0 + p.OH; d.vk = v0 + 2LL * p.OH;
+    p.frames[blockIdx.y] = d;
+  }
+  const int c = blockIdx.x * kFrameTablesThreads + threadIdx.x;
+  if (c >= p.OW + p.OH) return;
+  const bool col = c < p.OW;
+  const int in_size = col ? W : H, out_size = (int)(col ? g[4] : g[3]), kmax = col ? p.hkmax : p.vkmax;
+  const int count = col ? p.OW : p.OH, i = col ? c : c - p.OW, xx = i + (int)(col ? g[6] : g[5]);
+  if (!col) t += (2LL + p.hkmax) * p.OW;
+  const double scale = __ddiv_rn((double)in_size, (double)out_size);
+  const double support = scale < 1.0 ? 1.0 : scale;             // filterscale; bilinear support 1.0 * filterscale
+  const double ss = __ddiv_rn(1.0, support);
+  const double center = __dmul_rn(__dadd_rn((double)xx, 0.5), scale);
+  const int lo = max((int)__dadd_rn(__dsub_rn(center, support), 0.5), 0);
+  const int hi = min((int)__dadd_rn(__dadd_rn(center, support), 0.5), in_size);
+  const int n = max(min(hi - lo, kmax), 0);                     // hi - lo <= kmax when kmax is the image's (the host's)
+  double sum = 0.0;
+  for (int x = 0; x < n; ++x) sum = __dadd_rn(sum, resample_tap(x + lo, center, ss));
+  int* k = t + 2LL * count + (long long)i * kmax;
+  for (int x = 0; x < kmax; ++x) {
+    int v = 0;
+    if (x < n) {
+      double w = resample_tap(x + lo, center, ss);
+      if (sum != 0.0) w = __ddiv_rn(w, sum);
+      v = (int)__dadd_rn(__dmul_rn(w, (double)(1 << kPreprocPrecisionBits)), 0.5);
+    }
+    k[x] = v;
+  }
+  t[i] = lo;
+  t[count + i] = n;
+}
+
 // ---- loader-side counterpart: a uint8 image batch normalised on the device -------------------------------------------------
 // The reference's loaders end in ToTensor + Normalize on the host (test_RESNET50_Truncate_gram_attention.py:64-65,
 // train_best_RESNET50_Truncate_gram_attention.py:42-43) and every batch crosses PCIe as fp32: 154 MB for 256 images at

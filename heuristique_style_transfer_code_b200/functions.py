@@ -16,7 +16,7 @@ import torch
 import torch.nn as nn
 import torch.nn.functional as F
 
-from . import ops
+from . import _lib, ops, streaming
 from torch.utils.data import Subset
 
 
@@ -130,6 +130,114 @@ def uint8_transform(resize=256, crop=224):
     return transforms.Compose(steps + [transforms.PILToTensor()])
 
 
+class PackedImages:
+    """A loader batch of decoded RGB images of any sizes, built by GpuResizeTransform.collate in the worker:
+    `pixels`, one flat uint8 tensor holding every (H, W, 3) image back to back; `geometry`, (N, 7) int64 per image
+    (streaming.GEOMETRY_COLUMNS: H, W, byte offset in `pixels`, resized rh, rw, crop top, left); `labels` as the default
+    collate makes them; and what cuda_prefetch needs to resample them: the transform's `resize` / `crop`, the common
+    output size `out_hw` and the largest coefficient counts `kmax` = (hkmax, vkmax). pin_memory() lets
+    DataLoader(pin_memory=True) pin it like any other batch."""
+
+    def __init__(self, pixels, geometry, labels, resize, crop, out_hw, kmax):
+        self.pixels, self.geometry, self.labels = pixels, geometry, labels
+        self.resize, self.crop, self.out_hw, self.kmax = resize, crop, tuple(out_hw), tuple(kmax)
+
+    def __len__(self):
+        return int(self.geometry.shape[0])
+
+    def pin_memory(self):
+        labels = self.labels.pin_memory() if torch.is_tensor(self.labels) else self.labels
+        return PackedImages(self.pixels.pin_memory(), self.geometry.pin_memory(), labels, self.resize, self.crop,
+                            self.out_hw, self.kmax)
+
+    def images(self):
+        """The (H, W, 3) uint8 images, as numpy views of `pixels`."""
+        flat = self.pixels.numpy()
+        return [flat[o:o + h * w * 3].reshape(h, w, 3) for h, w, o in self.geometry[:, :3].tolist()]
+
+    def host_batch(self):
+        """The (N, 3, oh, ow) uint8 batch torchvision's own Resize + CenterCrop + PILToTensor give on the host (CPU runs)."""
+        from PIL import Image
+        from torchvision import transforms
+        steps = [transforms.Resize(self.resize)] + ([transforms.CenterCrop(self.crop)] if self.crop else [])
+        tf = transforms.Compose(steps + [transforms.PILToTensor()])
+        return torch.stack([tf(Image.fromarray(img, "RGB")) for img in self.images()])
+
+
+class GpuResizeTransform:
+    """Loader side of Resize + CenterCrop on the GPU (gpu_resize_transform). As the dataset's `transform` it maps an RGB
+    PIL image to its decoded (H, W, 3) uint8 pixels, without resampling; `.collate` is the DataLoader's collate_fn and
+    packs a batch of them into a PackedImages. cuda_prefetch then uploads the pixels, builds the resample tables on the
+    device and resamples the batch there, bit for bit what Resize(resize) + CenterCrop(crop) + PILToTensor give on the
+    host, before the usual ToTensor + Normalize of uint8 batches."""
+
+    def __init__(self, resize=256, crop=224, interpolation="bilinear", max_size=None):
+        from torchvision.transforms import InterpolationMode
+        if InterpolationMode(interpolation) != InterpolationMode.BILINEAR:
+            raise ValueError(f"gpu_resize_transform: only bilinear interpolation is reproduced on the GPU, got {interpolation!r}")
+        if max_size is not None:
+            raise ValueError("gpu_resize_transform: Resize(max_size=...) is not reproduced on the GPU")
+        pair = lambda v: (int(v), int(v)) if not isinstance(v, (tuple, list)) else (int(v[0]), int(v[-1]))
+        if resize is None or (isinstance(resize, (tuple, list)) and len(resize) not in (1, 2)):
+            raise ValueError(f"gpu_resize_transform: resize must be an int or an (h, w) pair, got {resize!r}")
+        if isinstance(resize, (tuple, list)) and len(resize) == 1:
+            resize = int(resize[0])
+        if crop is None and not isinstance(resize, (tuple, list)):
+            raise ValueError("gpu_resize_transform: Resize(int) without a CenterCrop gives each image its own size; one "
+                             "batch needs one size (give a crop, or resize to an (h, w) pair)")
+        if min(pair(resize)) <= 0 or (crop is not None and min(pair(crop)) <= 0):
+            raise ValueError(f"gpu_resize_transform: sizes must be positive, got resize={resize!r}, crop={crop!r}")
+        if crop is not None:
+            ch, cw = pair(crop)
+            # Resize(int) makes the short side `resize` and the long side at least that
+            lo_h, lo_w = pair(resize)
+            if ch > lo_h or cw > lo_w:
+                raise ValueError(f"gpu_resize_transform: CenterCrop({crop!r}) is larger than Resize({resize!r}) can give "
+                                 "(torchvision would pad); not reproduced on the GPU")
+        self.resize = tuple(int(v) for v in resize) if isinstance(resize, (tuple, list)) else int(resize)
+        self.crop = None if crop is None else pair(crop)
+
+    def __call__(self, img):
+        if getattr(img, "mode", None) != "RGB":
+            raise ValueError(f"gpu_resize_transform: takes RGB PIL images, got {getattr(img, 'mode', type(img).__name__)!r}")
+        return torch.from_numpy(np.array(img, dtype=np.uint8))
+
+    def collate(self, batch):
+        """[(pixels (H, W, 3) uint8, label), ...] -> PackedImages (pixels, geometry, labels built here, in the worker)."""
+        from torch.utils.data import default_collate
+        images = [img for img, _ in batch]
+        for img in images:
+            if not torch.is_tensor(img) or img.dtype != torch.uint8 or img.dim() != 3 or img.shape[2] != 3:
+                raise ValueError("gpu_resize_transform.collate: expects the (H, W, 3) uint8 tensors of its transform")
+        geometry, out_hw = streaming.frame_geometry([tuple(img.shape) for img in images], self.resize, self.crop)
+        sizes = [int(img.numel()) for img in images]
+        offsets = np.concatenate([[0], np.cumsum(sizes)[:-1]]).astype(np.int64)
+        pixels = torch.empty(int(sum(sizes)), dtype=torch.uint8)
+        for img, o, s in zip(images, offsets, sizes):
+            pixels[o:o + s].copy_(img.reshape(-1))
+        geom = torch.tensor([(h, w, int(o), rh, rw, top, left) for (h, w, rh, rw, top, left, _, _), o in zip(geometry, offsets)],
+                            dtype=torch.int64)
+        kmax = (max(streaming.resample_kmax(g[1], g[3]) for g in geometry),
+                max(streaming.resample_kmax(g[0], g[2]) for g in geometry))
+        return PackedImages(pixels, geom, default_collate([label for _, label in batch]), self.resize, self.crop, out_hw,
+                            kmax)
+
+
+def gpu_resize_transform(resize=256, crop=224, interpolation="bilinear", max_size=None):
+    """Opt-in loader transform that moves Resize + CenterCrop (the reference's test_...:62-63) to the GPU, for loaders
+    whose images have any sizes:
+
+        t = functions.gpu_resize_transform(256, 224)
+        loader = DataLoader(ImageFolder(root, transform=t), batch_size=..., collate_fn=t.collate, pin_memory=True)
+
+    The workers only decode; cuda_prefetch (and so train_model / evaluate_model / evaluate_model_test) uploads the
+    decoded pixels, resamples them on the device bit for bit as the host transforms would, and hands on the same
+    (B, 3, oh, ow) batch as a uint8_transform() loader. The upload is the decoded pixels (H * W * 3 bytes per image)
+    rather than the resampled ones. Raises ValueError for what the kernel does not reproduce: another interpolation,
+    max_size, or a crop larger than the resize."""
+    return GpuResizeTransform(resize, crop, interpolation, max_size)
+
+
 def _is_uint8_images(t):
     return torch.is_tensor(t) and t.dtype == torch.uint8 and t.dim() == 4 and 1 <= t.shape[1] <= 4
 
@@ -149,12 +257,20 @@ def cuda_prefetch(batches, device, reuse_buffers=False, normalize="default"):
 
     normalize: (mean, std) applied on the device to every (B, C <= 4, H, W) uint8 tensor of a batch after its upload --
     ToTensor's /255 and Normalize, bit-identical to the host transforms (ops.normalize_u8), for loaders built with
-    uint8_transform(); "default" takes functions.UINT8_NORMALIZE (the reference's ImageNet constants), None disables it."""
+    uint8_transform(); "default" takes functions.UINT8_NORMALIZE (the reference's ImageNet constants), None disables it.
+
+    A PackedImages batch (gpu_resize_transform's collate) is yielded as (images, labels): its decoded pixels and geometry
+    are uploaded, resampled on the device (streaming.resample_images) into a (B, 3, oh, ow) uint8 batch, which `normalize`
+    then treats as any uint8 batch. With reuse_buffers=True its variable-size buffers (pixels, tables) grow with the
+    largest batch seen instead of being allocated per batch. On a CPU device, torchvision's own Resize / CenterCrop /
+    PILToTensor resample the images."""
     device = torch.device(device)
     if normalize == "default":
         normalize = UINT8_NORMALIZE
     if device.type != 'cuda':
         for batch in batches:
+            if isinstance(batch, PackedImages):
+                batch = (batch.host_batch(), batch.labels)
             yield tuple((_normalize_host(t, *normalize) if normalize is not None and _is_uint8_images(t) else t.to(device))
                         if torch.is_tensor(t) else t for t in batch)
         return
@@ -185,6 +301,35 @@ def cuda_prefetch(batches, device, reuse_buffers=False, normalize="default"):
             return ops.normalize_u8(view, *normalize, out=staged(slot, (pos, "fp32"), t.shape, torch.float32))
         return view
 
+    def grown(slot, key, numel, dtype):
+        """A flat buffer of the slot with room for `numel` elements, reallocated (with 1/8 headroom) only to grow."""
+        buf = slots[slot].get(key)
+        if buf is None or buf.numel() < numel:
+            buf = torch.empty(numel + numel // 8, dtype=dtype, device=device)
+            slots[slot][key] = buf
+        return buf[:numel]
+
+    def resample(slot, packed):
+        n, (oh, ow), (hkmax, vkmax) = len(packed), packed.out_hw, packed.kmax
+        tables = frames = None
+        if reuse_buffers:
+            src = grown(slot, "packed", packed.pixels.numel(), torch.uint8)
+            src.copy_(packed.pixels, non_blocking=True)
+            geometry = staged(slot, "geometry", packed.geometry.shape, torch.int64)
+            geometry.copy_(packed.geometry, non_blocking=True)
+            tables = grown(slot, "tables", n * _lib.lib().gh_frame_tables_stride(oh, ow, hkmax, vkmax), torch.int32)
+            frames = grown(slot, "frames", n * streaming.FRAME_DESC_DTYPE.itemsize, torch.uint8)
+            out = staged(slot, "images", (n, 3, oh, ow), torch.uint8)
+        else:
+            src = packed.pixels.to(device, non_blocking=True)
+            geometry = packed.geometry.to(device, non_blocking=True)
+            out = torch.empty((n, 3, oh, ow), dtype=torch.uint8, device=device)
+        streaming.resample_images(src, geometry, packed.geometry.numpy(), out, hkmax, vkmax, tables, frames)
+        if normalize is None:
+            return out
+        return ops.normalize_u8(out, *normalize,
+                                out=staged(slot, "images_fp32", out.shape, torch.float32) if reuse_buffers else None)
+
     def upload(batch):
         nonlocal count
         slot = count % 2
@@ -194,7 +339,11 @@ def cuda_prefetch(batches, device, reuse_buffers=False, normalize="default"):
         with torch.cuda.stream(copy_stream):
             if reuse_buffers and consumed[slot] is not None:
                 copy_stream.wait_event(consumed[slot])       # the batch that last lived in these buffers is done with
-            moved = tuple(place(slot, i, t) if torch.is_tensor(t) else t for i, t in enumerate(batch))
+            if isinstance(batch, PackedImages):
+                labels = batch.labels
+                moved = (resample(slot, batch), place(slot, 1, labels) if torch.is_tensor(labels) else labels)
+            else:
+                moved = tuple(place(slot, i, t) if torch.is_tensor(t) else t for i, t in enumerate(batch))
         done = torch.cuda.Event()
         done.record(copy_stream)
         return moved, done, slot

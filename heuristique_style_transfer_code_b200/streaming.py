@@ -28,6 +28,11 @@ from ._lib import GramHeadError, check
 _PRECISION_BITS = 32 - 8 - 2
 
 
+def resample_kmax(in_size: int, out_size: int) -> int:
+    """Coefficients per output coordinate of the antialiased bilinear resample along one axis (Pillow's ksize)."""
+    return int(math.ceil(max(in_size / out_size, 1.0))) * 2 + 1
+
+
 def resample_tables(in_size: int, out_size: int, first: int = 0, count: Optional[int] = None):
     """Integer tables of the antialiased bilinear resample along one axis, for output coordinates [first, first+count):
     (min[count], size[count], coeff[count, kmax]) as int32 arrays."""
@@ -35,7 +40,7 @@ def resample_tables(in_size: int, out_size: int, first: int = 0, count: Optional
     scale = in_size / out_size
     filterscale = max(scale, 1.0)
     support = filterscale                       # bilinear: support 1.0 * filterscale
-    kmax = int(math.ceil(support)) * 2 + 1
+    kmax = resample_kmax(in_size, out_size)
     lo_a = np.zeros(count, dtype=np.int32)
     n_a = np.zeros(count, dtype=np.int32)
     kk = np.zeros((count, kmax), dtype=np.int32)
@@ -209,12 +214,9 @@ _TABLE_FIELDS = ("hx_min", "hx_size", "hk", "vy_min", "vy_size", "vk")
 _BAND_SMEM_BUDGET = 48 * 1024
 
 
-def pack_frame_tables(frame_shapes, resize, crop=None):
-    """Resample tables of N frame slots, packed for gh_preprocess_frames.
-
-    Returns dict(out_hw=(oh, ow), tables=int32 array, offsets=(N, 6) int64 (start of hx_min, hx_size, hk, vy_min,
-    vy_size, vk of each slot in `tables`), hkmax, vkmax, rows=[(vy_min, vy_size)] per slot). Coefficient rows are padded
-    with zeros to the largest kmax of the batch. Every slot must resize [and crop] to the same size."""
+def frame_geometry(frame_shapes, resize, crop=None):
+    """The geometry of torchvision's Resize(resize) [+ CenterCrop(crop)] for each (H, W, 3) frame shape:
+    ([(h, w, rh, rw, top, left, oh, ow)] per frame, (oh, ow)). Every frame must come out at the same (oh, ow)."""
     geometry = []
     for shape in frame_shapes:
         if len(shape) != 3 or int(shape[2]) != 3 or int(shape[0]) <= 0 or int(shape[1]) <= 0:
@@ -226,7 +228,7 @@ def pack_frame_tables(frame_shapes, resize, crop=None):
             oh, ow = (int(crop), int(crop)) if not isinstance(crop, (tuple, list)) else (int(crop[0]), int(crop[-1]))
             if oh > rh or ow > rw:
                 raise GramHeadError("gramhead: CenterCrop larger than the resized frame is not supported on the GPU path")
-            top, left = int(round((rh - oh) / 2.0)), int(round((rw - ow) / 2.0))
+            top, left = int(round((rh - oh) / 2.0)), int(round((rw - ow) / 2.0))     # half to even, as torchvision
         geometry.append((h, w, rh, rw, top, left, oh, ow))
     if not geometry:
         raise GramHeadError("gramhead: a frame batch needs at least one frame slot")
@@ -234,7 +236,16 @@ def pack_frame_tables(frame_shapes, resize, crop=None):
     if len(sizes) != 1:
         raise GramHeadError(f"gramhead: the frames come out of the transform at different sizes {sizes}; one batch needs "
                             "one size (Resize((h, w)), or a CenterCrop)")
-    oh, ow = sizes[0]
+    return geometry, sizes[0]
+
+
+def pack_frame_tables(frame_shapes, resize, crop=None):
+    """Resample tables of N frame slots, packed for gh_preprocess_frames.
+
+    Returns dict(out_hw=(oh, ow), tables=int32 array, offsets=(N, 6) int64 (start of hx_min, hx_size, hk, vy_min,
+    vy_size, vk of each slot in `tables`), hkmax, vkmax, rows=[(vy_min, vy_size)] per slot). Coefficient rows are padded
+    with zeros to the largest kmax of the batch. Every slot must resize [and crop] to the same size."""
+    geometry, (oh, ow) = frame_geometry(frame_shapes, resize, crop)
     hx = [resample_tables(w, rw, left, ow) for h, w, rh, rw, top, left, _, _ in geometry]
     vy = [resample_tables(h, rh, top, oh) for h, w, rh, rw, top, left, _, _ in geometry]
     hkmax = max(t[2].shape[1] for t in hx)
@@ -275,6 +286,83 @@ def max_band_rows(rows, ow: int, budget: int = _BAND_SMEM_BUDGET) -> int:
             break
         best = r
     return best
+
+
+def band_span_bound(h, rh, band_rows):
+    """An upper bound of band_span from the shapes alone, for images of heights h resized to rh (arrays): output rows
+    y .. y + R - 1 read input rows [int(c(y) - s + 0.5), int(c(y + R - 1) + s + 0.5)) with c(y) = (y + 0.5) * scale and
+    s = max(scale, 1), fewer than (R - 1) * scale + 2 s + 1 of them; one more row absorbs the rounding of those fp64
+    values, and no band reads more than the image's h rows. band_rows: an int, or an array of them (one bound each)."""
+    h, rh = np.asarray(h, dtype=np.int64), np.asarray(rh, dtype=np.int64)
+    scale = h / rh
+    r = np.asarray(band_rows, dtype=np.int64)[..., None]
+    bound = np.ceil((r - 1) * scale) + 2 * np.ceil(np.maximum(scale, 1.0)) + 2
+    return np.minimum(bound, h).max(axis=-1).astype(np.int64)
+
+
+# columns of a loader batch's geometry (functions.PackedImages, gh_frame_tables): per image H, W, the byte offset of its
+# pixels in the packed buffer, the resized rh, rw, and the centre crop's top, left
+GEOMETRY_COLUMNS = ("H", "W", "offset", "rh", "rw", "top", "left")
+_SM_COUNTS = {}
+
+
+def resample_images(pixels: torch.Tensor, geometry: torch.Tensor, geometry_host: np.ndarray, out: torch.Tensor,
+                    hkmax: int, vkmax: int, tables: Optional[torch.Tensor] = None,
+                    frames: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """N RGB images of any sizes, packed in one flat uint8 device buffer, -> Resize [+ CenterCrop] of each as one
+    (N, 3, oh, ow) uint8 batch in `out`, bit for bit torchvision's on the PIL images. The resample tables are built on the
+    device from the geometry (gh_frame_tables), then gh_preprocess_frames resamples; nothing per output coordinate runs
+    on the host. geometry: (N, 7) int64 on the device (GEOMETRY_COLUMNS), geometry_host: the same values on the host
+    (checked here, and used to pick the band height). tables / frames: optional int32 / uint8 device buffers of at least
+    N * gh_frame_tables_stride(...) ints / N * 80 bytes (allocated when None). Runs on the current stream."""
+    lib = _lib.lib()
+    g = np.asarray(geometry_host, dtype=np.int64)
+    n = len(g)
+    if (out.dim() != 4 or out.dtype != torch.uint8 or not out.is_contiguous() or tuple(out.shape[:2]) != (n, 3)
+            or g.shape != (n, 7) or n == 0 or tuple(geometry.shape) != g.shape):
+        raise GramHeadError("gramhead: resample_images needs (N, 7) geometry and a dense (N, 3, oh, ow) uint8 output")
+    for t, dtype in ((pixels, torch.uint8), (geometry, torch.int64)):
+        if t.device != out.device or t.dtype != dtype or not t.is_contiguous():
+            raise GramHeadError("gramhead: resample_images: pixels (uint8) and geometry (int64) must be dense, on out's device")
+    oh, ow = int(out.shape[2]), int(out.shape[3])
+    h, w, off, rh, rw, top, left = g.T
+    if (h.min() <= 0 or w.min() <= 0 or off.min() < 0 or int((off + h * w * 3).max()) > pixels.numel()
+            or (top < 0).any() or (left < 0).any() or (top + oh > rh).any() or (left + ow > rw).any()
+            or max(resample_kmax(a, b) for a, b in zip(w, rw)) > hkmax
+            or max(resample_kmax(a, b) for a, b in zip(h, rh)) > vkmax):
+        raise GramHeadError("gramhead: resample_images: the geometry does not fit the pixels, the output or kmax")
+    stride = lib.gh_frame_tables_stride(oh, ow, hkmax, vkmax)
+    if stride < 0:
+        check(int(stride), "gh_frame_tables_stride")
+    if tables is None:
+        tables = torch.empty(n * stride, dtype=torch.int32, device=out.device)
+    if frames is None:
+        frames = torch.empty(n * FRAME_DESC_DTYPE.itemsize, dtype=torch.uint8, device=out.device)
+    if (tables.numel() < n * stride or tables.dtype != torch.int32 or frames.numel() < n * FRAME_DESC_DTYPE.itemsize
+            or frames.dtype != torch.uint8 or tables.device != out.device or frames.device != out.device):
+        raise GramHeadError("gramhead: resample_images: the tables / frames buffers are too small")
+    dev = out.device
+    if dev not in _SM_COUNTS:
+        _SM_COUNTS[dev] = torch.cuda.get_device_properties(dev).multi_processor_count
+    band, span = images_band_rows(h, rh, oh, ow, vkmax, _SM_COUNTS[dev])
+    with torch.cuda.device(dev):
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        check(lib.gh_frame_tables(geometry.data_ptr(), n, pixels.data_ptr(), oh, ow, hkmax, vkmax, tables.data_ptr(),
+                                  frames.data_ptr(), stream), "gh_frame_tables")
+        check(lib.gh_preprocess_frames(frames.data_ptr(), n, oh, ow, band, span, tables.data_ptr(), hkmax, vkmax,
+                                       out.data_ptr(), stream), "gh_preprocess_frames")
+    return out
+
+
+def images_band_rows(h, rh, oh: int, ow: int, vkmax: int, sms: int):
+    """(band_rows, span_rows) of gh_preprocess_frames for images of heights h resized to rh, from the shapes alone
+    (band_span_bound; the host has no tables): bands as tall as the shared-memory budget allows, but not so tall that the
+    grid leaves SMs without two CTAs."""
+    rows = np.arange(1, oh + 1)
+    spans = np.maximum(band_span_bound(h, rh, rows), vkmax)
+    fits = np.nonzero(3 * ow * spans <= _BAND_SMEM_BUDGET)[0]
+    band = max(1, min(int(fits[-1]) + 1 if fits.size else 1, -(-len(h) * oh // (2 * sms))))
+    return band, int(spans[band - 1])
 
 
 class FrameBatchPipeline:

@@ -166,6 +166,20 @@ int gh_preprocess_frames(const GhFrameDesc* frames, int N, int OH, int OW, int b
  * GH_ERR_BAD_ARG for non-positive sizes, GH_ERR_UNSUPPORTED above what one CTA can have. No GPU needed. */
 int gh_preprocess_frames_smem(int OW, int span_rows);
 
+/* The tables and descriptors of gh_preprocess_frames for a batch of N images of any sizes, built on the device (a loader
+ * has new sizes in every batch). geom: [N][7] long long in DEVICE memory, per image H, W, the byte offset of its (H, W, 3)
+ * RGB pixels (pitch 3 * W) from `base`, its resized size rh, rw and the centre crop's top, left (OH x OW from there;
+ * top + OH <= rh, left + OW <= rw). hkmax / vkmax: at least every image's 2 * ceil(max(W / rw, 1)) + 1, resp. for H / rh.
+ * Writes, per image i, the tables of streaming.resample_tables(W, rw, left, OW) and (H, rh, top, OH) -- bit for bit: fp64
+ * in Pillow's order of operations, none fused -- at tables + i * gh_frame_tables_stride(...), coefficient rows padded
+ * with zeros to hkmax / vkmax, and frames[i] = { base + offset, 3 * W, H, W, RGB, offsets of those tables }.
+ * N <= 65535 (GH_ERR_UNSUPPORTED beyond). */
+int gh_frame_tables(const long long* geom, int N, const unsigned char* base, int OH, int OW, int hkmax, int vkmax,
+                    int* tables, GhFrameDesc* frames, void* stream);
+/* Host-only: the ints of one image's tables in gh_frame_tables' layout, (2 + hkmax) * OW + (2 + vkmax) * OH;
+ * GH_ERR_BAD_ARG for non-positive sizes. */
+long long gh_frame_tables_stride(int OH, int OW, int hkmax, int vkmax);
+
 /* Loader-side counterpart of gh_preprocess_frame: a dense (images, channels, H, W) uint8 batch -> the fp32 batch the
  * reference's loader transforms produce on the host, transforms.ToTensor() + transforms.Normalize(mean, std)
  * (test_RESNET50_Truncate_gram_attention.py:64-65, train_best_RESNET50_Truncate_gram_attention.py:42-43):
