@@ -49,6 +49,13 @@ _SIGNATURES = {
     "gh_patch_gram_workspace": (c_longlong, [c_int, c_int, c_int]),
     "gh_patch_gram_fwd": (c_int, [_P, _P, _P, _P, c_int, c_int, c_int, c_int, _P, _P, _P, _P]),
     "gh_patch_attn_fwd": (c_int, [_P] * 11 + [c_int] * 5 + [_P, _P, _P]),
+    "gh_gemm_f32_fixed": (c_int, [_P, c_longlong, c_longlong, _P, c_longlong, c_longlong, _P, _P, c_longlong, c_int,
+                                   c_int, c_int, _P]),
+    "gh_colsum_f32": (c_int, [_P, c_longlong, c_int, c_int, _P, _P]),
+    "gh_patch_bwd_workspace": (c_longlong, [c_int, c_int, c_int]),
+    "gh_patch_gram_bwd": (c_int, [_P, _P, c_int, c_int, c_int, c_int, _P, _P, _P, _P, _P, _P]),
+    "gh_patch_pool_bwd": (c_int, [_P, _P, _P, _P, _P, _P, c_int, c_int, c_int, c_int, _P, _P]),
+    "gh_patch_attn_bwd": (c_int, [_P] * 12 + [c_int] * 5 + [_P] * 5 + [_P]),
     "gh_attn_head_bwd_workspace": (c_longlong, [c_int, c_int, c_int]),
     "gh_attn_head_bwd": (c_int, [_P] * 10 + [c_int] * 4 + [_P] * 8 + [_P]),
     "gh_gram_mse_blocks": (c_int, [c_longlong]),

@@ -60,13 +60,15 @@ static int choose_ksplit(long long base_units, int nkb, int ctas, bool balance =
 }
 
 // D = A B (+ bias) with strided fp32 operands: tensor-core path when the layout allows it, fp32 FMA kernel otherwise.
+// max_split = 1: no K split, so every output element has one writer and the result is the same bits on every run
+// (both routes then reduce K in a fixed order).
 static cudaError_t gemm_auto(const float* A, long long a_sm, long long a_sk, const float* Bm, long long b_sk,
                              long long b_sn, const float* bias, float* D, long long ldd, int M, int N, int K,
-                             int accumulate, cudaStream_t st) {
+                             int accumulate, cudaStream_t st, int max_split = 0) {
   if (!accumulate && (a_sk == 1 || a_sm == 1) && (b_sk == 1 || b_sn == 1)) {
     const bool a_mn = (a_sk != 1), b_mn = (b_sk != 1);
     cudaError_t e = launch_umma_gemm(A, a_mn, a_mn ? a_sk : a_sm, Bm, b_mn, b_mn ? b_sk : b_sn, bias, D, ldd, M, N, K,
-                                     sm_count_cached(), st);
+                                     sm_count_cached(), st, max_split);
     if (e != cudaErrorNotSupported) return e;
   }
   return launch_sgemm(A, a_sm, a_sk, Bm, b_sk, b_sn, bias, D, ldd, M, N, K, accumulate, st);
@@ -756,6 +758,18 @@ int gh_gemm_f32(const float* A, long long a_sm, long long a_sk, const float* Bm,
   return (int)gemm_auto(A, a_sm, a_sk, Bm, b_sk, b_sn, bias, D, ldd, M, N, K, 0, (cudaStream_t)stream);
 }
 
+int gh_gemm_f32_fixed(const float* A, long long a_sm, long long a_sk, const float* Bm, long long b_sk, long long b_sn,
+                      const float* bias, float* D, long long ldd, int M, int N, int K, void* stream) {
+  if (!A || !Bm || !D || M <= 0 || N <= 0 || K <= 0) return GH_ERR_BAD_ARG;
+  return (int)gemm_auto(A, a_sm, a_sk, Bm, b_sk, b_sn, bias, D, ldd, M, N, K, 0, (cudaStream_t)stream, 1);
+}
+
+int gh_colsum_f32(const float* X, long long ldx, int M, int N, float* out, void* stream) {
+  if (!X || !out || M <= 0 || N <= 0 || ldx < N) return GH_ERR_BAD_ARG;
+  colsum_kernel<<<(N + 31) / 32, dim3(32, 8), 0, (cudaStream_t)stream>>>(X, ldx, out, M, N);
+  return (int)cudaGetLastError();
+}
+
 int gh_maxpool2d_nhwc(const void* in, int dtype, void* out, int B, int H, int W, int C, int k, int stride, int pad,
                       void* stream) {
   if (!in || !out || B <= 0 || H <= 0 || W <= 0 || C <= 0 || k <= 0 || stride <= 0 || pad < 0) return GH_ERR_BAD_ARG;
@@ -909,6 +923,104 @@ int gh_patch_attn_fwd(const float* feat, const float* W_in1, const float* b_in1,
   const int sms = gh_sm_count();
   const int grid = B < 4 * sms ? B : 4 * sms;
   patch_attention_kernel<<<grid, kPatchThreads, smem, (cudaStream_t)stream>>>(p);
+  return (int)cudaGetLastError();
+}
+
+long long gh_patch_bwd_workspace(int L, int B, int D) {
+  if (L <= 0 || B <= 0 || D <= 0) return 0;
+  return (long long)L * B * (D * kPatchBins + kPatchBwdScalars);   // coefficient tables, then 4 scalars per image
+}
+
+int gh_patch_gram_bwd(const int* H, const int* W, int L, int B, int D, int ln_input, const float* d_gram,
+                      const float* d_norm, const float* gram_norm, const float* fwd_workspace, float* bwd_workspace,
+                      void* stream) {
+  if (!H || !W || !d_gram || !d_norm || !gram_norm || !fwd_workspace || !bwd_workspace || L <= 0 || B <= 0 || D <= 0)
+    return GH_ERR_BAD_ARG;
+  if ((uintptr_t)fwd_workspace % 8 != 0 || (uintptr_t)bwd_workspace % 16 != 0) return GH_ERR_BAD_ARG;
+  if (L > kPatchMaxLayers || D > kPatchMaxD || B > 65535) return GH_ERR_UNSUPPORTED;
+  PatchGramParams p{};
+  for (int l = 0; l < L; ++l) {
+    if (H[l] <= 0 || W[l] <= 0) return GH_ERR_BAD_ARG;
+    p.layer[l].H = H[l];
+    p.layer[l].W = W[l];
+  }
+  p.L = L; p.B = B; p.D = D; p.ln_input = ln_input ? 1 : 0;
+  p.gram_norm = const_cast<float*>(gram_norm);        // read: the forward's norms
+  const long long planes = (long long)L * B * D;
+  const double* stats = reinterpret_cast<const double*>(fwd_workspace);   // gh_patch_gram_fwd's layout
+  const float* pooled = fwd_workspace + planes * 4;
+  float* coef = bwd_workspace;
+  float* scal = bwd_workspace + planes * kPatchBins;
+  const size_t smem = ((size_t)D * kPatchBins + (size_t)D * (D + 1) + kPatchBins * kPatchBins) * 4 + 32 * sizeof(double);
+  cudaError_t e = cudaFuncSetAttribute(patch_gram_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return (int)e;
+  patch_gram_bwd_kernel<<<dim3(B, L), kPatchThreads, smem, (cudaStream_t)stream>>>(p, pooled, stats, d_gram, d_norm, coef,
+                                                                                  scal);
+  return (int)cudaGetLastError();
+}
+
+int gh_patch_pool_bwd(const float* const* maps, float* const* d_maps, const int* H, const int* W, const long long* strides,
+                      const long long* d_strides, int L, int B, int D, int ln_input, const float* bwd_workspace,
+                      void* stream) {
+  if (!d_maps || !H || !W || !d_strides || !bwd_workspace || L <= 0 || B <= 0 || D <= 0) return GH_ERR_BAD_ARG;
+  if (ln_input && (!maps || !strides)) return GH_ERR_BAD_ARG;
+  if ((uintptr_t)bwd_workspace % 16 != 0) return GH_ERR_BAD_ARG;
+  if (L > kPatchMaxLayers || D > kPatchMaxD || B > 0x7fffffff / 2) return GH_ERR_UNSUPPORTED;
+  PatchPoolBwdParams p{};
+  for (int l = 0; l < L; ++l) {
+    if (!d_maps[l] || H[l] <= 0 || W[l] <= 0 || (ln_input && !maps[l])) return GH_ERR_BAD_ARG;
+    p.layer[l].x = ln_input ? maps[l] : nullptr;
+    p.layer[l].H = H[l];
+    p.layer[l].W = W[l];
+    if (ln_input) {
+      p.layer[l].s_img = strides[4 * l + 0];
+      p.layer[l].s_c = strides[4 * l + 1];
+      p.layer[l].s_y = strides[4 * l + 2];
+      p.layer[l].s_x = strides[4 * l + 3];
+    }
+    p.grad[l].dx = d_maps[l];
+    p.grad[l].s_img = d_strides[4 * l + 0];
+    p.grad[l].s_c = d_strides[4 * l + 1];
+    p.grad[l].s_y = d_strides[4 * l + 2];
+    p.grad[l].s_x = d_strides[4 * l + 3];
+  }
+  p.L = L; p.B = B; p.D = D; p.ln_input = ln_input ? 1 : 0;
+  const long long planes = (long long)L * B * D;
+  p.coef = bwd_workspace;
+  p.scal = bwd_workspace + planes * kPatchBins;
+  const long long gx = (long long)B * ((D + 7) / 8);
+  if (gx > 0x7fffffffLL) return GH_ERR_UNSUPPORTED;
+  patch_pool_bwd_kernel<<<dim3((unsigned)gx, L), kPatchThreads, 0, (cudaStream_t)stream>>>(p);
+  return (int)cudaGetLastError();
+}
+
+int gh_patch_attn_bwd(const float* feat, const float* W_in1, const float* b_in1, const float* W_out1,
+                      const float* b_out1, const float* W_in2, const float* b_in2, const float* W_out2,
+                      const float* b_out2, const float* W_c, const float* d_emb, const float* d_logits, int L, int B,
+                      int E, int heads, int nc, float* d_feat, float* x1, float* dqkv, float* o, float* dy,
+                      void* stream) {
+  if (!feat || !W_in1 || !b_in1 || !W_out1 || !b_out1 || !W_in2 || !b_in2 || !W_out2 || !b_out2 || !W_c || !d_emb ||
+      !d_logits || !d_feat || !x1 || !dqkv || !o || !dy)
+    return GH_ERR_BAD_ARG;
+  if (L <= 0 || B <= 0 || E <= 0 || heads <= 0 || nc <= 0 || E % heads != 0) return GH_ERR_BAD_ARG;
+  if (L > kPatchMaxLayers || E > 128 || E % 4 != 0) return GH_ERR_UNSUPPORTED;
+  const float* ptrs[4] = {W_in1, W_out1, W_in2, W_out2};
+  for (int i = 0; i < 4; ++i)
+    if ((uintptr_t)ptrs[i] % 16 != 0) return GH_ERR_UNSUPPORTED;       // in_proj rows are read as float4
+  PatchAttnBwdParams p{};
+  p.f.feat = feat;
+  p.f.w_in[0] = W_in1; p.f.b_in[0] = b_in1; p.f.w_out[0] = W_out1; p.f.b_out[0] = b_out1;
+  p.f.w_in[1] = W_in2; p.f.b_in[1] = b_in2; p.f.w_out[1] = W_out2; p.f.b_out[1] = b_out2;
+  p.f.w_c = W_c;
+  p.f.L = L; p.f.B = B; p.f.E = E; p.f.heads = heads; p.f.nc = nc;
+  p.d_emb = d_emb; p.d_logits = d_logits;
+  p.d_feat = d_feat; p.x1 = x1; p.dqkv = dqkv; p.o = o; p.dy = dy;
+  const size_t smem = ((size_t)L * E * 15 + (size_t)heads * L * L * 3 + E) * 4;
+  cudaError_t e = cudaFuncSetAttribute(patch_attention_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return (int)e;
+  const int sms = gh_sm_count();
+  const int grid = B < 2 * sms ? B : 2 * sms;
+  patch_attention_bwd_kernel<<<grid, kPatchThreads, smem, (cudaStream_t)stream>>>(p);
   return (int)cudaGetLastError();
 }
 

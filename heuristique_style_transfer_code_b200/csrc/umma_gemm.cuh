@@ -296,9 +296,10 @@ __global__ void __launch_bounds__(kUgThreads, 1) umma_gemm_kernel(const UmmaGemm
 }
 
 // Launcher. Returns cudaErrorNotSupported when the shape needs the SIMT path (caller falls through to launch_sgemm).
+// max_split > 0 caps the K split; 1 gives every output tile a single writer (no reduce-adds: the same bits on every run).
 inline cudaError_t launch_umma_gemm(const float* A, bool a_mn, long long lda, const float* B, bool b_mn, long long ldb,
                                     const float* bias, float* D, long long ldd, int M, int N, int K, int sms,
-                                    cudaStream_t st) {
+                                    cudaStream_t st, int max_split = 0) {
   if (M <= 0 || N <= 0 || K <= 0) return cudaSuccess;
   const bool aligned = (lda % 4 == 0) && (ldb % 4 == 0) && ((reinterpret_cast<uintptr_t>(A) & 15u) == 0) &&
                        ((reinterpret_cast<uintptr_t>(B) & 15u) == 0) && ((a_mn ? M : K) % 4 == 0) &&
@@ -315,6 +316,7 @@ inline cudaError_t launch_umma_gemm(const float* A, bool a_mn, long long lda, co
     ks = sms / ntiles;
     const int kmax = p.nkb / 2 > 1 ? p.nkb / 2 : 1;
     if (ks > kmax) ks = kmax;
+    if (max_split > 0 && ks > max_split) ks = max_split;
     if (ks < 1) ks = 1;
   }
   p.ksplit = ks;

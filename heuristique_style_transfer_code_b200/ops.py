@@ -406,7 +406,20 @@ def patch_gram(maps: Sequence[torch.Tensor], ln_input: bool = True):
     """The L collected (B, D, H_l, W_l) fp32 maps of one Multi-PatchGAN discriminator -> (gram (L, B, D*D),
     gram_norm (L, B)) through gh_patch_gram_fwd: [layer norm over the map,] 4x4 adaptive average pooling, layer norm,
     Gram over the 16 positions / (16 + 1e-6), Frobenius norm (Models_Multi_PatchGAN.py:198, :210-223)."""
-    import ctypes
+    gram, norm, _ = _patch_gram_fwd(maps, ln_input)
+    return gram, norm
+
+
+def _patch_map_arrays(maps: Sequence[torch.Tensor]):
+    """HOST arrays of the C ABI: map pointers, heights, widths, 4 element strides per map."""
+    L = len(maps)
+    return ((ctypes.c_void_p * L)(*[m.data_ptr() for m in maps]), (ctypes.c_int * L)(*[m.shape[2] for m in maps]),
+            (ctypes.c_int * L)(*[m.shape[3] for m in maps]),
+            (ctypes.c_longlong * (4 * L))(*[v for m in maps for v in m.stride()]))
+
+
+def _patch_gram_fwd(maps: Sequence[torch.Tensor], ln_input: bool):
+    """patch_gram, also returning the workspace (bin means and channel sums) the backward starts from."""
     L = len(maps)
     if L == 0:
         raise GramHeadError("gramhead: patch_gram needs at least one feature map")
@@ -419,16 +432,13 @@ def patch_gram(maps: Sequence[torch.Tensor], ln_input: bool = True):
     gram = torch.empty((L, b, d * d), device=dev, dtype=torch.float32)
     norm = torch.empty((L, b), device=dev, dtype=torch.float32)
     scratch = torch.empty((_lib.lib().gh_patch_gram_workspace(L, b, d) + 1) // 2, device=dev, dtype=torch.float64)
-    ptrs = (ctypes.c_void_p * L)(*[m.data_ptr() for m in maps])
-    hs = (ctypes.c_int * L)(*[m.shape[2] for m in maps])
-    ws = (ctypes.c_int * L)(*[m.shape[3] for m in maps])
-    st = (ctypes.c_longlong * (4 * L))(*[v for m in maps for v in m.stride()])
+    ptrs, hs, ws, st = _patch_map_arrays(maps)
     work = dict(bytes=sum(m.numel() for m in maps) * 4 + gram.numel() * 4, flops=2 * L * b * d * d * 16, kind="patch_gram")
     with torch.cuda.device(dev), _Timed(f"patch_gram[L={L},D={d},HW0={maps[0].shape[2]}x{maps[0].shape[3]}]", 2, dev, **work):
         rc = _lib.lib().gh_patch_gram_fwd(ptrs, hs, ws, st, L, b, d, 1 if ln_input else 0, gram.data_ptr(),
                                           norm.data_ptr(), scratch.data_ptr(), _stream_ptr(maps[0]))
     check(rc, "gh_patch_gram_fwd")
-    return gram, norm
+    return gram, norm, scratch
 
 
 def patch_attention(feat: torch.Tensor, attn1: torch.nn.MultiheadAttention, attn2: torch.nn.MultiheadAttention,
@@ -436,27 +446,190 @@ def patch_attention(feat: torch.Tensor, attn1: torch.nn.MultiheadAttention, attn
     """feat (L, B, E) -> (embeddings (B, E), output (B, nc)): the two multi-head attentions over the layer tokens, the
     mean over layers and the classifier (Models_Multi_PatchGAN.py:243-256) in one launch (gh_patch_attn_fwd)."""
     _require_cuda(feat, "feat")
-    L, b, e = feat.shape
-    feat = feat.contiguous()
-    nc = classifier.out_features
-    emb = torch.empty((b, e), device=feat.device, dtype=torch.float32)
-    out = torch.empty((b, nc), device=feat.device, dtype=torch.float32)
+    return _patch_attention_fwd(feat.contiguous(), _patch_attention_params(feat, attn1, attn2, classifier), attn1.num_heads)
+
+
+def _patch_attention_params(feat, attn1, attn2, classifier) -> List[torch.Tensor]:
+    """[in_proj_weight, in_proj_bias, out_proj.weight, out_proj.bias] of both attentions, then classifier weight, bias."""
+    e = feat.shape[2]
     tensors = []
     for a in (attn1, attn2):
         if a.in_proj_weight is None or a.in_proj_bias is None or a.embed_dim != e or a.num_heads != attn1.num_heads:
             raise GramHeadError("gramhead: patch_attention needs packed in_proj weights with biases and one embed_dim")
         tensors += [a.in_proj_weight, a.in_proj_bias, a.out_proj.weight, a.out_proj.bias]
     tensors += [classifier.weight, classifier.bias]
+    return tensors
+
+
+def _patch_attention_fwd(feat: torch.Tensor, tensors: Sequence[torch.Tensor], heads: int):
+    L, b, e = feat.shape
+    nc = tensors[-1].shape[0]
+    emb = torch.empty((b, e), device=feat.device, dtype=torch.float32)
+    out = torch.empty((b, nc), device=feat.device, dtype=torch.float32)
     tensors = [t.detach().contiguous() for t in tensors]
     for t in tensors:
         _require_cuda(t, "head parameter")
     work = dict(bytes=(feat.numel() + emb.numel() + out.numel() + sum(t.numel() for t in tensors)) * 4,
                 flops=2 * b * L * (2 * 4 * e * e) + 2 * b * e * nc, kind="patch_attention")
     with torch.cuda.device(feat.device), _Timed(f"patch_attention[L={L},E={e}]", 1, feat.device, **work):
-        rc = _lib.lib().gh_patch_attn_fwd(feat.data_ptr(), *[t.data_ptr() for t in tensors], L, b, e, attn1.num_heads, nc,
+        rc = _lib.lib().gh_patch_attn_fwd(feat.data_ptr(), *[t.data_ptr() for t in tensors], L, b, e, heads, nc,
                                           emb.data_ptr(), out.data_ptr(), _stream_ptr(feat))
     check(rc, "gh_patch_attn_fwd")
     return emb, out
+
+
+# ---- Multi-PatchGAN Gram head, backward ------------------------------------------------------------------------------
+def gemm_f32_fixed(a: torch.Tensor, b: torch.Tensor) -> torch.Tensor:
+    """a (M, K) @ b (K, N) for strided fp32 CUDA views through gh_gemm_f32_fixed: never split over K, so the same bits
+    on every run (weight gradients, whose K is the batch)."""
+    m, k = a.shape
+    k2, n = b.shape
+    assert k == k2 and a.dtype == torch.float32 and b.dtype == torch.float32
+    out = torch.empty((m, n), device=a.device, dtype=torch.float32)
+    work = dict(bytes=(m * k + k * n + m * n) * 4, flops=2 * m * n * k, kind="gemm")
+    with torch.cuda.device(a.device), _Timed(f"gemm_f32_fixed[M={m},N={n},K={k}]", 1, a.device, **work):
+        rc = _lib.lib().gh_gemm_f32_fixed(a.data_ptr(), a.stride(0), a.stride(1), b.data_ptr(), b.stride(0), b.stride(1),
+                                          0, out.data_ptr(), n, m, n, k, _stream_ptr(a))
+    check(rc, "gh_gemm_f32_fixed")
+    return out
+
+
+def colsum_f32(x: torch.Tensor) -> torch.Tensor:
+    """(M, N) fp32 rows (unit column stride) -> (N,) column sums in a fixed order (gh_colsum_f32)."""
+    m, n = x.shape
+    assert x.dtype == torch.float32 and x.stride(1) == 1
+    out = torch.empty((n,), device=x.device, dtype=torch.float32)
+    with torch.cuda.device(x.device), _Timed(f"colsum_f32[M={m},N={n}]", 1, x.device, bytes=(m + 1) * n * 4, flops=m * n,
+                                             kind="colsum"):
+        rc = _lib.lib().gh_colsum_f32(x.data_ptr(), x.stride(0), m, n, out.data_ptr(), _stream_ptr(x))
+    check(rc, "gh_colsum_f32")
+    return out
+
+
+def patch_gram_backward(maps: Sequence[torch.Tensor], ln_input: bool, d_gram: torch.Tensor, d_norm: torch.Tensor,
+                        norm: torch.Tensor, scratch: torch.Tensor) -> List[torch.Tensor]:
+    """Gradients of the L maps of patch_gram (each in its map's layout) from d_gram (L, B, D*D) and d_norm (L, B):
+    gh_patch_gram_bwd then gh_patch_pool_bwd. norm, scratch: the forward's norms and workspace."""
+    L = len(maps)
+    b, d = maps[0].shape[:2]
+    dev = maps[0].device
+    d_gram, d_norm = d_gram.contiguous(), d_norm.contiguous()
+    bws = torch.empty(_lib.lib().gh_patch_bwd_workspace(L, b, d), device=dev, dtype=torch.float32)
+    _, hs, ws, _ = _patch_map_arrays(maps)
+    with torch.cuda.device(dev), _Timed(f"patch_gram_bwd[L={L},D={d}]", 1, dev, bytes=(d_gram.numel() + bws.numel()) * 4,
+                                        flops=2 * L * b * d * d * 16 * 2, kind="patch_gram_bwd"):
+        rc = _lib.lib().gh_patch_gram_bwd(hs, ws, L, b, d, 1 if ln_input else 0, d_gram.data_ptr(), d_norm.data_ptr(),
+                                          norm.data_ptr(), scratch.data_ptr(), bws.data_ptr(), _stream_ptr(d_gram))
+    check(rc, "gh_patch_gram_bwd")
+    grads = [torch.empty_like(m) for m in maps]
+    ptrs, _, _, st = _patch_map_arrays(maps)
+    gptrs, _, _, gst = _patch_map_arrays(grads)
+    nbytes = sum(m.numel() for m in maps) * 4 * (2 if ln_input else 1)
+    with torch.cuda.device(dev), _Timed(f"patch_pool_bwd[L={L},D={d},HW0={maps[0].shape[2]}x{maps[0].shape[3]}]", 1, dev,
+                                        bytes=nbytes, flops=0, kind="patch_pool_bwd"):
+        rc = _lib.lib().gh_patch_pool_bwd(ptrs, gptrs, hs, ws, st, gst, L, b, d, 1 if ln_input else 0, bws.data_ptr(),
+                                          _stream_ptr(d_gram))
+    check(rc, "gh_patch_pool_bwd")
+    return grads
+
+
+class _PatchGram(torch.autograd.Function):
+    """maps -> (gram (L, B, D*D), gram_norm (L, B)): patch_gram, with gh_patch_gram_bwd + gh_patch_pool_bwd backward."""
+
+    @staticmethod
+    def forward(ctx, ln_input, *maps):
+        gram, norm, scratch = _patch_gram_fwd(maps, ln_input)
+        ctx.ln_input, ctx.scratch = ln_input, scratch
+        ctx.save_for_backward(norm, *maps)
+        return gram, norm
+
+    @staticmethod
+    def backward(ctx, d_gram, d_norm):
+        norm, *maps = ctx.saved_tensors
+        if not any(ctx.needs_input_grad[1:]):
+            return (None,) * (1 + len(maps))
+        return (None, *patch_gram_backward(maps, ctx.ln_input, d_gram, d_norm, norm, ctx.scratch))
+
+
+class _PatchProjection(torch.autograd.Function):
+    """gram (L, B, D*D) -> feat (L, B, E) = gram W^T + b (feature_projection, :229) on gh_gemm_f32; backward on
+    gh_gemm_f32_fixed / gh_colsum_f32 over the L*B rows."""
+
+    @staticmethod
+    def forward(ctx, gram, weight, bias):
+        L, b, dd = gram.shape
+        ctx.save_for_backward(gram, weight)
+        return gemm_f32(gram.view(L * b, dd), weight.t(), bias).view(L, b, -1)
+
+    @staticmethod
+    def backward(ctx, d_feat):
+        gram, weight = ctx.saved_tensors
+        L, b, dd = gram.shape
+        d = d_feat.contiguous().view(L * b, -1)
+        d_gram = gemm_f32_fixed(d, weight).view(L, b, dd) if ctx.needs_input_grad[0] else None
+        d_w = gemm_f32_fixed(d.t(), gram.view(L * b, dd)) if ctx.needs_input_grad[1] else None
+        d_b = colsum_f32(d) if ctx.needs_input_grad[2] else None
+        return d_gram, d_w, d_b
+
+
+class _PatchAttention(torch.autograd.Function):
+    """feat (L, B, E) -> (embeddings (B, E), output (B, nc)): patch_attention, with gh_patch_attn_bwd backward and the
+    weight gradients as gh_gemm_f32_fixed / gh_colsum_f32 over the rows it writes."""
+
+    @staticmethod
+    def forward(ctx, feat, heads, *params):
+        feat = feat.contiguous()
+        emb, out = _patch_attention_fwd(feat, params, heads)
+        ctx.heads = heads
+        ctx.save_for_backward(feat, emb, *params)
+        return emb, out
+
+    @staticmethod
+    def backward(ctx, d_emb, d_out):
+        feat, emb, *params = ctx.saved_tensors
+        L, b, e = feat.shape
+        nc = params[-1].shape[0]
+        dev = feat.device
+        w = [t.contiguous() for t in params]
+        d_emb, d_out = d_emb.contiguous(), d_out.contiguous()
+        d_feat = torch.empty_like(feat)
+        x1 = torch.empty_like(feat)
+        dqkv = torch.empty((2, L, b, 3 * e), device=dev, dtype=torch.float32)
+        o = torch.empty((2, L, b, e), device=dev, dtype=torch.float32)
+        dy = torch.empty((2, L, b, e), device=dev, dtype=torch.float32)
+        work = dict(bytes=(feat.numel() * 11 + d_emb.numel() + d_out.numel()) * 4,
+                    flops=3 * (2 * b * L * (2 * 4 * e * e)) + 2 * b * e * nc, kind="patch_attention_bwd")
+        with torch.cuda.device(dev), _Timed(f"patch_attention_bwd[L={L},E={e}]", 1, dev, **work):
+            rc = _lib.lib().gh_patch_attn_bwd(feat.data_ptr(), *[t.data_ptr() for t in w[:9]], d_emb.data_ptr(),
+                                              d_out.data_ptr(), L, b, e, ctx.heads, nc, d_feat.data_ptr(), x1.data_ptr(),
+                                              dqkv.data_ptr(), o.data_ptr(), dy.data_ptr(), _stream_ptr(feat))
+        check(rc, "gh_patch_attn_bwd")
+        rows = L * b
+        grads = []
+        for a, x in enumerate((feat, x1)):
+            dq = dqkv[a].view(rows, 3 * e)
+            grads += [gemm_f32_fixed(dq.t(), x.view(rows, e)), colsum_f32(dq),
+                      gemm_f32_fixed(dy[a].view(rows, e).t(), o[a].view(rows, e)), colsum_f32(dy[a].view(rows, e))]
+        grads += [gemm_f32_fixed(d_out.t(), emb), colsum_f32(d_out)]
+        grads = [g if need else None for g, need in zip(grads, ctx.needs_input_grad[2:])]
+        return (d_feat if ctx.needs_input_grad[0] else None, None, *grads)
+
+
+def patch_gram_autograd(maps: Sequence[torch.Tensor], ln_input: bool = True):
+    """patch_gram with autograd history: gradients flow to the maps (d_gram and d_norm both used)."""
+    return _PatchGram.apply(ln_input, *maps)
+
+
+def patch_projection_autograd(gram: torch.Tensor, linear: torch.nn.Linear) -> torch.Tensor:
+    """feature_projection (:229) of the (L, B, D*D) Grams, with autograd history for gram, weight and bias."""
+    return _PatchProjection.apply(gram, linear.weight, linear.bias)
+
+
+def patch_attention_autograd(feat: torch.Tensor, attn1: torch.nn.MultiheadAttention,
+                             attn2: torch.nn.MultiheadAttention, classifier: torch.nn.Linear):
+    """patch_attention with autograd history for feat and every parameter of the two attentions and the classifier."""
+    _require_cuda(feat, "feat")
+    return _PatchAttention.apply(feat, attn1.num_heads, *_patch_attention_params(feat, attn1, attn2, classifier))
 
 
 # ----------------------------------------------------------------------------------------------------------------------

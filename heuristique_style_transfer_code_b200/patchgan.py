@@ -20,14 +20,17 @@ norm and the softmax over layers all propagate it), so here the forward runs onc
 (B, ndf) / (B, nc) results, and -- only if they hold a NaN -- runs again layer by layer with the reference's checks,
 messages and replacements. Clean inputs pay one tiny check instead of ~20 synchronisations.
 
-Gradients. The kernels implement the forward only: the classification / evaluation / camera call sites
-(functions_Multi_PatchGAN.py:164, :200, :464) run under torch.no_grad(). One upstream mode needs gradients THROUGH the
-head down to the input image -- `style_transfer_patches` (functions_Multi_PatchGAN.py:272-287: `model(noise_image)` with
-noise_image.requires_grad, then `loss.backward()`), a mode outside this package's path (DESIGN.md section 8). So that it
-keeps working where the reference works, a forward that needs autograd history is handed to the reference's OWN forward
-(Models/Models_Multi_PatchGAN.py:177-256, executed on this module's parameters; loaded by _reference.py) instead of the
-kernels; when no copy of the reference is available it raises GramHeadError rather than returning tensors without
-history.
+Gradients. By default the kernels serve forwards without autograd history: the classification / evaluation / camera
+call sites (functions_Multi_PatchGAN.py:164, :200, :464) run under torch.no_grad(). A forward that needs autograd history
+(fine-tuning the discriminator, a GAN loss through it, a regulariser on get_gram_norms(), or `style_transfer_patches`,
+functions_Multi_PatchGAN.py:272-287, which optimises an image through it) is handed to the reference's OWN forward
+(Models/Models_Multi_PatchGAN.py:177-256, executed on this module's parameters; loaded by _reference.py); when no copy of
+the reference is available it raises GramHeadError rather than returning tensors without history.
+`set_library_backward(True)` (or GRAMHEAD_PATCHGAN_BACKWARD=1 in the environment, for unmodified scripts) runs such a
+forward on the kernels instead, under three autograd Functions that mirror the three launches (ops._PatchGram,
+ops._PatchProjection, ops._PatchAttention) and backpropagate on the library's backward kernels. It is opt-in only so
+that the default does not move; the next step is to make it the default and delete _reference_forward (DESIGN.md
+section 8).
 """
 from __future__ import annotations
 
@@ -41,6 +44,10 @@ from . import ops
 from ._lib import GramHeadError
 
 PATCH_TYPES = {'small': (4, 30), 'medium': (31, 80), 'large': (81, 150)}          # Models_Multi_PatchGAN.py:11-15
+
+
+def _library_backward_from_env() -> bool:
+    return os.environ.get("GRAMHEAD_PATCHGAN_BACKWARD", "").strip() == "1"
 
 
 class VariablePatchesNLayerDiscriminator_test(nn.Module):
@@ -79,6 +86,14 @@ class VariablePatchesNLayerDiscriminator_test(nn.Module):
         self.attention_per_patch = nn.MultiheadAttention(embed_dim=ndf, num_heads=8)
         self.classifier = nn.Linear(ndf, num_classes)                                      # :172
         self.feature_projection = nn.Linear(gram_matrix_dim * gram_matrix_dim, ndf)        # :175
+        # plain attribute (no state_dict key): grad-enabled forwards on the library's kernels instead of the reference's
+        self.library_backward = _library_backward_from_env()
+
+    def set_library_backward(self, enabled: bool = True):
+        """Run forwards that need autograd history on the library's kernels and backward kernels (see the module
+        docstring). Returns self."""
+        self.library_backward = bool(enabled)
+        return self
 
     # -- the head ------------------------------------------------------------------------------------------------------
     def _needs_autograd(self, x):
@@ -95,7 +110,7 @@ class VariablePatchesNLayerDiscriminator_test(nn.Module):
                                 "torch.no_grad(), or " + str(exc)) from exc
         return ref.VariablePatchesNLayerDiscriminator_test.forward(self, x)
 
-    def _forward(self, x, careful: bool):
+    def _forward(self, x, careful: bool, grad: bool = False):
         maps, k = [], 0
         for idx, layer in enumerate(self.feature_extractor):
             x = layer(x)
@@ -112,17 +127,31 @@ class VariablePatchesNLayerDiscriminator_test(nn.Module):
         if not maps:
             raise ValueError("No feature maps were collected. Check the model architecture and input data.")
         # layer norm :198 is folded into the pooling pass (pooling is linear, the norm a per-image affine map)
-        gram, norms = ops.patch_gram(maps, ln_input=True)
-        L, b, dd = gram.shape
-        feat = ops.gemm_f32(gram.view(L * b, dd), self.feature_projection.weight.detach().t(),
-                            self.feature_projection.bias.detach()).view(L, b, -1)
+        if grad:
+            gram, norms = ops.patch_gram_autograd(maps, ln_input=True)
+            feat = ops.patch_projection_autograd(gram, self.feature_projection)
+        else:
+            gram, norms = ops.patch_gram(maps, ln_input=True)
+            L, b, dd = gram.shape
+            feat = ops.gemm_f32(gram.view(L * b, dd), self.feature_projection.weight.detach().t(),
+                                self.feature_projection.bias.detach()).view(L, b, -1)
         if careful:
             bad = torch.isnan(feat).flatten(1).any(dim=1).tolist()
+            rows = list(feat.unbind(0)) if grad else None      # out of place under autograd: nan_to_num's own gradient
             for fm_idx, flag in enumerate(bad):
                 if flag:
                     print(f"NaN detected in projected features at layer {fm_idx}, replacing NaNs with zeros.")
-                    feat[fm_idx] = torch.nan_to_num(feat[fm_idx], nan=0.0)
-        emb, out = ops.patch_attention(feat, self.attention_per_layer, self.attention_per_patch, self.classifier)
+                    if grad:
+                        rows[fm_idx] = torch.nan_to_num(rows[fm_idx], nan=0.0)
+                    else:
+                        feat[fm_idx] = torch.nan_to_num(feat[fm_idx], nan=0.0)
+            if grad:
+                feat = torch.stack(rows, dim=0)
+        if grad:
+            emb, out = ops.patch_attention_autograd(feat, self.attention_per_layer, self.attention_per_patch,
+                                                    self.classifier)
+        else:
+            emb, out = ops.patch_attention(feat, self.attention_per_layer, self.attention_per_patch, self.classifier)
         return emb, out, norms
 
     def forward(self, input):
@@ -130,7 +159,13 @@ class VariablePatchesNLayerDiscriminator_test(nn.Module):
         if not input.is_cuda:
             raise GramHeadError(f"gramhead: input must be a CUDA tensor (got {input.device}); the head has no CPU path")
         if self._needs_autograd(input):
-            return self._reference_forward(input)
+            if not self.library_backward:
+                return self._reference_forward(input)
+            emb, out, norms = self._forward(input, careful=False, grad=True)
+            if bool(torch.isnan(emb).any() | torch.isnan(out).any()):
+                emb, out, norms = self._forward(input, careful=True, grad=True)
+            self.gram_norms = list(norms.unbind(0))
+            return emb, out
         with torch.no_grad():
             emb, out, norms = self._forward(input, careful=False)
             if bool(torch.isnan(emb).any() | torch.isnan(out).any()):
@@ -157,6 +192,12 @@ class MultiScaleDiscriminator_test(nn.Module):
                 input_nc=input_nc, patch_size=patch_sizes.get(patch_type, 70), ndf=ndf, norm=norm,
                 tensorboard_logdir=logdir, global_step=global_step, num_classes=num_classes,
                 gram_matrix_dim=gram_matrix_dim, pooling_type=pooling_type)
+
+    def set_library_backward(self, enabled: bool = True):
+        """set_library_backward of every scale. Returns self."""
+        for discriminator in self.scale_discriminators.values():
+            discriminator.set_library_backward(enabled)
+        return self
 
     def forward(self, input):
         embs, outs = [], []

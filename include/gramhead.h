@@ -197,6 +197,15 @@ int gh_normalize_u8(const unsigned char* src, float* dst, long long images, int 
 int gh_gemm_f32(const float* A, long long a_sm, long long a_sk, const float* B, long long b_sk, long long b_sn,
                 const float* bias, float* D, long long ldd, int M, int N, int K, void* stream);
 
+/* gh_gemm_f32 on the same routes, but K is never split: every output element has one writer and K is reduced in a fixed
+ * order, so the result is the same bits on every run (gh_gemm_f32 may split a long K over CTAs that meet in reduce-adds
+ * when the output has fewer tiles than the GPU has SMs). For weight gradients, whose K is the batch. */
+int gh_gemm_f32_fixed(const float* A, long long a_sm, long long a_sk, const float* B, long long b_sk, long long b_sn,
+                      const float* bias, float* D, long long ldd, int M, int N, int K, void* stream);
+
+/* out[n] = sum_{m < M} X[m*ldx + n] for n < N, summed in a fixed order (bias gradients over the rows of a batch). */
+int gh_colsum_f32(const float* X, long long ldx, int M, int N, float* out, void* stream);
+
 /* Max pooling of a channels_last activation, values only (inference plan of the encoder, frozen_encoder.py). Replaces the
  * nn.MaxPool2d child of the truncated encoder (torchvision resnet `maxpool`: kernel 3, stride 2, padding 1; child 3 of
  * `self.truncated_encoder`, Models/Models_RESNET50_TRUNCATE_GRAM_with_Attention.py:17,40) under eval + no_grad, where
@@ -273,6 +282,44 @@ int gh_patch_attn_fwd(const float* feat, const float* W_in1, const float* b_in1,
                       const float* b_out1, const float* W_in2, const float* b_in2, const float* W_out2,
                       const float* b_out2, const float* W_c, const float* b_c, int L, int B, int E, int heads, int nc,
                       float* emb, float* logits, void* stream);
+
+/* ---- Backward of the Multi-PatchGAN Gram head ------------------------------------------------------------------------
+ * Per image and collected layer the forward is x^ = LN(X) (:198, with ln_input), P = pool4x4(x^) (:210),
+ * Z = LN(P) over (D, 16) (:213), G = Z Z^T / (16 + 1e-6) (:217-220), n = |G|_F (:223), feat = vec(G) W^T + b (:229).
+ *
+ * gh_patch_gram_bwd: from d_gram (L, B, D*D) and d_norm (L, B), the backward of :213-223 and of the pooling's bin
+ * weights, per (image, layer):  dG += dn G / n (0 where n == 0, as torch's norm backward);  dZ = (dG + dG^T) Z /
+ * (16 + 1e-6);  dP = r2 (dZ - mean dZ - Z mean(dZ Z)). It writes bwd_workspace (gh_patch_bwd_workspace(L, B, D) floats,
+ * 16 B aligned): the table r dP[d][i] / |bin i| (L, B, D, 16), then per (layer, image) the scalars a = -r sum(dP) / N,
+ * c = -r^2 sum(dP P) / N and the map mean mu (0, 0, 0 without ln_input; N = D H W; r: the map's rstd, 1 without
+ * ln_input). Z, r and mu are recomputed with the forward's own code from fwd_workspace (gh_patch_gram_fwd's workspace,
+ * unchanged since that call); gram_norm is that call's output. H, W: HOST arrays of length L.
+ * gh_patch_pool_bwd: one pass that writes the gradient of every map,
+ *   dX(d, y, x) = sum over the 4x4 adaptive bins i holding (y, x) of table[d][i] + a + c (X(d, y, x) - mu),
+ * i.e. the pooling's backward (ATen's bins overlap when H % 4 != 0) and, with ln_input, the whole-map layer norm's
+ * backward r (dx^ - mean dx^ - x^ mean(dx^ x^)), whose two means are exact functions of the 16 D bin values. X (maps,
+ * strides as in gh_patch_gram_fwd) is read only when ln_input != 0. d_maps / d_strides: the gradients and their element
+ * strides (any layout: pass the map's own layout, channels_last included). L <= 8, D <= 128 (GH_ERR_UNSUPPORTED beyond). */
+long long gh_patch_bwd_workspace(int L, int B, int D);
+int gh_patch_gram_bwd(const int* H, const int* W, int L, int B, int D, int ln_input, const float* d_gram,
+                      const float* d_norm, const float* gram_norm, const float* fwd_workspace, float* bwd_workspace,
+                      void* stream);
+int gh_patch_pool_bwd(const float* const* maps, float* const* d_maps, const int* H, const int* W,
+                      const long long* strides, const long long* d_strides, int L, int B, int D, int ln_input,
+                      const float* bwd_workspace, void* stream);
+
+/* gh_patch_attn_bwd: backward of gh_patch_attn_fwd (:243-256) from d_emb (B, E) and d_logits (B, nc), one CTA per image:
+ * the image's forward is recomputed in shared memory, then classifier, mean over layers (:247), and for
+ * attention_per_patch then attention_per_layer: out_proj, softmax attention (q scaled by sqrt(1/hd)), in_proj. Writes
+ * d_feat (L, B, E) and the rows the weight gradients are GEMMs over (gh_gemm_f32_fixed / gh_colsum_f32 over the L*B rows):
+ * x1 (L, B, E) the input of attention_per_patch (the input of attention_per_layer is feat), and for a = 0 (per layer), 1
+ * (per patch): dqkv[a] (L, B, 3E) the gradient of the in_proj output, o[a] (L, B, E) the out_proj input, dy[a] (L, B, E)
+ * the gradient of the attention's output. Same weights and limits as gh_patch_attn_fwd (b_c is not needed). */
+int gh_patch_attn_bwd(const float* feat, const float* W_in1, const float* b_in1, const float* W_out1,
+                      const float* b_out1, const float* W_in2, const float* b_in2, const float* W_out2,
+                      const float* b_out2, const float* W_c, const float* d_emb, const float* d_logits, int L, int B,
+                      int E, int heads, int nc, float* d_feat, float* x1, float* dqkv, float* o, float* dy,
+                      void* stream);
 
 /* Number of fp32 elements gh_attn_head_bwd needs in `workspace`. */
 long long gh_attn_head_bwd_workspace(int B, int L, int E);
