@@ -354,8 +354,10 @@ __global__ void __launch_bounds__(kAttn2Threads) attn2_core_bwd_kernel(const flo
     if (threadIdx.x < L) {
       const int l = threadIdx.x;
       float dot = 0.f;
-      for (int m = 0; m < L; ++m) dot += sdAv[m] * inv_l * sA[l * LT + m];
-      for (int m = 0; m < L; ++m) sdS[l * LT + m] = sA[l * LT + m] * (sdAv[m] * inv_l - dot) * inv_sqrt_e;
+      for (int m = 0; m < L; ++m) dot += __fmul_rn(sdAv[m], inv_l) * sA[l * LT + m];
+      // dA[m] - dot rounded once, not contracted into an FMA: on a one-hot row (scores of 1e4 and more) the two are
+      // equal and the difference must be exactly 0, not the product's rounding error scaled by the size of the scores
+      for (int m = 0; m < L; ++m) sdS[l * LT + m] = sA[l * LT + m] * (__fmul_rn(sdAv[m], inv_l) - dot) * inv_sqrt_e;
     }
     __syncthreads();
     if (ok) {

@@ -1077,13 +1077,14 @@ int gh_gemm_planes(const void* A_planes, long long lda, long long a_plane_stride
   if (sms < 2) return GH_ERR_UNSUPPORTED;
   tg_plan(&s, 1, sms / 2);
   cudaStream_t st = (cudaStream_t)stream;
-  cudaError_t e;
+  TgLaunch l;
+  cudaError_t e = tg_prepare(&s, 1, sms, &l);       // before the K-split zeroing: a refused call writes nothing
+  if (e != cudaSuccess) return e == cudaErrorNotSupported ? GH_ERR_UNSUPPORTED : (int)e;
   if (s.ksplit > 1) {
     e = cudaMemset2DAsync(D, (size_t)ldd * 4, 0, (size_t)N * 4, (size_t)M, st);
     if (e != cudaSuccess) return (int)e;
   }
-  e = launch_tgemm(&s, 1, sms, st);
-  return e == cudaErrorNotSupported ? GH_ERR_UNSUPPORTED : (int)e;
+  return (int)tg_launch(l, st);
 }
 
 int gh_attn_head_fwd2(const float* desc, const void* w_in_planes, const float* b_in, const void* w_out_planes,
@@ -1093,32 +1094,37 @@ int gh_attn_head_fwd2(const float* desc, const void* w_in_planes, const float* b
     return GH_ERR_BAD_ARG;
   if (B <= 0 || L <= 0 || E <= 0 || nc <= 0) return GH_ERR_BAD_ARG;
   if (!attn2_supported(B, L, E, nc)) return GH_ERR_UNSUPPORTED;
+  if ((uintptr_t)W_c % 16 != 0) return GH_ERR_UNSUPPORTED;      // the classifier reads its rows as float4
   cudaStream_t st = (cudaStream_t)stream;
   const int sms = sm_count_cached();
   const long long BL = (long long)B * L;
-  // X -> planes (the A operand of the in_proj GEMM, and of dW_in in the backward)
-  int rc = gh_split_bf16(desc, x_planes, BL * E, BL * E, stream);
-  if (rc != 0) return rc;
   // QKV = X W_in^T + b_in           (B*L, 3E); at most two K partitions, so the sum is bitwise reproducible
   TgSpec s1 = tg_spec(tg_op(x_planes, E, BL, 0), tg_op(w_in_planes, E, 3LL * E, 0), (int)BL, 3 * E, E, b_in, qkv, 3LL * E, 2);
   tg_plan(&s1, 1, sms / 2);
-  cudaError_t e;
+  // emb = Obar W_out^T + b_out      (B, E)
+  TgSpec s2 = tg_spec(tg_op(obar_planes, E, B, 0), tg_op(w_out_planes, E, E, 0), B, E, E, b_out, emb, E, 2);
+  tg_plan(&s2, 1, sms / 2);
+  // both GEMMs are checked (alignment, tensor maps) before the first write, so a refused call writes nothing
+  TgLaunch l1, l2;
+  cudaError_t e = tg_prepare(&s1, 1, sms, &l1);
+  if (e == cudaSuccess) e = tg_prepare(&s2, 1, sms, &l2);
+  if (e != cudaSuccess) return e == cudaErrorNotSupported ? GH_ERR_UNSUPPORTED : (int)e;
+  // X -> planes (the A operand of the in_proj GEMM, and of dW_in in the backward)
+  int rc = gh_split_bf16(desc, x_planes, BL * E, BL * E, stream);
+  if (rc != 0) return rc;
   if (s1.ksplit > 1) {
     e = cudaMemsetAsync(qkv, 0, (size_t)BL * 3 * E * 4, st);
     if (e != cudaSuccess) return (int)e;
   }
-  e = launch_tgemm(&s1, 1, sms, st);
-  if (e != cudaSuccess) return e == cudaErrorNotSupported ? GH_ERR_UNSUPPORTED : (int)e;
-  // emb = Obar W_out^T + b_out      (B, E)
-  TgSpec s2 = tg_spec(tg_op(obar_planes, E, B, 0), tg_op(w_out_planes, E, E, 0), B, E, E, b_out, emb, E, 2);
-  tg_plan(&s2, 1, sms / 2);
+  e = tg_launch(l1, st);
+  if (e != cudaSuccess) return (int)e;
   __nv_bfloat16* ob = (__nv_bfloat16*)obar_planes;
   float* ez = s2.ksplit > 1 ? emb : nullptr;
   if (L <= 4) e = launch_pdl(attn2_core_fwd_kernel<4>, dim3(B), dim3(kAttn2Threads), 0, st, qkv, probs, ob, (long long)B * E, ez, L, E);
   else e = launch_pdl(attn2_core_fwd_kernel<kMaxL>, dim3(B), dim3(kAttn2Threads), 0, st, qkv, probs, ob, (long long)B * E, ez, L, E);
   if (e != cudaSuccess) return (int)e;
-  e = launch_tgemm(&s2, 1, sms, st);
-  if (e != cudaSuccess) return e == cudaErrorNotSupported ? GH_ERR_UNSUPPORTED : (int)e;
+  e = tg_launch(l2, st);
+  if (e != cudaSuccess) return (int)e;
   return (int)launch_pdl(attn2_classifier_kernel, dim3((B + 3) / 4), dim3(128), 0, st, emb, W_c, b_c, logits, B, E, nc);
 }
 
@@ -1137,6 +1143,8 @@ int gh_attn_head_bwd2(const void* x_planes, const void* w_in_planes, const void*
     return GH_ERR_BAD_ARG;
   if (B <= 0 || L <= 0 || E <= 0 || nc <= 0) return GH_ERR_BAD_ARG;
   if (!attn2_supported(B, L, E, nc) || (uintptr_t)workspace % 16 != 0) return GH_ERR_UNSUPPORTED;
+  // read (and db_in zeroed) as float4
+  if (((uintptr_t)qkv | (uintptr_t)emb | (uintptr_t)W_c | (uintptr_t)d_emb_ext | (uintptr_t)db_in) % 16 != 0) return GH_ERR_UNSUPPORTED;
   cudaStream_t st = (cudaStream_t)stream;
   const int sms = sm_count_cached();
   const long long BL = (long long)B * L, BE = (long long)B * E;
@@ -1158,6 +1166,11 @@ int gh_attn_head_bwd2(const void* x_planes, const void* w_in_planes, const void*
   if (dW_in) g2[n2++] = tg_spec(tg_op(dqkv, 3LL * E, BL, 1), tg_op(x_planes, E, BL, 1), 3 * E, E, (int)BL, nullptr, dW_in, E, 64);
   if (d_desc) g2[n2++] = tg_spec(tg_op(dqkv, 3LL * E, BL, 0), tg_op(w_in_planes, E, 3LL * E, 1), (int)BL, E, 3 * E, nullptr, d_desc, E, 64);
   if (n2) tg_plan(g2, n2, sms / 2);
+  // both launches are checked (alignment, tensor maps) before the first write, so a refused call writes nothing
+  TgLaunch l1, l2;
+  cudaError_t e = tg_prepare(g1, n1, sms, &l1);
+  if (e == cudaSuccess && n2) e = tg_prepare(g2, n2, sms, &l2);
+  if (e != cudaSuccess) return e == cudaErrorNotSupported ? GH_ERR_UNSUPPORTED : (int)e;
 
   float* dbin = db_in ? db_in : dbin_scratch;
   ZeroList z0{};
@@ -1165,7 +1178,6 @@ int gh_attn_head_bwd2(const void* x_planes, const void* w_in_planes, const void*
   z0.ptr[1] = (n1 > 1 && g1[1].ksplit > 1) ? dW_out : nullptr; z0.n4[1] = (long long)E * E / 4;
   z0.ptr[2] = dbin; z0.n4[2] = 3LL * E / 4;
   const size_t prep_smem = attn2_prep_smem_bytes(nc);
-  cudaError_t e = cudaSuccess;
   if (prep_smem > 48 * 1024) {
     e = cudaFuncSetAttribute(attn2_bwd_prep_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prep_smem);
     if (e != cudaSuccess) return (int)e;
@@ -1173,8 +1185,8 @@ int gh_attn_head_bwd2(const void* x_planes, const void* w_in_planes, const void*
   e = launch_pdl(attn2_bwd_prep_kernel, dim3((E + 127) / 128, kPrepSplit), dim3(kPrepThreads), prep_smem, st, d_logits,
                  d_emb_ext, W_c, emb, demb, BE, db_out, dW_c, db_c, B, E, nc, z0);
   if (e != cudaSuccess) return (int)e;
-  e = launch_tgemm(g1, n1, sms, st);
-  if (e != cudaSuccess) return e == cudaErrorNotSupported ? GH_ERR_UNSUPPORTED : (int)e;
+  e = tg_launch(l1, st);
+  if (e != cudaSuccess) return (int)e;
   ZeroList z1{};
   for (int i = 0; i < n2; ++i) {
     z1.ptr[i] = g2[i].ksplit > 1 ? g2[i].D_f32 : nullptr;
@@ -1186,8 +1198,8 @@ int gh_attn_head_bwd2(const void* x_planes, const void* w_in_planes, const void*
   else e = launch_pdl(attn2_core_bwd_kernel<kMaxL>, dim3(grid), dim3(kAttn2Threads), 0, st, qkv, probs, (const float*)dobar, dqkv, BL * 3 * E, dbin, B, L, E, z1);
   if (e != cudaSuccess) return (int)e;
   if (n2) {
-    e = launch_tgemm(g2, n2, sms, st);
-    if (e != cudaSuccess) return e == cudaErrorNotSupported ? GH_ERR_UNSUPPORTED : (int)e;
+    e = tg_launch(l2, st);
+    if (e != cudaSuccess) return (int)e;
   }
   return (int)cudaGetLastError();
 }

@@ -422,14 +422,22 @@ inline void tg_plan(TgSpec* specs, int n, int npairs) {
   for (int i = 0; i < n; ++i) { specs[i].tn = best_tn[i]; specs[i].ksplit = best_ks[i]; }
 }
 
+// A planned launch: parameters and tensor maps, built on the host before anything is enqueued.
+struct TgLaunch {
+  TgParams p;
+  TgMaps maps;
+  int npairs;
+};
+
 // Supported: K-major operands with ld % 8 == 0; MN-major operands whose M / N extent is a multiple of 64; 16 B aligned
 // planes. Returns cudaErrorNotSupported otherwise (the caller then uses the ld.global kernels of umma_gemm.cuh).
-// specs[] must have been planned with tg_plan(); a problem with ksplit > 1 accumulates into D_f32, which the caller
-// has zeroed earlier in the stream.
-inline cudaError_t launch_tgemm(const TgSpec* specs, int n, int sms, cudaStream_t st) {
+// specs[] must have been planned with tg_plan(). Enqueues nothing, so a caller that has more to do before the launch
+// (zeroing a K-split output, kernels that feed the GEMM) checks here first and writes nothing when the shape is refused.
+inline cudaError_t tg_prepare(const TgSpec* specs, int n, int sms, TgLaunch* out) {
   if (n < 1 || n > kTgMaxProblems || sms < 2) return cudaErrorNotSupported;
-  TgParams p{};
-  TgMaps maps;
+  TgParams& p = out->p;
+  TgMaps& maps = out->maps;
+  p = TgParams{};
   int units = 0;
   for (int i = 0; i < n; ++i) {
     const TgSpec& s = specs[i];
@@ -455,11 +463,15 @@ inline cudaError_t launch_tgemm(const TgSpec* specs, int n, int sms, cudaStream_
   }
   p.nprob = n;
   p.total_units = units;
-  int npairs = sms / 2;
-  if (units < npairs) npairs = units;
+  out->npairs = sms / 2;
+  if (units < out->npairs) out->npairs = units;
+  return cudaSuccess;
+}
+// A problem with ksplit > 1 accumulates into D_f32, which the caller has zeroed earlier in the stream.
+inline cudaError_t tg_launch(const TgLaunch& l, cudaStream_t st) {
   cudaError_t e = cudaFuncSetAttribute(tgemm_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTgSmemBytes);
   if (e != cudaSuccess) return e;
-  return launch_pdl(tgemm_pair_kernel, dim3(2 * npairs), dim3(kTgThreads), kTgSmemBytes, st, p, maps);
+  return launch_pdl(tgemm_pair_kernel, dim3(2 * l.npairs), dim3(kTgThreads), kTgSmemBytes, st, l.p, l.maps);
 }
 
 }  // namespace gh

@@ -7,7 +7,9 @@ Behind every Gram entry point sit two kernel families, forced here one at a time
              fp32 features feed kind::tf32, rounded to the nearest tf32 by the TMA unit (TFLOAT32 tensor maps);
   * "auto" - whatever the library picks for the shape (the shipped default).
 This file feeds fresh tensors at the shipped shapes. tests/test_gpu_gram_routes.py covers the routes a tensor's layout
-selects (strided and misaligned views, every loader, ragged channel counts) and checks which kernel ran.
+selects (strided and misaligned views, every loader, ragged channel counts) and checks which kernel ran;
+tests/test_gpu_attention_routes.py does the same for the attention head (both kernel families, batch edges, token
+counts, gradient subsets, launch options, large scores) and for the general GEMMs beneath it.
 
 Tolerances (written next to each assert):
   * Gram / descriptor vs the fp64 oracle on fp32 inputs:            normwise rel. err <= 1e-3  (task statement)
@@ -306,7 +308,8 @@ class attention_impl:
 
 @pytest.mark.parametrize("impl", ("tma", "ldg"))
 @pytest.mark.parametrize("B,L,g,nc", [(5, 3, 8, 4), (33, 3, 32, 4), (4, 1, 16, 3), (7, 4, 8, 10), (1, 3, 32, 4), (2, 8, 8, 16),
-                                      (96, 3, 32, 4), (3, 3, 10, 4)])
+                                      (96, 3, 32, 4), (3, 3, 10, 4), (1, 2, 8, 1), (3, 5, 24, 16), (4, 7, 5, 17),
+                                      (2, 6, 12, 100)])
 def test_attention_head_forward_backward(ops, B, L, g, nc, impl):
     E = g * g
     torch.manual_seed(0)
@@ -372,7 +375,7 @@ def test_attention_head_tma_forward_is_bitwise_reproducible_and_follows_weight_u
 
 
 @pytest.mark.parametrize("M,N,K", [(256, 256, 64), (100, 192, 320), (1536, 1024, 3072), (15, 64, 64), (768, 3072, 1024)])
-@pytest.mark.parametrize("a_mn,b_mn", [(False, False), (False, True), (True, True)])
+@pytest.mark.parametrize("a_mn,b_mn", [(False, False), (False, True), (True, False), (True, True)])
 def test_split_plane_gemm(ops, M, N, K, a_mn, b_mn):
     """gh_gemm_planes (TMA-fed, CTA pairs, hi/lo bf16 planes): every operand layout the attention head uses, fp32 output
     (plain, two K partitions, free K split with reduce-adds) and split-plane output: <= 2e-5 vs fp64."""
