@@ -70,6 +70,11 @@ _SIGNATURES = {
     "gh_attn_head_fwd2": (c_int, [_P] * 7 + [c_int] * 4 + [_P] * 6 + [_P]),
     "gh_attn_head_bwd2_workspace": (c_longlong, [c_int, c_int, c_int]),
     "gh_attn_head_bwd2": (c_int, [_P] * 10 + [c_int] * 4 + [_P] * 8 + [_P]),
+    "gh_jpeg_table_ints": (c_int, []),
+    "gh_jpeg_records_bytes": (c_longlong, [c_longlong, c_int, c_int]),
+    "gh_jpeg_check": (c_int, [c_longlong, c_int, c_int, c_longlong, c_longlong, c_int, c_int]),
+    "gh_jpeg_decode": (c_int, [_P, c_longlong, _P, c_int, _P, c_int, _P, c_longlong, c_longlong, c_int, _P, _P, _P, _P,
+                               _P, c_int, _P]),
 }
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)
 

@@ -8,7 +8,7 @@ import subprocess
 CSRC = os.path.join(os.path.dirname(os.path.abspath(__file__)), "csrc")
 LIB_PATH = os.path.join(CSRC, "libgramhead.so")
 SOURCES = ["gramhead.cu", "common.cuh", "gram_fwd.cuh", "pair.cuh", "gram_fwd_pair.cuh", "gram_bwd2.cuh", "gram_bwd_pair.cuh",
-           "umma_gemm.cuh", "tgemm_pair.cuh", "launch.cuh", "attn_head.cuh", "attn_head2.cuh", "preprocess.cuh", "transpose.cuh", "patchgan.cuh", "pool.cuh", "stem.cuh", "style_loss.cuh"]
+           "umma_gemm.cuh", "tgemm_pair.cuh", "launch.cuh", "attn_head.cuh", "attn_head2.cuh", "preprocess.cuh", "transpose.cuh", "patchgan.cuh", "pool.cuh", "stem.cuh", "style_loss.cuh", "jpeg.cuh"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared"]
 

@@ -16,6 +16,7 @@
 #include "pool.cuh"
 #include "stem.cuh"
 #include "style_loss.cuh"
+#include "jpeg.cuh"
 #include <string>
 
 namespace gh {
@@ -1253,6 +1254,53 @@ int gh_attn_head_bwd(const float* desc, const float* W_in, const float* W_out, c
     e = gemm_auto(dqkv, 3LL * E, 1, W_in, E, 1, nullptr, d_desc, E, B * L, E, 3 * E, 0, st);
     if (e != cudaSuccess) return (int)e;
   }
+  return (int)cudaGetLastError();
+}
+
+
+int gh_jpeg_table_ints(void) { return GH_JPEG_TABLE_INTS; }
+
+long long gh_jpeg_records_bytes(long long scan_bytes, int n_segs, int subseq_bytes) {
+  if (scan_bytes < 0 || n_segs <= 0 || subseq_bytes <= 0) return GH_ERR_BAD_ARG;
+  // segment i's records start at (its first byte / subseq_bytes + i): room for every segment's ceil(len / subseq) ones
+  return (scan_bytes / subseq_bytes + n_segs + 1) * (long long)kJpegRecordInts * 4;
+}
+
+int gh_jpeg_check(long long scan_bytes, int n_segs, int n_imgs, long long max_blocks, long long max_pixels,
+                  int subseq_bytes, int phases) {
+  if (scan_bytes <= 0 || n_segs <= 0 || n_imgs <= 0 || max_blocks <= 0 || max_pixels <= 0 || subseq_bytes <= 0)
+    return GH_ERR_BAD_ARG;
+  if (phases <= 0 || phases > (GH_JPEG_PHASE_HUFFMAN | GH_JPEG_PHASE_IDCT | GH_JPEG_PHASE_COLOR)) return GH_ERR_BAD_ARG;
+  // the batch's scan data has no size limit (offsets are 64-bit; a segment's own length is bounded by the caller and by
+  // the kernel, GH_JPEG_MAX_SEGMENT_BYTES); grids: images on y, blocks and pixels on x
+  if (n_imgs > 65535 || (max_blocks + 31) / 32 > 0x7fffffffLL ||
+      (max_pixels + kJpegColorThreads - 1) / kJpegColorThreads > 0x7fffffffLL)
+    return GH_ERR_UNSUPPORTED;
+  return 0;
+}
+
+int gh_jpeg_decode(const unsigned char* scan, long long scan_bytes, const long long* segs, int n_segs,
+                   const long long* imgs, int n_imgs, const int* tables, long long max_blocks, long long max_pixels,
+                   int subseq_bytes, short* coef, unsigned char* planes, int* records, int* status, unsigned char* arena,
+                   int phases, void* stream) {
+  if (!scan || !segs || !imgs || !tables || !coef || !planes || !records || !status || !arena) return GH_ERR_BAD_ARG;
+  const int rc = gh_jpeg_check(scan_bytes, n_segs, n_imgs, max_blocks, max_pixels, subseq_bytes, phases);
+  if (rc != 0) return rc;
+  JpegParams p;
+  p.scan = scan; p.scan_bytes = scan_bytes; p.segs = segs; p.imgs = imgs; p.tables = tables;
+  p.n_segs = n_segs; p.n_imgs = n_imgs; p.subseq = subseq_bytes;
+  p.coef = coef; p.planes = planes; p.records = records; p.status = status; p.arena = arena;
+  const cudaStream_t st = (cudaStream_t)stream;
+  if (phases & GH_JPEG_PHASE_HUFFMAN) {
+    const cudaError_t e = cudaMemsetAsync(status, 0, sizeof(int) * (size_t)n_imgs, st);
+    if (e != cudaSuccess) return (int)e;
+    jpeg_huffman_kernel<<<n_segs, kJpegHuffThreads, 0, st>>>(p);
+  }
+  if (phases & GH_JPEG_PHASE_IDCT)
+    jpeg_idct_kernel<<<dim3((unsigned)((max_blocks + 31) / 32), (unsigned)n_imgs), kJpegIdctThreads, 0, st>>>(p);
+  if (phases & GH_JPEG_PHASE_COLOR)
+    jpeg_color_kernel<<<dim3((unsigned)((max_pixels + kJpegColorThreads - 1) / kJpegColorThreads), (unsigned)n_imgs),
+                        kJpegColorThreads, 0, st>>>(p);
   return (int)cudaGetLastError();
 }
 

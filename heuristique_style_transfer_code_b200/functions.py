@@ -17,6 +17,7 @@ import torch.nn as nn
 import torch.nn.functional as F
 
 from . import _lib, ops, streaming
+from ._lib import GramHeadError
 from torch.utils.data import Subset
 
 
@@ -136,24 +137,39 @@ class PackedImages:
     (streaming.GEOMETRY_COLUMNS: H, W, byte offset in `pixels`, resized rh, rw, crop top, left); `labels` as the default
     collate makes them; and what cuda_prefetch needs to resample them: the transform's `resize` / `crop`, the common
     output size `out_hw` and the largest coefficient counts `kmax` = (hkmax, vkmax). pin_memory() lets
-    DataLoader(pin_memory=True) pin it like any other batch."""
+    DataLoader(pin_memory=True) pin it like any other batch.
 
-    def __init__(self, pixels, geometry, labels, resize, crop, out_hw, kmax):
+    With decode="gpu", `jpeg` = (scan, segs, imgs, tables) holds the compressed part (jpeg.pack) of the images the device
+    decodes, `files` their paths (the bytes of a file parsed without one; only CPU runs read them, with Pillow), and
+    `arena_bytes` the size of the pixel arena: `pixels` holds only the images the worker decoded, at the start of the
+    arena, and the geometry's offsets place every image in it."""
+
+    def __init__(self, pixels, geometry, labels, resize, crop, out_hw, kmax, jpeg=None, files=None, arena_bytes=None):
         self.pixels, self.geometry, self.labels = pixels, geometry, labels
         self.resize, self.crop, self.out_hw, self.kmax = resize, crop, tuple(out_hw), tuple(kmax)
+        self.jpeg, self.files = jpeg, files
+        self.arena_bytes = int(pixels.numel()) if arena_bytes is None else int(arena_bytes)
 
     def __len__(self):
         return int(self.geometry.shape[0])
 
     def pin_memory(self):
         labels = self.labels.pin_memory() if torch.is_tensor(self.labels) else self.labels
+        jpeg = None if self.jpeg is None else tuple(t.pin_memory() for t in self.jpeg)
         return PackedImages(self.pixels.pin_memory(), self.geometry.pin_memory(), labels, self.resize, self.crop,
-                            self.out_hw, self.kmax)
+                            self.out_hw, self.kmax, jpeg, self.files, self.arena_bytes)
 
     def images(self):
-        """The (H, W, 3) uint8 images, as numpy views of `pixels`."""
+        """The (H, W, 3) uint8 images, as numpy views of `pixels` (decoded with Pillow for the device-decoded files)."""
         flat = self.pixels.numpy()
-        return [flat[o:o + h * w * 3].reshape(h, w, 3) for h, w, o in self.geometry[:, :3].tolist()]
+        out = [None if o + h * w * 3 > flat.size else flat[o:o + h * w * 3].reshape(h, w, 3)
+               for h, w, o in self.geometry[:, :3].tolist()]
+        if self.jpeg is not None:
+            import io
+            from PIL import Image
+            for row, src in zip(self.jpeg[2][:, 12].tolist(), self.files):
+                out[row] = np.asarray(Image.open(io.BytesIO(src) if isinstance(src, bytes) else src).convert("RGB"))
+        return out
 
     def host_batch(self):
         """The (N, 3, oh, ow) uint8 batch torchvision's own Resize + CenterCrop + PILToTensor give on the host (CPU runs)."""
@@ -171,8 +187,11 @@ class GpuResizeTransform:
     device and resamples the batch there, bit for bit what Resize(resize) + CenterCrop(crop) + PILToTensor give on the
     host, before the usual ToTensor + Normalize of uint8 batches."""
 
-    def __init__(self, resize=256, crop=224, interpolation="bilinear", max_size=None):
+    def __init__(self, resize=256, crop=224, interpolation="bilinear", max_size=None, decode="host"):
         from torchvision.transforms import InterpolationMode
+        if decode not in ("host", "gpu"):
+            raise ValueError(f"gpu_resize_transform: decode must be 'host' or 'gpu', got {decode!r}")
+        self.decode = decode
         if InterpolationMode(interpolation) != InterpolationMode.BILINEAR:
             raise ValueError(f"gpu_resize_transform: only bilinear interpolation is reproduced on the GPU, got {interpolation!r}")
         if max_size is not None:
@@ -197,33 +216,67 @@ class GpuResizeTransform:
         self.resize = tuple(int(v) for v in resize) if isinstance(resize, (tuple, list)) else int(resize)
         self.crop = None if crop is None else pair(crop)
 
+    def loader(self, path):
+        """decode="gpu": the dataset's loader. Reads the file; Image.open without loading pixels gives Pillow's own
+        decompression-bomb check and its error on files that are not images. A baseline JPEG the device decodes comes
+        back as a jpeg.JpegFile; any other file is decoded here exactly as torchvision's default_loader does."""
+        import io
+        from PIL import Image
+        from . import jpeg
+        if self.decode != "gpu":
+            raise ValueError('gpu_resize_transform: .loader is for decode="gpu"')
+        with open(path, "rb") as f:
+            data = f.read()
+        img = Image.open(io.BytesIO(data))
+        parsed = jpeg.parse(data) if img.format == "JPEG" else None
+        if parsed is not None and parsed.W == img.size[0] and parsed.H == img.size[1]:
+            parsed.path = path
+            return parsed
+        return img.convert("RGB")
+
     def __call__(self, img):
+        from . import jpeg
+        if isinstance(img, jpeg.JpegFile):
+            return img
         if getattr(img, "mode", None) != "RGB":
             raise ValueError(f"gpu_resize_transform: takes RGB PIL images, got {getattr(img, 'mode', type(img).__name__)!r}")
         return torch.from_numpy(np.array(img, dtype=np.uint8))
 
     def collate(self, batch):
-        """[(pixels (H, W, 3) uint8, label), ...] -> PackedImages (pixels, geometry, labels built here, in the worker)."""
+        """[(pixels (H, W, 3) uint8, label), ...] -> PackedImages (pixels, geometry, labels built here, in the worker).
+        decode="gpu": items may be jpeg.JpegFile too; their compressed part goes into PackedImages.jpeg and their pixels
+        are placed after the worker-decoded ones in the arena."""
         from torch.utils.data import default_collate
+        from . import jpeg
         images = [img for img, _ in batch]
-        for img in images:
-            if not torch.is_tensor(img) or img.dtype != torch.uint8 or img.dim() != 3 or img.shape[2] != 3:
+        dev = [isinstance(img, jpeg.JpegFile) for img in images]
+        for img, d in zip(images, dev):
+            if not d and (not torch.is_tensor(img) or img.dtype != torch.uint8 or img.dim() != 3 or img.shape[2] != 3):
                 raise ValueError("gpu_resize_transform.collate: expects the (H, W, 3) uint8 tensors of its transform")
         geometry, out_hw = streaming.frame_geometry([tuple(img.shape) for img in images], self.resize, self.crop)
-        sizes = [int(img.numel()) for img in images]
-        offsets = np.concatenate([[0], np.cumsum(sizes)[:-1]]).astype(np.int64)
-        pixels = torch.empty(int(sum(sizes)), dtype=torch.uint8)
-        for img, o, s in zip(images, offsets, sizes):
-            pixels[o:o + s].copy_(img.reshape(-1))
+        sizes = [int(np.prod(img.shape)) for img in images]
+        order = [i for i in range(len(images)) if not dev[i]] + [i for i in range(len(images)) if dev[i]]
+        offsets = np.zeros(len(images), np.int64)
+        offsets[order] = np.concatenate([[0], np.cumsum([sizes[i] for i in order])[:-1]])
+        host_bytes = sum(sizes[i] for i in range(len(images)) if not dev[i])
+        pixels = torch.empty(host_bytes, dtype=torch.uint8)
+        for img, o, s, d in zip(images, offsets, sizes, dev):
+            if not d:
+                pixels[o:o + s].copy_(img.reshape(-1))
         geom = torch.tensor([(h, w, int(o), rh, rw, top, left) for (h, w, rh, rw, top, left, _, _), o in zip(geometry, offsets)],
                             dtype=torch.int64)
         kmax = (max(streaming.resample_kmax(g[1], g[3]) for g in geometry),
                 max(streaming.resample_kmax(g[0], g[2]) for g in geometry))
+        packed, files = None, None
+        if any(dev):
+            rows = [i for i in range(len(images)) if dev[i]]
+            packed = jpeg.pack([images[i] for i in rows], offsets[rows], rows)
+            files = [images[i].path or images[i].data for i in rows]      # bytes only without a path
         return PackedImages(pixels, geom, default_collate([label for _, label in batch]), self.resize, self.crop, out_hw,
-                            kmax)
+                            kmax, packed, files, sum(sizes))
 
 
-def gpu_resize_transform(resize=256, crop=224, interpolation="bilinear", max_size=None):
+def gpu_resize_transform(resize=256, crop=224, interpolation="bilinear", max_size=None, decode="host"):
     """Opt-in loader transform that moves Resize + CenterCrop (the reference's test_...:62-63) to the GPU, for loaders
     whose images have any sizes:
 
@@ -234,8 +287,18 @@ def gpu_resize_transform(resize=256, crop=224, interpolation="bilinear", max_siz
     decoded pixels, resamples them on the device bit for bit as the host transforms would, and hands on the same
     (B, 3, oh, ow) batch as a uint8_transform() loader. The upload is the decoded pixels (H * W * 3 bytes per image)
     rather than the resampled ones. Raises ValueError for what the kernel does not reproduce: another interpolation,
-    max_size, or a crop larger than the resize."""
-    return GpuResizeTransform(resize, crop, interpolation, max_size)
+    max_size, or a crop larger than the resize.
+
+    decode="gpu" also moves the decoding of baseline JPEG files to the device; give the dataset the transform's loader:
+
+        t = functions.gpu_resize_transform(256, 224, decode="gpu")
+        loader = DataLoader(ImageFolder(root, loader=t.loader, transform=t), batch_size=..., collate_fn=t.collate,
+                            pin_memory=True)
+
+    The workers then only read those files and parse their headers; the upload is the compressed scan data, and the
+    device decodes it bit for bit as Pillow does (csrc/jpeg.cuh). Every other file (progressive, arithmetic-coded, CMYK,
+    12-bit, PNG, ...) is decoded in the worker as before."""
+    return GpuResizeTransform(resize, crop, interpolation, max_size, decode)
 
 
 def _is_uint8_images(t):
@@ -312,23 +375,54 @@ def cuda_prefetch(batches, device, reuse_buffers=False, normalize="default"):
     def resample(slot, packed):
         n, (oh, ow), (hkmax, vkmax) = len(packed), packed.out_hw, packed.kmax
         tables = frames = None
+        jp = packed.jpeg
         if reuse_buffers:
-            src = grown(slot, "packed", packed.pixels.numel(), torch.uint8)
-            src.copy_(packed.pixels, non_blocking=True)
+            src = grown(slot, "packed", packed.arena_bytes, torch.uint8)
+            src[:packed.pixels.numel()].copy_(packed.pixels, non_blocking=True)
             geometry = staged(slot, "geometry", packed.geometry.shape, torch.int64)
             geometry.copy_(packed.geometry, non_blocking=True)
             tables = grown(slot, "tables", n * _lib.lib().gh_frame_tables_stride(oh, ow, hkmax, vkmax), torch.int32)
             frames = grown(slot, "frames", n * streaming.FRAME_DESC_DTYPE.itemsize, torch.uint8)
             out = staged(slot, "images", (n, 3, oh, ow), torch.uint8)
         else:
-            src = packed.pixels.to(device, non_blocking=True)
+            if jp is None:
+                src = packed.pixels.to(device, non_blocking=True)
+            else:
+                src = torch.empty(packed.arena_bytes, dtype=torch.uint8, device=device)
+                src[:packed.pixels.numel()].copy_(packed.pixels, non_blocking=True)
             geometry = packed.geometry.to(device, non_blocking=True)
             out = torch.empty((n, 3, oh, ow), dtype=torch.uint8, device=device)
+        status = None
+        if jp is not None:
+            status = decode(slot, packed, src)
         streaming.resample_images(src, geometry, packed.geometry.numpy(), out, hkmax, vkmax, tables, frames)
-        if normalize is None:
-            return out
-        return ops.normalize_u8(out, *normalize,
-                                out=staged(slot, "images_fp32", out.shape, torch.float32) if reuse_buffers else None)
+        if normalize is not None:
+            out = ops.normalize_u8(out, *normalize,
+                                   out=staged(slot, "images_fp32", out.shape, torch.float32) if reuse_buffers else None)
+        return out, status
+
+    def decode(slot, packed, arena):
+        """Uploads the compressed part of a decode="gpu" batch and decodes it into the arena; returns the images'
+        status words (uploaded to pinned host memory, read when the batch is handed on)."""
+        from . import jpeg
+        scan_h, segs_h, imgs_h, tables_h = packed.jpeg
+        imgs_np, segs_np = imgs_h.numpy(), segs_h.numpy()
+        if reuse_buffers:
+            up = []
+            for key, t in zip(("jscan", "jsegs", "jimgs", "jtables"), packed.jpeg):
+                buf = grown(slot, key, t.numel(), t.dtype)
+                buf.copy_(t.reshape(-1), non_blocking=True)
+                up.append(buf.view(t.shape))
+            n_coef, n_plane, n_rec = jpeg.workspace(imgs_np, scan_h.numel(), len(segs_np))
+            work = dict(coef=grown(slot, "jcoef", n_coef, torch.int16), planes=grown(slot, "jplanes", n_plane, torch.uint8),
+                        records=grown(slot, "jrecords", n_rec // 4, torch.int32),
+                        status=grown(slot, "jstatus", len(imgs_np), torch.int32))
+        else:
+            up, work = [t.to(device, non_blocking=True) for t in packed.jpeg], {}
+        status = jpeg.decode_batch(*up, imgs_np, segs_np, arena, packed.arena_bytes, **work)
+        host = torch.empty(status.shape, dtype=torch.int32, pin_memory=True)
+        host.copy_(status, non_blocking=True)
+        return host, imgs_np[:, 12]
 
     def upload(batch):
         nonlocal count
@@ -339,14 +433,16 @@ def cuda_prefetch(batches, device, reuse_buffers=False, normalize="default"):
         with torch.cuda.stream(copy_stream):
             if reuse_buffers and consumed[slot] is not None:
                 copy_stream.wait_event(consumed[slot])       # the batch that last lived in these buffers is done with
+            status = None
             if isinstance(batch, PackedImages):
                 labels = batch.labels
-                moved = (resample(slot, batch), place(slot, 1, labels) if torch.is_tensor(labels) else labels)
+                images, status = resample(slot, batch)
+                moved = (images, place(slot, 1, labels) if torch.is_tensor(labels) else labels)
             else:
                 moved = tuple(place(slot, i, t) if torch.is_tensor(t) else t for i, t in enumerate(batch))
         done = torch.cuda.Event()
         done.record(copy_stream)
-        return moved, done, slot
+        return moved, done, slot, status
 
     it = iter(batches)
     try:
@@ -355,7 +451,13 @@ def cuda_prefetch(batches, device, reuse_buffers=False, normalize="default"):
         return
     try:
         while pending is not None:
-            current, done, slot = pending
+            current, done, slot, status = pending
+            if status is not None:                  # decode="gpu": no batch is handed on with a broken image in it
+                done.synchronize()
+                bad = np.flatnonzero(status[0].numpy())
+                if bad.size:
+                    raise GramHeadError("gramhead: gpu JPEG decoding failed for batch index "
+                                        f"{', '.join(str(int(status[1][i])) for i in bad)} (corrupt or truncated scan)")
             main = torch.cuda.current_stream(device)
             main.wait_event(done)
             if not reuse_buffers:

@@ -409,6 +409,49 @@ int gh_attn_head_bwd2(const void* x_planes, const void* w_in_planes, const void*
                       float* dW_in, float* db_in, float* dW_out, float* db_out, float* dW_c, float* db_c, void* workspace,
                       void* stream);
 
+/* ---- Baseline JPEG decoding for the loaders (csrc/jpeg.cuh; functions.gpu_resize_transform(decode="gpu")) ----
+ * The output equals `np.asarray(Image.open(f).convert('RGB'))` byte for byte (Pillow + libjpeg-turbo: islow IDCT, fancy
+ * upsampling). The worker parses each file (jpeg.py): `scan` holds every restart segment's entropy-coded bytes with
+ * stuffing removed, back to back; `segs` one row per segment, `imgs` one row per image, `tables` GH_JPEG_TABLE_INTS
+ * ints per image: quantisation tables per component (64 ints, natural order), then per component a DC and an AC
+ * Huffman table of GH_JPEG_HUFF_INTS ints (a 9-bit lookahead of length << 8 | symbol, maxcode[17] and valoff[17] per
+ * code length, the symbols packed four per int). */
+enum { GH_JPEG_SEG_START, GH_JPEG_SEG_LEN, GH_JPEG_SEG_IMAGE, GH_JPEG_SEG_MCU, GH_JPEG_SEG_MCUS, GH_JPEG_SEG_COLS };
+enum { GH_JPEG_H, GH_JPEG_W, GH_JPEG_NCOMP, GH_JPEG_H0, GH_JPEG_V0, GH_JPEG_MCUX, GH_JPEG_MCUY, GH_JPEG_COEF_OFF,
+       GH_JPEG_BLOCKS, GH_JPEG_PLANE_OFF, GH_JPEG_ARENA_OFF, GH_JPEG_TABLE_OFF, GH_JPEG_BATCH_INDEX, GH_JPEG_IMG_COLS };
+#define GH_JPEG_QUANT_INTS 192
+#define GH_JPEG_HUFF_MAXCODE 512
+#define GH_JPEG_HUFF_VALOFF 530
+#define GH_JPEG_HUFF_VALS 547
+#define GH_JPEG_HUFF_INTS 612
+#define GH_JPEG_TABLE_INTS (GH_JPEG_QUANT_INTS + 6 * GH_JPEG_HUFF_INTS)
+#define GH_JPEG_PHASE_HUFFMAN 1
+#define GH_JPEG_PHASE_IDCT 2
+#define GH_JPEG_PHASE_COLOR 4
+/* A segment's length in bytes stays below this (bit positions inside a segment are 32-bit); the batch has no limit. */
+#define GH_JPEG_MAX_SEGMENT_BYTES (1LL << 28)
+
+/* Host-only: the ints per image of `tables` (GH_JPEG_TABLE_INTS). */
+int gh_jpeg_table_ints(void);
+/* Host-only: bytes of `records` gh_jpeg_decode needs for scan_bytes of scan data in n_segs segments cut into
+ * subsequences of subseq_bytes; GH_ERR_BAD_ARG for a non-positive count or size. */
+long long gh_jpeg_records_bytes(long long scan_bytes, int n_segs, int subseq_bytes);
+/* Decodes n_imgs images. All pointers are DEVICE memory. `phases` (GH_JPEG_PHASE_*) selects the launches, so that each
+ * can be timed alone: Huffman decoding (one CTA per segment, subsequences of subseq_bytes) into `coef` (int16, 64 per
+ * block, zeroed by the caller), which also zeroes and then sets `status[i]` to nonzero for an image whose scan runs out
+ * of bits, meets an invalid code or yields fewer blocks than its frame; the IDCT into `planes`; upsampling and colour
+ * into `arena`. max_blocks / max_pixels: the largest block count / H * W of an image. The caller checks every range in
+ * `segs` / `imgs` against the buffers, and every segment's length against GH_JPEG_MAX_SEGMENT_BYTES (the kernel sets the
+ * image's status for a longer one). Arguments as gh_jpeg_check. */
+/* Host-only: the argument check of gh_jpeg_decode (0, GH_ERR_BAD_ARG, or GH_ERR_UNSUPPORTED for n_imgs > 65535 or
+ * grids beyond the launch limits). The total scan_bytes of a batch is not limited. */
+int gh_jpeg_check(long long scan_bytes, int n_segs, int n_imgs, long long max_blocks, long long max_pixels,
+                  int subseq_bytes, int phases);
+int gh_jpeg_decode(const unsigned char* scan, long long scan_bytes, const long long* segs, int n_segs,
+                   const long long* imgs, int n_imgs, const int* tables, long long max_blocks, long long max_pixels,
+                   int subseq_bytes, short* coef, unsigned char* planes, int* records, int* status, unsigned char* arena,
+                   int phases, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
